@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- CTC fwd+bwd valid frames/s on B200 (BASELINE.json metric), one JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfgX] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfgX] [--impl reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path (log-softmax, alpha/beta recursion, gradient to the logits) over one
 synthetic batch.
@@ -32,6 +32,10 @@ Workloads (BASELINE.json `configs`):
            probe (N = 1, rank 0 only; bounded samples).
 `--impl reference`: the same C restatement as the measured arm (the reference's MXNet operator is not
            installable here -- DESIGN.md section 2), all host threads, SAME workload, seeds and config keys.
+`--dump-outputs DIR`: after the K timed steps, the outputs of the last one -- per-utterance losses `loss.npy` and
+           the logit gradient `grad.npy`, float32 -- go to DIR (one rank only).  The gradient is written whole when
+           it fits 63 MB, otherwise as a fixed seeded sample of utterances; `grad_rows.npy` lists which.  The inputs
+           depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import ctypes
@@ -109,6 +113,20 @@ def frames_per_step(name, steps, frames_of_set):
     return sum(frames_of_set[i % n] for i in range(steps)) / float(steps)
 
 
+DUMP_GRAD_BYTES = 63 * 10 ** 6      # the gradient's share of the 64 MB a dump may take; losses and row indices are small
+
+
+def dump_outputs(out_dir, loss, grad):
+    """Writes one step's outputs as float32 .npy files: loss (B,), grad (rows, T, V) and grad_rows, the utterance of
+    every gradient row -- all of them when the gradient fits DUMP_GRAD_BYTES, else a sample drawn with a fixed seed."""
+    B = grad.shape[0]
+    n = min(B, DUMP_GRAD_BYTES // (4 * grad[0].size))
+    rows = np.arange(B) if n == B else np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for key, a in (("loss", loss), ("grad", grad[rows]), ("grad_rows", rows)):
+        np.save(os.path.join(out_dir, key + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 class ClockSampler(threading.Thread):
     """NVML samples of SM clock and throttle reasons while the timed region runs."""
 
@@ -181,7 +199,7 @@ def cpu_step_fn(d, threads=None):
 
 def time_cpu_rotation(name, steps, warmup, budget_s=None, threads=None):
     """`steps` CPU steps over the same rotation of input sets the CUDA arm uses; returns (seconds per step list,
-    frames per step list, cores)."""
+    frames per step list, cores, (loss, grad, feasible) of the last step)."""
     n = n_sets(name)
     sets, fns = {}, {}
 
@@ -193,17 +211,17 @@ def time_cpu_rotation(name, steps, warmup, budget_s=None, threads=None):
         return fns[k][0], float(sets[k]["pred_lengths"].sum()), fns[k][1]
     for i in range(warmup):
         fn(i)[0]()
-    ts, fr, cores = [], [], 1
+    ts, fr, cores, out = [], [], 1, None
     t_start = time.perf_counter()
     for i in range(steps):
         f, frames, cores = fn(i)
         t0 = time.perf_counter()
-        f()
+        out = f()
         ts.append(time.perf_counter() - t0)
         fr.append(frames)
         if budget_s is not None and time.perf_counter() - t_start > budget_s and len(ts) >= 3:
             break
-    return ts, fr, cores
+    return ts, fr, cores, out
 
 
 def run_reference(args, rank, world):
@@ -212,7 +230,9 @@ def run_reference(args, rank, world):
     name = args.workload or default_workload(world)
     B, T, V, L = CONFIGS[name]
     warm = max(args.warmup, 1)
-    ts, fr, cores = time_cpu_rotation(name, args.steps, min(warm, 3))
+    ts, fr, cores, last = time_cpu_rotation(name, args.steps, min(warm, 3))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last[0], last[1])
     ms = 1e3 * sum(ts) / len(ts)
     val = sum(fr) / sum(ts)
     n = n_sets(name)
@@ -453,6 +473,9 @@ def run_cuda(args, rank, world, local_rank):
     sampler.sample()
     torch.cuda.synchronize()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        last = sets[(args.steps - 1) % nset]
+        dump_outputs(args.dump_outputs, last["loss"].cpu().numpy(), last["grad"].cpu().numpy())
     barrier()
     ms_total = e0.elapsed_time(e1)
     frames_all = sum(frames_global[i % nset] for i in range(args.steps))
@@ -733,7 +756,7 @@ def run_cuda(args, rank, world, local_rank):
 
     cpu_baseline = None
     if rank == 0 and world == 1:
-        ts, fr, cores = time_cpu_rotation(name, 1000, 2, budget_s=10.0)
+        ts, fr, cores, _ = time_cpu_rotation(name, 1000, 2, budget_s=10.0)
         cms = 1e3 * sum(ts) / len(ts)
         cpu_baseline = {"value": sum(fr) / sum(ts), "unit": UNIT, "cores": cores, "kind": "port",
                         "ms_per_step": cms,
@@ -901,16 +924,20 @@ def main():
                     help="N>1: loss-sum exchange through the library's peer mailbox (default) or torch.distributed's NCCL all-reduce")
     ap.add_argument("--peer-lag", type=int, default=4, help="slack between the ranks of the peer mailbox exchange, in steps")
     ap.add_argument("--no-allreduce", action="store_true", help="experiment: no loss-sum collective at all (N>1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's losses and gradient to DIR as .npy files (one rank)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
-        if args.steps > 50:
-            args.steps = 50          # each step is a full CPU pass (tens of ms and more); keep the run to minutes
         run_reference(args, rank, world)
         return
+    if args.dump_outputs and world > 1:
+        ap.error("--dump-outputs writes the outputs of one process: run it with WORLD_SIZE=1")
     run_cuda(args, rank, world, local_rank)
 
 
