@@ -46,9 +46,14 @@ typedef enum {
 typedef enum { CTCB_I32 = 0, CTCB_I64 = 1, CTCB_F32 = 2, CTCB_F64 = 3 } ctcb_dtype_t;
 
 /* per-utterance status bits written to ctcb_problem_t.status (optional) */
-#define CTCB_UTT_INFEASIBLE   1  /* L + repeats > T (or T == 0): loss 0, grad 0 (SURVEY 7.3-6) */
-#define CTCB_UTT_BAD_LABEL    2  /* a label was < 0, >= V or == blank: clamped / treated as is */
-#define CTCB_UTT_LEN_CLAMPED  4  /* data_length > T or label_length > Lmax: clamped */
+/* The parameter layer, identical on every kernel path.  Lengths are truncated toward zero, then clamped to [0, T] and
+ * [0, Lmax]; labels are truncated toward zero, then clamped to [0, V-1]; an inferred label length (label_lengths NULL)
+ * compares the unclamped truncated label with label_pad.  A label equal to the blank is a lattice state of its own that
+ * emits with the blank's probability, and the skip into label j is allowed exactly when label j != label j-1 (torch's
+ * rule), so every utterance with L + repeats <= T has a finite loss.  NaN labels or lengths have no defined meaning. */
+#define CTCB_UTT_INFEASIBLE   1  /* L + repeats > T (or T == 0), repeats of the clamped labels: loss 0, grad 0 (SURVEY 7.3-6) */
+#define CTCB_UTT_BAD_LABEL    2  /* one of the first L truncated labels was < 0, >= V or == blank: clamped / kept as a state */
+#define CTCB_UTT_LEN_CLAMPED  4  /* a truncated length was < 0, > T or > Lmax: clamped (a fractional length sets nothing) */
 #define CTCB_UTT_WIDE_LOGITS  8  /* CONTRACT DIFFERENCE from mx.nd.contrib.ctc_loss: an emission of a valid frame lay
                                   * more than 100 bits (69.3 nats) below the frame's largest softmax numerator and was
                                   * FLOORED there (small vocabularies: any symbol of the frame; wide ones: a blank or

@@ -41,6 +41,7 @@ import numpy as np
 
 __all__ = [
     "infer_lengths",
+    "param_layer",
     "ctc_loss_grad",
     "ctc_loss_op",
     "CtcLossOracle",
@@ -73,17 +74,71 @@ def infer_lengths(label, data_lengths, label_lengths, T, use_data_lengths,
     label = np.asarray(label)
     B, Lmax = label.shape
     if use_data_lengths:
-        T_b = np.asarray(data_lengths).astype(np.float64).astype(np.int64)
+        T_b = _trunc(data_lengths)
     else:
         T_b = np.full((B,), T, dtype=np.int64)
     if use_label_lengths:
-        L_b = np.asarray(label_lengths).astype(np.float64).astype(np.int64)
+        L_b = _trunc(label_lengths)
     else:
         pad = 0 if blank_label == "first" else -1
-        lab_i = label.astype(np.float64).astype(np.int64)
-        is_pad = lab_i == pad
+        is_pad = _trunc(label) == pad
         L_b = np.where(is_pad.any(axis=1), is_pad.argmax(axis=1), Lmax).astype(np.int64)
     return T_b, L_b
+
+
+UTT_INFEASIBLE, UTT_BAD_LABEL, UTT_LEN_CLAMPED = 1, 2, 4
+
+
+def _trunc(a):
+    """Truncation toward zero to int64, like the operator's cast (integers pass unchanged)."""
+    a = np.asarray(a)
+    if a.dtype.kind in "iu":
+        return a.astype(np.int64)
+    return np.trunc(a.astype(np.float64)).astype(np.int64)
+
+
+def param_layer(label, data_lengths, label_lengths, T, V, blank_label="first"):
+    """The operator's parameter layer: what the lattice kernels make of the caller's labels and lengths.
+
+    label (B, Lmax) of any numeric dtype; ``data_lengths`` / ``label_lengths`` (B,) or None (= T, resp. the
+    index of the first padding value -- 0 for blank_label='first', -1 for 'last' -- or Lmax).  Contract:
+
+    * lengths are truncated toward zero and clamped to [0, T] and [0, Lmax]; CTCB_UTT_LEN_CLAMPED (4) when a
+      clamp changed the truncated value (a fractional length sets nothing);
+    * an inferred label length compares the truncated, *unclamped* label with the padding value;
+    * labels are truncated toward zero and clamped to [0, V-1]; CTCB_UTT_BAD_LABEL (2) when one of the first
+      L_b truncated labels was < 0, >= V or equal to the blank (such a label is a lattice state of its own);
+    * CTCB_UTT_INFEASIBLE (1) when T_b == 0 or L_b + repeats > T_b (repeats of the clamped labels).
+
+    Returns (T_b, L_b, labels, status): int64 (B,), int64 (B,), int64 (B, Lmax) clamped, int32 (B,) without
+    CTCB_UTT_WIDE_LOGITS (8), which depends on the logits.
+    """
+    raw = _trunc(label)
+    B, Lmax = raw.shape
+    blank = 0 if blank_label == "first" else V - 1
+    status = np.zeros((B,), np.int32)
+    if data_lengths is None:
+        T_b = np.full((B,), T, np.int64)
+    else:
+        t = _trunc(data_lengths)
+        T_b = np.clip(t, 0, T)
+        status |= np.where(T_b != t, UTT_LEN_CLAMPED, 0).astype(np.int32)
+    if label_lengths is None:
+        _, L_b = infer_lengths(raw, None, None, T, False, False, blank_label)
+    else:
+        l = _trunc(label_lengths)
+        L_b = np.clip(l, 0, Lmax)
+        status |= np.where(L_b != l, UTT_LEN_CLAMPED, 0).astype(np.int32)
+    lab = np.clip(raw, 0, V - 1)
+    for b in range(B):
+        r = raw[b, :L_b[b]]
+        if np.any((r < 0) | (r >= V) | (r == blank)):
+            status[b] |= UTT_BAD_LABEL
+        c = lab[b, :L_b[b]]
+        repeats = int(np.sum(c[1:] == c[:-1])) if L_b[b] > 1 else 0
+        if T_b[b] <= 0 or L_b[b] + repeats > T_b[b]:
+            status[b] |= UTT_INFEASIBLE
+    return T_b, L_b, lab, status
 
 
 def _one_utterance(x, lab, blank):
@@ -100,9 +155,12 @@ def _one_utterance(x, lab, blank):
 
     ext = np.full((S,), blank, dtype=np.int64)
     ext[1::2] = lab
-    skip = np.zeros((S,), dtype=bool)                   # s-2 -> s transition allowed
+    # s-2 -> s transition allowed exactly when the two symbols differ.  Even states are blanks (never); a label
+    # state j skips in when label j != label j-1 -- a label equal to the blank is a state of its own (torch's rule;
+    # warp-ctc also forbids the skip into it, which can leave an utterance of L + repeats <= T_b without a path)
+    skip = np.zeros((S,), dtype=bool)
     if S > 2:
-        skip[2:] = (ext[2:] != blank) & (ext[2:] != ext[:-2])
+        skip[2:] = ext[2:] != ext[:-2]
     repeats = int(np.sum(lab[1:] == lab[:-1])) if L > 1 else 0
     if Tb <= 0 or L + repeats > Tb:
         # infeasible alignment: defined behaviour = cost 0, gradient 0 (SURVEY.md 7.3-6,
@@ -160,13 +218,13 @@ def ctc_loss_grad(data_tbv, label, T_b, L_b, blank=0, head_grad=None):
 
     data_tbv : (T, B, V) logits (unnormalised; the softmax is inside the op).
     label    : (B, Lmax) any numeric dtype, truncated to int (reader_kaldi_io.py:33-35
-               delivers float32 labels).
+               delivers float32 labels) and clamped to [0, V-1].
     Padded frames t >= T_b[b] get gradient 0 (SURVEY.md section 0 fact 6).
     Returns (loss, grad, feasible) as float64 / bool arrays.
     """
     x = np.asarray(data_tbv, dtype=np.float64)
     T, B, V = x.shape
-    lab = np.asarray(label).astype(np.float64).astype(np.int64)
+    lab = np.clip(_trunc(label), 0, V - 1)
     loss = np.zeros((B,))
     grad = np.zeros_like(x)
     ok = np.zeros((B,), dtype=bool)
@@ -190,9 +248,9 @@ def ctc_loss_op(data, label, data_lengths=None, label_lengths=None,
     T, B, V = data.shape
     assert blank_label in ("first", "last")
     blank = 0 if blank_label == "first" else V - 1
-    T_b, L_b = infer_lengths(label, data_lengths, label_lengths, T,
-                             use_data_lengths, use_label_lengths, blank_label)
-    return ctc_loss_grad(data, label, T_b, L_b, blank=blank, head_grad=head_grad)
+    T_b, L_b, lab, _ = param_layer(label, data_lengths if use_data_lengths else None,
+                                   label_lengths if use_label_lengths else None, T, V, blank_label)
+    return ctc_loss_grad(data, lab, T_b, L_b, blank=blank, head_grad=head_grad)
 
 
 class CtcLossOracle:
@@ -225,13 +283,18 @@ class CtcLossOracle:
         return loss, g, ok
 
 
+def _clamped_length(lengths, b, T):
+    """Frame count of utterance b: truncated toward zero, clamped to [0, T] (as the decode kernel does)."""
+    return int(min(max(int(_trunc(np.asarray(lengths)[b])), 0), T))
+
+
 def greedy_decode(logits_btv, lengths, blank=0):
     """Greedy CTC decode of scripts/swbd/train_ctc_ce.py:149-160: argmax over V, collapse
     repeats, drop blank (index 0).  Returns a list of int lists."""
     logits = np.asarray(logits_btv)
     out = []
     for b in range(logits.shape[0]):
-        n = int(np.asarray(lengths)[b])
+        n = _clamped_length(lengths, b, logits.shape[1])
         path = np.argmax(logits[b, :n], axis=1)
         seq, prev = [], None
         for j, c in enumerate(path):
@@ -253,7 +316,7 @@ def greedy_decode_unk(logits_btv, lengths, unk, blank=0):
     logits = np.asarray(logits_btv)
     out = []
     for b in range(logits.shape[0]):
-        n = int(np.asarray(lengths)[b])
+        n = _clamped_length(lengths, b, logits.shape[1])
         order = np.argsort(-logits[b, :n], axis=1, kind="stable")
         trans, trans2 = order[:, 0], order[:, 1] if logits.shape[2] > 1 else order[:, 0]
         seq = []

@@ -11,7 +11,8 @@
  * from the published algorithm (SURVEY.md section 8 rows a4-a8), not from its source:
  *
  *   a4  probability-space softmax per valid frame, max-subtracted;
- *   a5  blank-extended label lattice, repeats, feasibility (L + repeats <= T);
+ *   a5  blank-extended label lattice (labels clamped to [0, V-1]), repeats, feasibility
+ *       (L + repeats <= T);
  *   a6  log-space alpha recursion with the reachable-band limits;
  *   a7  log-space beta recursion fused with the per-label log-sum-exp of alpha+beta
  *       and  grad = y - exp(acc - log y - loglik);
@@ -32,6 +33,9 @@
 #ifdef _OPENMP
 #include <omp.h>
 #endif
+
+/* the operator's label clamp: out-of-range labels become the nearest valid symbol */
+static inline int clamp_label(int v, int V) { return v < 0 ? 0 : (v >= V ? V - 1 : v); }
 
 #define CAT_(a, b) a##b
 #define CAT(a, b) CAT_(a, b)

@@ -44,6 +44,14 @@ def max_threads() -> int:
     return int(lib().ctc_ref_max_threads())
 
 
+def _to_i32(a):
+    """Truncated toward zero, then saturated to int32: the library clamps lengths to [0, T] / [0, Lmax] and labels
+    to [0, V-1], so values beyond int32 (a length of 2^40, a label of 1e10) keep their meaning."""
+    a = np.asarray(a)
+    a = a.astype(np.int64) if a.dtype.kind in "iu" else np.trunc(a.astype(np.float64)).astype(np.int64)
+    return np.clip(a, np.iinfo(np.int32).min, np.iinfo(np.int32).max).astype(np.int32)
+
+
 def ctc_ref(data, label, T_b, L_b, blank=0, head_grad=None, layout="TNC", dtype=np.float32,
             need_grad=True, num_threads=0, out_grad=None):
     """Loss (B,) and gradient (same layout as data) of the C restatement.
@@ -58,12 +66,12 @@ def ctc_ref(data, label, T_b, L_b, blank=0, head_grad=None, layout="TNC", dtype=
     else:
         B, T, V = x.shape
         st_t, st_b = V, T * V
-    lab = np.ascontiguousarray(np.asarray(label).astype(np.float64).astype(np.int32))
+    lab = np.ascontiguousarray(_to_i32(label))
     Lmax = lab.shape[1] if lab.ndim == 2 and lab.shape[1] > 0 else 0
     if Lmax == 0:
         lab = np.zeros((B, 1), np.int32)
-    tl = np.ascontiguousarray(np.asarray(T_b).astype(np.float64).astype(np.int32))
-    ll = np.ascontiguousarray(np.asarray(L_b).astype(np.float64).astype(np.int32))
+    tl = np.ascontiguousarray(_to_i32(T_b))
+    ll = np.ascontiguousarray(_to_i32(L_b))
     costs = np.zeros((B,), dtype=dtype)
     feas = np.zeros((B,), dtype=np.int32)
     g = None

@@ -16,7 +16,7 @@ static int CAT(one_utt_, SUFFIX)(const REAL* x, long st_t, REAL* g, long gst_t,
                                  REAL head, REAL* cost) {
     const int S = 2 * L + 1;
     int repeats = 0;
-    for (int i = 1; i < L; ++i) repeats += (lab[i] == lab[i - 1]);
+    for (int i = 1; i < L; ++i) repeats += (clamp_label(lab[i], V) == clamp_label(lab[i - 1], V));
     *cost = 0;
     if (Tb <= 0 || L + repeats > Tb) return 0;
 
@@ -28,8 +28,10 @@ static int CAT(one_utt_, SUFFIX)(const REAL* x, long st_t, REAL* g, long gst_t,
     int* ext = (int*)malloc(sizeof(int) * 2 * (size_t)S);
     int* skip = ext + S;   /* skip[s] = 1 when the s-2 -> s transition is allowed */
 
-    for (int s = 0; s < S; ++s) ext[s] = (s & 1) ? lab[s / 2] : blank;
-    for (int s = 0; s < S; ++s) skip[s] = (s >= 2 && ext[s] != blank && ext[s] != ext[s - 2]);
+    /* labels clamped to [0, V-1]; a skip into a state is allowed exactly when its symbol differs from the one two
+     * states back (a label equal to the blank is a state of its own, as in torch's ctc_loss) */
+    for (int s = 0; s < S; ++s) ext[s] = (s & 1) ? clamp_label(lab[s / 2], V) : blank;
+    for (int s = 0; s < S; ++s) skip[s] = (s >= 2 && ext[s] != ext[s - 2]);
 
     /* a4: softmax in probability space */
     for (int t = 0; t < Tb; ++t) {

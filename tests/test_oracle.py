@@ -199,3 +199,144 @@ def test_greedy_decode_unk_rule():
     # reference compares with the RAW previous symbol, so the repeated 1 is NOT collapsed); j=5: curr=0 blank dropped
     assert O.greedy_decode_unk(x, [7], unk) == [[2, 1, 1, 4]]
     assert O.greedy_decode_unk(x, [7], -1) == O.greedy_decode(x, [7])
+
+
+# ---- the parameter layer: labels equal to the blank, out-of-range labels, clamped lengths -----------------------------
+def _torch_fp64_loss(x_tbv, lab, Tb, Lb, blank):
+    """torch's CPU ctc_loss in fp64 (an independent restatement of the forward), per utterance."""
+    torch = pytest.importorskip("torch")
+    xt = torch.tensor(x_tbv, dtype=torch.float64)
+    return torch.nn.functional.ctc_loss(xt.log_softmax(-1), torch.tensor(lab, dtype=torch.long),
+                                        torch.tensor(Tb, dtype=torch.long), torch.tensor(Lb, dtype=torch.long),
+                                        blank=blank, reduction="none", zero_infinity=False).numpy()
+
+
+@pytest.mark.parametrize("blank_last", [False, True])
+def test_label_equal_to_blank_matches_torch_fp64(blank_last):
+    """A label equal to the blank is a lattice state of its own that emits with the blank's probability, and the skip
+    into label j is allowed exactly when label j != label j-1 (torch's rule).  Both oracles agree with torch's fp64
+    ctc_loss on rows with such labels at the first, middle and last position, twice in a row, and with only L + repeats
+    frames -- where forbidding the skip into it (warp-ctc's rule) leaves no path at all and an infinite loss.
+
+    The gradients are checked against central differences of torch's loss: torch's own backward is wrong when the
+    LAST label equals the blank (it does not match the derivative of its forward there)."""
+    rng = np.random.default_rng(31)
+    T, V = 9, 6
+    bl = V - 1 if blank_last else 0
+    a, c = (1, 2) if not blank_last else (0, 2)
+    rows = [([a, bl, c], 6), ([bl, a, bl], 7), ([a, bl, bl], 4), ([bl, bl, bl], 5), ([c, a, bl], 9),
+            ([a, c, a], 3), ([bl, c, c], 5)]
+    B, L = len(rows), 3
+    lab = np.array([r for r, _ in rows], np.int64)
+    Tb = np.array([t for _, t in rows], np.int64)
+    Lb = np.full((B,), L, np.int64)
+    x = rng.standard_normal((T, B, V))
+    head = rng.uniform(0.5, 1.5, B)
+    lt = _torch_fp64_loss(x, lab, Tb, Lb, bl)
+    assert np.isfinite(lt).all()
+    eps = 1e-6
+    gt = np.zeros_like(x)
+    for idx in np.ndindex(*x.shape):
+        xp = x.copy(); xp[idx] += eps
+        xm = x.copy(); xm[idx] -= eps
+        gt[idx] = ((_torch_fp64_loss(xp, lab, Tb, Lb, bl) - _torch_fp64_loss(xm, lab, Tb, Lb, bl)) * head).sum() / (2 * eps)
+    lo, go, ok = O.ctc_loss_grad(x, lab, Tb, Lb, bl, head)
+    lc, gc, okc = R.ctc_ref(x, lab, Tb, Lb, bl, head, dtype=np.float64)
+    assert ok.all() and okc.all()
+    for b in range(B):
+        gc[Tb[b]:, b] = 0.0                      # the C restatement leaves padded frames to its caller's buffer
+    np.testing.assert_allclose(lo, lt, rtol=1e-12, atol=1e-12)
+    np.testing.assert_allclose(lc, lt, rtol=1e-11, atol=1e-11)
+    np.testing.assert_allclose(go, gt, rtol=0, atol=2e-8)
+    np.testing.assert_allclose(gc, go, rtol=1e-9, atol=1e-11)
+
+
+def test_param_layer_status_words():
+    """param_layer on a hand-written table: truncation toward zero, clamps, which clamps report CTCB_UTT_LEN_CLAMPED (4),
+    which labels report CTCB_UTT_BAD_LABEL (2), feasibility on the clamped labels (CTCB_UTT_INFEASIBLE, 1)."""
+    T, V = 10, 7
+    #            labels (blank 0)              T_b       L_b    -> T_b L_b status
+    table = [([1, 2, 3, 4], 10, 4, 10, 4, 0),
+             ([1, 2, 3, 4], 10.9, 3.9, 10, 3, 0),         # fractional: truncated, no bit
+             ([1, 2, 3, 4], 11, 4, 10, 4, 4),             # > T
+             ([1, 2, 3, 4], -1, 4, 0, 4, 4 | 1),          # negative: 0 frames
+             ([1, 2, 3, 4], -0.9, 4, 0, 4, 1),            # truncates to 0: no clamp
+             ([1, 2, 3, 4], 0, 4, 0, 4, 1),               # no frames
+             ([1, 2, 3, 4], 2 ** 40, 4, 10, 4, 4),        # huge
+             ([1, 2, 3, 4], 10, 5, 10, 4, 4),             # > Lmax
+             ([1, 2, 3, 4], 10, -3, 10, 0, 4),            # negative: empty label sequence
+             ([1, 7, 3, 4], 10, 4, 10, 4, 2),             # == V
+             ([1, 2, -1, 4], 10, 4, 10, 4, 2),            # negative label
+             ([1, 2, 3, -1], 10, 3, 10, 3, 0),            # a bad label past L_b is not read
+             ([1, 0, 3, 4], 10, 4, 10, 4, 2),             # == blank
+             ([1, 2.9, -0.9, 4], 10, 4, 10, 4, 2),        # -0.9 truncates to 0 == blank; 2.9 -> 2
+             ([1e10, 9, 3, 4], 10, 4, 10, 4, 2),          # 1e10 and 9 both clamp to 6: a repeat (5 frames)
+             ([1e10, 9, 3, 4], 4, 4, 4, 4, 2 | 1),        # ... so 4 frames are too few
+             ([0, 0, 0, 0], 7, 4, 7, 4, 2),               # all blank: 3 repeats, 7 frames suffice
+             ([0, 0, 0, 0], 6, 4, 6, 4, 2 | 1),
+             ([1, 2, 3, 4], 12.5, 9, 10, 4, 4)]           # both clamped: one bit
+    lab = np.array([r[0] for r in table], np.float64)
+    dl = np.array([r[1] for r in table], np.float64)
+    ll = np.array([r[2] for r in table], np.float64)
+    Tb, Lb, labc, st = O.param_layer(lab, dl, ll, T, V, "first")
+    assert list(Tb) == [r[3] for r in table]
+    assert list(Lb) == [r[4] for r in table]
+    assert list(st) == [r[5] for r in table]
+    assert labc.min() >= 0 and labc.max() <= V - 1 and labc[13].tolist() == [1, 2, 0, 4]
+    # inferred lengths: the first TRUNCATED label equal to the padding value (0 blank first, -1 blank last), unclamped
+    lab = np.array([[3, 2, 0, 5], [3, -0.5, 2, 1], [0, 1, 2, 3], [1, 2, 3, 4], [9, -3, 0, 1]], np.float32)
+    Tb, Lb, _, st = O.param_layer(lab, None, None, T, V, "first")
+    assert list(Tb) == [T] * 5 and list(Lb) == [2, 1, 0, 4, 2] and list(st) == [0, 0, 0, 0, 2]
+    lab = np.array([[3, 2, -1, 5], [3, -1.5, 2, 1], [-1, 1, 2, 3], [0, 6, 3, 4], [9, -3, -1, 1]], np.float32)
+    _, Lb, labc, st = O.param_layer(lab, None, None, T, V, "last")
+    assert list(Lb) == [2, 1, 0, 4, 2] and list(st) == [0, 0, 0, 2, 2]
+    assert labc[4, :2].tolist() == [6, 0]
+    # integer dtypes give the same answer as the float dtypes holding the same values
+    for dt in (np.int32, np.int64):
+        _, Lb2, labc2, st2 = O.param_layer(lab.astype(np.float64).astype(dt), None, None, T, V, "last")
+        assert list(Lb2) == list(Lb) and list(st2) == list(st) and (labc2 == labc).all()
+
+
+@pytest.mark.parametrize("blank_last,inferred", [(False, False), (True, False), (False, True), (True, True)])
+def test_oracles_agree_on_out_of_range_inputs(blank_last, inferred):
+    """The numpy and the C oracle (1e-11) on the hostile batch: labels >= V, negative, fractional, huge, equal to the
+    blank; lengths beyond T and Lmax, negative, fractional, huge; inferred label lengths.  Both clamp as the operator
+    does; infeasible rows are exactly 0.  The C oracle takes the labels unclamped (it clamps while building the lattice)."""
+    from tests.synth import hostile_batch
+    T, V, Lmax = 40, 11, 12
+    bl = "last" if blank_last else "first"
+    for ld, nd in (("f32", "f64"), ("i64", "i32"), ("f64", "i64")):
+        d = hostile_batch(T, V, Lmax, blank_last=blank_last, label_dtype=ld, length_dtype=nd, inferred=inferred, seed=3)
+        B = d["pred"].shape[0]
+        head = np.linspace(0.5, 1.5, B)
+        lo, go, ok = O.CtcLossOracle("NTC", "NT", bl)(d["pred"], d["label"], d["pred_lengths"], d["label_lengths"],
+                                                      head_grad=head)
+        Tb, Lb, labc, st = O.param_layer(d["label"], d["pred_lengths"], d["label_lengths"], T, V, bl)
+        np.testing.assert_array_equal(ok, (st & 1) == 0)
+        assert (st & 1).any() and (st & 2).any() and ((st & 4).any() or inferred)
+        assert (lo[~ok] == 0).all() and (go[~ok] == 0).all() and np.isfinite(lo).all()
+        lc, gc, okc = R.ctc_ref(d["pred"], d["label"], Tb, Lb, blank=V - 1 if blank_last else 0, head_grad=head,
+                                layout="NTC", dtype=np.float64)
+        np.testing.assert_array_equal(okc, ok)
+        for b in range(B):
+            gc[b, Tb[b]:] = 0.0
+        np.testing.assert_allclose(lc, lo, rtol=1e-11, atol=1e-11)
+        np.testing.assert_allclose(gc, go, rtol=1e-9, atol=1e-11)
+        # the raw lengths straight into the C oracle: it clamps them itself (huge values saturate on the way to int32)
+        if not inferred:
+            lc2, _, _ = R.ctc_ref(d["pred"], d["label"], d["pred_lengths"], d["label_lengths"],
+                                  blank=V - 1 if blank_last else 0, head_grad=head, layout="NTC", dtype=np.float64)
+            np.testing.assert_array_equal(lc2, lc)
+
+
+def test_greedy_decode_clamps_lengths():
+    """Frame counts are truncated toward zero and clamped to [0, T]: a negative one decodes nothing (it does not
+    slice from the end), one beyond T decodes every frame."""
+    rng = np.random.default_rng(4)
+    x = rng.standard_normal((5, 12, 6))
+    full = O.greedy_decode(x, [12] * 5)
+    assert O.greedy_decode(x, np.array([-3, 40, 7.9, -0.5, 2 ** 40], dtype=np.float64)) == [
+        [], full[1], O.greedy_decode(x[2:3], [7])[0], [], full[4]]
+    assert O.greedy_decode_unk(x, np.array([-3, 40, 5, 0, 12], np.int64), unk=2) == [
+        [], O.greedy_decode_unk(x[1:2], [12], 2)[0], O.greedy_decode_unk(x[2:3], [5], 2)[0], [],
+        O.greedy_decode_unk(x[4:5], [12], 2)[0]]
