@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("CTCB_LIB_PATH") or os.path.join(_HERE, "libctcb.so")
 
 CTCB_OK, CTCB_INVALID_VALUE, CTCB_WORKSPACE_TOO_SMALL, CTCB_EXECUTION_FAILED, CTCB_MEMOPS_FAILED, CTCB_UNSUPPORTED = range(6)
 DT_I32, DT_I64, DT_F32, DT_F64 = range(4)
+DT_BF16 = 4             # CTCB_BF16: a logits type only (the *_typed entries), never a label or length type
 UTT_INFEASIBLE, UTT_BAD_LABEL, UTT_LEN_CLAMPED, UTT_WIDE_LOGITS = 1, 2, 4, 8
 LAYOUT_NTC, LABEL_TN, KEEP_FOR_BACKWARD = 1, 2, 4
 PHASE_FUSED, PHASE_FORWARD, PHASE_BACKWARD = 0 << 8, 1 << 8, 2 << 8
@@ -28,6 +29,7 @@ EXPORTS = (
     "ctcb_mailbox_flush", "ctcb_mailbox_destroy", "ctcb_mailbox_exchange_with_next",
     "ctcb_set_option", "ctcb_get_option", "ctcb_greedy_decode_unk", "ctcb_last_grad_kernel",
     "ctcb_proj_forward", "ctcb_proj_loss_grad",
+    "ctcb_loss_grad_typed", "ctcb_forward_typed", "ctcb_backward_typed", "ctcb_greedy_decode_typed",
 )
 
 
@@ -82,6 +84,9 @@ def load():
     lib.ctcb_loss_grad.argtypes = [PP, vp, sz, vp]
     lib.ctcb_forward.argtypes = [PP, i32, vp, sz, vp]
     lib.ctcb_backward.argtypes = [PP, vp, sz, vp]
+    lib.ctcb_loss_grad_typed.argtypes = [PP, i32, vp, sz, vp]
+    lib.ctcb_forward_typed.argtypes = [PP, i32, i32, vp, sz, vp]
+    lib.ctcb_backward_typed.argtypes = [PP, i32, vp, sz, vp]
     lib.ctcb_loss_grad_timed.argtypes = [PP, vp, sz, vp, ctypes.POINTER(ctypes.c_float), ctypes.POINTER(i32)]
     lib.ctcb_loss_grad_host.argtypes = [PP, ctypes.c_int]
     lib.ctcb_loss_grad_host_resident.argtypes = [PP, ctypes.c_int, ctypes.POINTER(vp)]
@@ -99,6 +104,7 @@ def load():
     lib.ctcb_mailbox_destroy.argtypes = [vp]
     lib.ctcb_greedy_decode.argtypes = [vp, i64, i64, vp, i32, i32, i32, i32, i32, vp, vp, vp]
     lib.ctcb_greedy_decode_unk.argtypes = [vp, i64, i64, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp]
+    lib.ctcb_greedy_decode_typed.argtypes = [vp, i32, i64, i64, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp]
     lib.ctcb_scale_rows.argtypes = [vp, i64, i64, i32, i32, i32, vp, vp]
     lib.ctcb_edit_distance.argtypes = [vp, i64, vp, vp, i64, vp, i32, i32, i32, vp, vp, vp]
     lib.ctcb_loss_sum_allreduce.argtypes = [vp, vp, i32, vp]

@@ -99,9 +99,10 @@ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 struct WalkCfg { int P, NW; };
 
 using WalkFn = void (*)(ctcb::WalkArgs);
-struct WalkEntry { int P, NW; WalkFn fn[2][2]; };   // [FUSED][HIST]
+struct WalkEntry { int P, NW; WalkFn fn[2][2]; WalkFn fused_bf16[2]; };   // fn[FUSED][HIST]; bf16 logits: fused_bf16[HIST]
 #define WALK(P_, NW_) {P_, NW_, {{ctcb::k_walk<P_, NW_, false, false>, ctcb::k_walk<P_, NW_, true, false>}, \
-                                 {ctcb::k_walk<P_, NW_, false, true>, ctcb::k_walk<P_, NW_, true, true>}}}
+                                 {ctcb::k_walk<P_, NW_, false, true>, ctcb::k_walk<P_, NW_, true, true>}},  \
+                                 {ctcb::k_walk<P_, NW_, false, true, ctcb::bf16>, ctcb::k_walk<P_, NW_, true, true, ctcb::bf16>}}
 #ifdef CTCB_SMALL_TABLE   // experiment builds: the configurations the BASELINE shapes use
 const WalkEntry kWalkTable[] = { WALK(1, 1), WALK(2, 1), WALK(1, 4), WALK(2, 2), WALK(4, 1), WALK(2, 3), WALK(2, 5) };
 #else
@@ -152,7 +153,8 @@ bool overlap_allowed(int B, bool fused) {
     return B <= 296;
 }
 
-// the one-kernel path (k_meet): opt-in / opt-out through the "meet" option, automatic otherwise
+// the one-kernel path (k_meet): opt-in / opt-out through the "meet" option, automatic otherwise.  fp32 logits only: a call
+// with bf16 logits takes the two-kernel path whatever the option says (k_meet has no bf16 instantiation)
 bool meet_wanted(int B) {
     if (opt(OPT_MEET) >= 0) return opt(OPT_MEET) != 0;
     (void)B;
@@ -270,14 +272,21 @@ ctcb::Workspace carve(const Layout& l, void* ws) {
     return w;
 }
 
-int pick_vec(const void* base, long long st_t, long long st_b, int V) {
+// elements per vector load (VEC is counted in elements; the base must be aligned to VEC * esz bytes)
+int pick_vec(const void* base, long long st_t, long long st_b, int V, int esz = 4) {
     auto ok = [&](int v) {
-        return V % v == 0 && st_t % v == 0 && st_b % v == 0 && (reinterpret_cast<uintptr_t>(base) % (v * sizeof(float))) == 0;
+        return V % v == 0 && st_t % v == 0 && st_b % v == 0 && (reinterpret_cast<uintptr_t>(base) % (v * esz)) == 0;
     };
     if (ok(4)) return 4;
     if (ok(2)) return 2;
     return 1;
 }
+// rows that 1-D bulk copies (TMA) can move: 16-byte aligned row starts and a row of a multiple of 16 bytes.  For fp32 rows
+// VEC = 4 already says so; bf16 rows with VEC = 4 are only 8-byte aligned and need the check
+bool rows16(const void* base, long long st_t, long long st_b, int V, int esz) {
+    return ((long long)V * esz) % 16 == 0 && (st_t * esz) % 16 == 0 && (st_b * esz) % 16 == 0 && reinterpret_cast<uintptr_t>(base) % 16 == 0;
+}
+inline int dtype_size(int logits_dtype) { return logits_dtype == CTCB_BF16 ? 2 : 4; }
 
 int validate(const ctcb_problem_t* p) {
     if (!p) return fail(CTCB_INVALID_VALUE, "problem is NULL");
@@ -488,9 +497,16 @@ int launch_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const ctcb::Prob
     return CTCB_OK;
 }
 
-int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream_, int phases, bool keep_hist) {
+// ldt: element type of p->logits and p->grad (CTCB_F32 or CTCB_BF16)
+int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream_, int phases, bool keep_hist,
+            int ldt = CTCB_F32) {
     g_grad_kernel = 0;
     if (int rc = validate(p)) return rc;
+    if (ldt != CTCB_F32 && ldt != CTCB_BF16)
+        return fail(CTCB_INVALID_VALUE, "logits dtype %d is neither CTCB_F32 nor CTCB_BF16 (fp16 logits are not supported)", ldt);
+    if (ldt != CTCB_F32 && g_proj) return fail(CTCB_INVALID_VALUE, "the fused projection writes fp32 logits");
+    const bool bf = ldt == CTCB_BF16;
+    const int esz = dtype_size(ldt);
     const bool need_grad = keep_hist || (phases & PH_BACKWARD);
     if ((phases & PH_BACKWARD) && !p->grad) return fail(CTCB_INVALID_VALUE, "grad is NULL");
     const Layout lay = make_layout(p->T, p->B, p->V, p->Lmax, need_grad);
@@ -507,7 +523,7 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
     w.poll_ns = opt(OPT_GRAD_POLL_NS);
 
     // ---- the one-kernel path (ctcb_meet.cuh): forward and gradient of small-vocabulary utterances in one CTA each ----
-    if (phases == (PH_FORWARD | PH_BACKWARD) && lay.fused && p->V <= 64 && p->Lmax + 1 <= 128 && meet_wanted(p->B)) {
+    if (phases == (PH_FORWARD | PH_BACKWARD) && !bf && lay.fused && p->V <= 64 && p->Lmax + 1 <= 128 && meet_wanted(p->B)) {
         const int mp = p->Lmax + 1 <= 32 ? 1 : p->Lmax + 1 <= 64 ? 2 : 4;
         const size_t need = sizeof(int2) * (size_t)p->B * lay.NB * ctcb::kHR * 32 * mp;
         if (lay.off_hA + need <= lay.total) {
@@ -534,7 +550,7 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
         int stages = 0;
         if (!pick_stages(lay.W, we->NW, lay.fused ? lay.Lp : 0, &stages))
             return fail(CTCB_UNSUPPORTED, "Lmax=%d V=%d: the emission ring does not fit in shared memory", p->Lmax, p->V);
-        const WalkFn wfn = we->fn[lay.fused][need_grad ? 1 : 0];
+        const WalkFn wfn = (bf && lay.fused) ? we->fused_bf16[need_grad ? 1 : 0] : we->fn[lay.fused][need_grad ? 1 : 0];
         size_t smem = ctcb::walk_smem_bytes(lay.W, we->NW, stages, lay.fused ? lay.Lp : 0);
         if (lay.fused && need_grad && (phases & PH_BACKWARD) && overlap_allowed(p->B, true)) {
             // SM partitioning by shared-memory reservation: the gradient kernel runs concurrently
@@ -558,14 +574,16 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
             if (want > cap) want = cap;
             if (want > smem) smem = want;
         }
-        const int vec = pick_vec(p->logits, p->logits_stride_t, p->logits_row_offsets ? 0 : p->logits_stride_b, p->V);
+        const int vec = pick_vec(p->logits, p->logits_stride_t, p->logits_row_offsets ? 0 : p->logits_stride_b, p->V, esz);
         CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(wfn), smem));
         // NQ: vector loads per lane that hold one logits row in registers (0 = two-pass)
         const int units = (p->V / vec + 31) / 32;
         int nq = units <= 1 ? 1 : units <= 2 ? 2 : units <= 4 ? 4 : units <= 8 ? 8 : units <= 16 ? 16 : 0;
         // wide vocabularies with 16-byte aligned rows: the frame block's rows staged in shared memory by bulk copies
+        // (bf16 rows: also V * 2 a multiple of 16 bytes and 16-byte aligned rows)
         const bool staged = !lay.fused && vec == 4 && (nq == 0 || nq >= 8) && ctcb::emit_smem_bytes(lay.Lp, p->V) <= 75 * 1024 &&
-                            opt(OPT_EMIT_STAGED) != 0;
+                            opt(OPT_EMIT_STAGED) != 0 &&
+                            rows16(p->logits, p->logits_stride_t, p->logits_row_offsets ? 0 : p->logits_stride_b, p->V, esz);
         if (staged) nq = -1;
         auto launch_emit = [&]() -> int {
             const int bpc = ctcb::emit_blocks_per_cta(nq);
@@ -573,11 +591,11 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
             const dim3 egrid(nblk, p->B);
             const size_t esm = ctcb::emit_smem_bytes(lay.Lp, staged ? p->V : 0);
             if (staged) {
-                auto efn = ctcb::k_emit<4, -1>;
+                auto efn = bf ? ctcb::k_emit<4, -1, ctcb::bf16> : ctcb::k_emit<4, -1>;
                 if (esm > 48 * 1024) CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(efn), esm));
                 efn<<<egrid, 256, esm, stream>>>(dp, w);
             } else {
-#define EMIT_LAUNCH(V_, Q_) ctcb::k_emit<V_, Q_><<<egrid, 128, esm, stream>>>(dp, w)
+#define EMIT_LAUNCH(V_, Q_) (bf ? ctcb::k_emit<V_, Q_, ctcb::bf16> : ctcb::k_emit<V_, Q_>)<<<egrid, 128, esm, stream>>>(dp, w)
 #define EMIT_NQ(V_) switch (nq) { case 1: EMIT_LAUNCH(V_, 1); break; case 2: EMIT_LAUNCH(V_, 2); break; \
                                   case 4: EMIT_LAUNCH(V_, 4); break; case 8: EMIT_LAUNCH(V_, 8); break;  \
                                   case 16: EMIT_LAUNCH(V_, 16); break; default: EMIT_LAUNCH(V_, 0); break; }
@@ -643,8 +661,8 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
         size_t gsm = ctcb::grad_smem_bytes(lay.Lp, 32 * gch);
         int gthreads = 128;
         if (gsm > 200 * 1024) return fail(CTCB_UNSUPPORTED, "Lmax=%d too long for the gradient kernel", p->Lmax);
-        int vec = pick_vec(p->logits, p->logits_stride_t, p->logits_row_offsets ? 0 : p->logits_stride_b, p->V);
-        const int gvec = pick_vec(p->grad, p->grad_stride_t, p->grad_stride_b, p->V);
+        int vec = pick_vec(p->logits, p->logits_stride_t, p->logits_row_offsets ? 0 : p->logits_stride_b, p->V, esz);
+        const int gvec = pick_vec(p->grad, p->grad_stride_t, p->grad_stride_b, p->V, esz);
         if (gvec < vec) vec = gvec;
         const int ch = gch;
         const int units = (p->V / vec + 31) / 32;
@@ -652,17 +670,21 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
         const dim3 ggrid(p->B, lay.NB);                  // one frame block per CTA, utterance-fastest
         using GradFn = void (*)(ctcb::GradArgs);
         GradFn gfn = nullptr;
-#define GRAD_X(V_, C_) (xq == 1 ? ctcb::k_grad<V_, C_, 1> : xq == 2 ? ctcb::k_grad<V_, C_, 2> : xq == 4 ? ctcb::k_grad<V_, C_, 4> : ctcb::k_grad<V_, C_, 0>)
-#define GRAD_CH(V_) (ch == 1 ? GRAD_X(V_, 1) : ch == 2 ? GRAD_X(V_, 2) : ch == 4 ? GRAD_X(V_, 4) : ch == 8 ? GRAD_X(V_, 8) : \
-                     ch == 16 ? GRAD_X(V_, 16) : GRAD_X(V_, 0))
-        gfn = vec == 4 ? GRAD_CH(4) : vec == 2 ? GRAD_CH(2) : GRAD_CH(1);
+#define GRAD_X(V_, C_, T_) (xq == 1 ? ctcb::k_grad<V_, C_, 1, 0, T_> : xq == 2 ? ctcb::k_grad<V_, C_, 2, 0, T_> : \
+                            xq == 4 ? ctcb::k_grad<V_, C_, 4, 0, T_> : ctcb::k_grad<V_, C_, 0, 0, T_>)
+#define GRAD_CH(V_, T_) (ch == 1 ? GRAD_X(V_, 1, T_) : ch == 2 ? GRAD_X(V_, 2, T_) : ch == 4 ? GRAD_X(V_, 4, T_) : ch == 8 ? GRAD_X(V_, 8, T_) : \
+                         ch == 16 ? GRAD_X(V_, 16, T_) : GRAD_X(V_, 0, T_))
+        if (bf) gfn = vec == 4 ? GRAD_CH(4, ctcb::bf16) : vec == 2 ? GRAD_CH(2, ctcb::bf16) : GRAD_CH(1, ctcb::bf16);
+        else    gfn = vec == 4 ? GRAD_CH(4, float) : vec == 2 ? GRAD_CH(2, float) : GRAD_CH(1, float);
 #undef GRAD_CH
 #undef GRAD_X
         // batches that run after the walkers (no overlap): the high-occupancy variant of the register-resident kernels
         if (ch >= 1 && ch <= 4 && !((phases & PH_FORWARD) && !g_prof_events && overlap_allowed(p->B, lay.fused != 0))) {
-#define GRADO_X(V_, C_) (xq == 1 ? ctcb::k_grad<V_, C_, 1, 1> : xq == 2 ? ctcb::k_grad<V_, C_, 2, 1> : xq == 4 ? ctcb::k_grad<V_, C_, 4, 1> : ctcb::k_grad<V_, C_, 0, 1>)
-#define GRADO_CH(V_) (ch == 1 ? GRADO_X(V_, 1) : ch == 2 ? GRADO_X(V_, 2) : GRADO_X(V_, 4))
-            gfn = vec == 4 ? GRADO_CH(4) : vec == 2 ? GRADO_CH(2) : GRADO_CH(1);
+#define GRADO_X(V_, C_, T_) (xq == 1 ? ctcb::k_grad<V_, C_, 1, 1, T_> : xq == 2 ? ctcb::k_grad<V_, C_, 2, 1, T_> : \
+                             xq == 4 ? ctcb::k_grad<V_, C_, 4, 1, T_> : ctcb::k_grad<V_, C_, 0, 1, T_>)
+#define GRADO_CH(V_, T_) (ch == 1 ? GRADO_X(V_, 1, T_) : ch == 2 ? GRADO_X(V_, 2, T_) : GRADO_X(V_, 4, T_))
+            if (bf) gfn = vec == 4 ? GRADO_CH(4, ctcb::bf16) : vec == 2 ? GRADO_CH(2, ctcb::bf16) : GRADO_CH(1, ctcb::bf16);
+            else    gfn = vec == 4 ? GRADO_CH(4, float) : vec == 2 ? GRADO_CH(2, float) : GRADO_CH(1, float);
 #undef GRADO_CH
 #undef GRADO_X
         }
@@ -676,9 +698,11 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
             // kernel, 72 registers / 7 CTAs per SM for batches whose gradient kernel runs after the walkers
             bool occ = (phases & PH_FORWARD) && !g_prof_events && overlap_allowed(p->B, true);
             if (opt(OPT_GRAD2_OCC) >= 0) occ = opt(OPT_GRAD2_OCC) != 0;
-#define GRAD2_O(V_, C_) (occ ? ctcb::k_grad2<V_, C_, 1> : ctcb::k_grad2<V_, C_, 0>)
-#define GRAD2_CH(V_) (ch == 1 ? GRAD2_O(V_, 1) : ch == 2 ? GRAD2_O(V_, 2) : ch == 4 ? GRAD2_O(V_, 4) : ch == 8 ? GRAD2_O(V_, 8) : GRAD2_O(V_, 16))
-            gfn = vec == 4 ? GRAD2_CH(4) : vec == 2 ? GRAD2_CH(2) : GRAD2_CH(1);
+#define GRAD2_O(V_, C_, T_) (occ ? ctcb::k_grad2<V_, C_, 1, T_> : ctcb::k_grad2<V_, C_, 0, T_>)
+#define GRAD2_CH(V_, T_) (ch == 1 ? GRAD2_O(V_, 1, T_) : ch == 2 ? GRAD2_O(V_, 2, T_) : ch == 4 ? GRAD2_O(V_, 4, T_) : \
+                          ch == 8 ? GRAD2_O(V_, 8, T_) : GRAD2_O(V_, 16, T_))
+            if (bf) gfn = vec == 4 ? GRAD2_CH(4, ctcb::bf16) : vec == 2 ? GRAD2_CH(2, ctcb::bf16) : GRAD2_CH(1, ctcb::bf16);
+            else    gfn = vec == 4 ? GRAD2_CH(4, float) : vec == 2 ? GRAD2_CH(2, float) : GRAD2_CH(1, float);
 #undef GRAD2_CH
 #undef GRAD2_O
             gsm = ctcb::grad2_smem_bytes(ch);
@@ -686,9 +710,14 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
         }
         // wide vocabularies with 16-byte aligned rows: the frame block's rows staged in shared memory by bulk copies
         const size_t gsm_staged = ctcb::grad_smem_bytes(lay.Lp, 32 * gch, p->V);
-        if (xq == 0 && vec == 4 && gsm_staged <= 75 * 1024 && opt(OPT_GRAD_STAGED) != 0) {
-            gfn = ch == 1 ? ctcb::k_grad<4, 1, -1> : ch == 2 ? ctcb::k_grad<4, 2, -1> : ch == 4 ? ctcb::k_grad<4, 4, -1> :
-                  ch == 8 ? ctcb::k_grad<4, 8, -1> : ch == 16 ? ctcb::k_grad<4, 16, -1> : ctcb::k_grad<4, 0, -1>;
+        // (bf16 rows: also V * 2 a multiple of 16 bytes and 16-byte aligned rows, logits and gradient)
+        if (xq == 0 && vec == 4 && gsm_staged <= 75 * 1024 && opt(OPT_GRAD_STAGED) != 0 &&
+            rows16(p->logits, p->logits_stride_t, p->logits_row_offsets ? 0 : p->logits_stride_b, p->V, esz) &&
+            rows16(p->grad, p->grad_stride_t, p->grad_stride_b, p->V, esz)) {
+#define GRAD_ST(T_) (ch == 1 ? ctcb::k_grad<4, 1, -1, 0, T_> : ch == 2 ? ctcb::k_grad<4, 2, -1, 0, T_> : ch == 4 ? ctcb::k_grad<4, 4, -1, 0, T_> : \
+                     ch == 8 ? ctcb::k_grad<4, 8, -1, 0, T_> : ch == 16 ? ctcb::k_grad<4, 16, -1, 0, T_> : ctcb::k_grad<4, 0, -1, 0, T_>)
+            gfn = bf ? GRAD_ST(ctcb::bf16) : GRAD_ST(float);
+#undef GRAD_ST
             gsm = gsm_staged;
             gthreads = 256;                      // 8 warps, one frame each
         }
@@ -722,9 +751,13 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
 }  // namespace
 
 int ctcb_loss_grad(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream) {
+    return ctcb_loss_grad_typed(p, CTCB_F32, workspace, workspace_bytes, stream);
+}
+
+int ctcb_loss_grad_typed(const ctcb_problem_t* p, int32_t logits_dtype, void* workspace, size_t workspace_bytes, void* stream) {
     g_launches = 0;
     const bool need_grad = p && p->grad != nullptr;
-    return enqueue(p, workspace, workspace_bytes, stream, need_grad ? (PH_FORWARD | PH_BACKWARD) : PH_FORWARD, need_grad);
+    return enqueue(p, workspace, workspace_bytes, stream, need_grad ? (PH_FORWARD | PH_BACKWARD) : PH_FORWARD, need_grad, logits_dtype);
 }
 
 int ctcb_loss_grad_timed(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream_,
@@ -748,13 +781,22 @@ int ctcb_loss_grad_timed(const ctcb_problem_t* p, void* workspace, size_t worksp
 }
 
 int ctcb_forward(const ctcb_problem_t* p, int32_t keep_for_backward, void* workspace, size_t workspace_bytes, void* stream) {
+    return ctcb_forward_typed(p, CTCB_F32, keep_for_backward, workspace, workspace_bytes, stream);
+}
+
+int ctcb_forward_typed(const ctcb_problem_t* p, int32_t logits_dtype, int32_t keep_for_backward, void* workspace,
+                       size_t workspace_bytes, void* stream) {
     g_launches = 0;
-    return enqueue(p, workspace, workspace_bytes, stream, PH_FORWARD, keep_for_backward != 0);
+    return enqueue(p, workspace, workspace_bytes, stream, PH_FORWARD, keep_for_backward != 0, logits_dtype);
 }
 
 int ctcb_backward(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream) {
+    return ctcb_backward_typed(p, CTCB_F32, workspace, workspace_bytes, stream);
+}
+
+int ctcb_backward_typed(const ctcb_problem_t* p, int32_t logits_dtype, void* workspace, size_t workspace_bytes, void* stream) {
     g_launches = 0;
-    return enqueue(p, workspace, workspace_bytes, stream, PH_BACKWARD, true);
+    return enqueue(p, workspace, workspace_bytes, stream, PH_BACKWARD, true, logits_dtype);
 }
 
 int ctcb_proj_forward(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t keep_for_backward, void* workspace,
@@ -1166,17 +1208,33 @@ int ctcb_greedy_decode(const float* logits, int64_t stride_t, int64_t stride_b, 
 int ctcb_greedy_decode_unk(const float* logits, int64_t stride_t, int64_t stride_b, const void* data_lengths,
                            int32_t data_lengths_dtype, int32_t T, int32_t B, int32_t V, int32_t blank, int32_t unk,
                            int32_t* out_tokens, int32_t* out_lengths, void* stream) {
+    return ctcb_greedy_decode_typed(logits, CTCB_F32, stride_t, stride_b, data_lengths, data_lengths_dtype, T, B, V, blank, unk,
+                                    out_tokens, out_lengths, stream);
+}
+
+int ctcb_greedy_decode_typed(const void* logits, int32_t logits_dtype, int64_t stride_t, int64_t stride_b, const void* data_lengths,
+                             int32_t data_lengths_dtype, int32_t T, int32_t B, int32_t V, int32_t blank, int32_t unk,
+                             int32_t* out_tokens, int32_t* out_lengths, void* stream) {
     if (!logits || !out_tokens || !out_lengths) return fail(CTCB_INVALID_VALUE, "NULL argument");
+    if (logits_dtype != CTCB_F32 && logits_dtype != CTCB_BF16)
+        return fail(CTCB_INVALID_VALUE, "logits dtype %d is neither CTCB_F32 nor CTCB_BF16 (fp16 logits are not supported)", logits_dtype);
     if (T <= 0 || B <= 0 || V <= 0) return fail(CTCB_INVALID_VALUE, "bad shape");
     if (unk >= V) return fail(CTCB_INVALID_VALUE, "unk %d outside the vocabulary (V=%d; -1 = no <unk> rule)", unk, V);
     if (!is_device_ptr(logits) || !is_device_ptr(out_tokens)) return fail(CTCB_INVALID_VALUE, "buffers must be CUDA device memory");
     const size_t smem = 2 * sizeof(int) * (size_t)T;
     if (smem > 200 * 1024) return fail(CTCB_UNSUPPORTED, "T=%d too long for the decode kernel", T);
-    if (smem > 48 * 1024)
-        CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(ctcb::k_greedy_decode), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ctcb::k_greedy_decode<<<B, 256, smem, static_cast<cudaStream_t>(stream)>>>(logits, stride_t, stride_b, data_lengths,
-                                                                                data_lengths_dtype, T, B, V, blank, unk < 0 ? -1 : unk,
-                                                                                out_tokens, out_lengths);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (logits_dtype == CTCB_BF16) {
+        if (smem > 48 * 1024)
+            CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(ctcb::k_greedy_decode<ctcb::bf16>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        ctcb::k_greedy_decode<ctcb::bf16><<<B, 256, smem, st>>>(static_cast<const ctcb::bf16*>(logits), stride_t, stride_b, data_lengths,
+                                                                data_lengths_dtype, T, B, V, blank, unk < 0 ? -1 : unk, out_tokens, out_lengths);
+    } else {
+        if (smem > 48 * 1024)
+            CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(ctcb::k_greedy_decode<float>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        ctcb::k_greedy_decode<float><<<B, 256, smem, st>>>(static_cast<const float*>(logits), stride_t, stride_b, data_lengths,
+                                                           data_lengths_dtype, T, B, V, blank, unk < 0 ? -1 : unk, out_tokens, out_lengths);
+    }
     CUDA_TRY(cudaGetLastError());
     return CTCB_OK;
 }
@@ -1368,8 +1426,10 @@ int ctcb_loss_grad_dlpack(const DLManagedTensor* logits, const DLManagedTensor* 
     const DLTensor& y = labels->dl_tensor;
     if (!dl_cuda(x) || !dl_cuda(y) || !dl_cuda(loss->dl_tensor))
         return fail(CTCB_INVALID_VALUE, "tensors must live on a CUDA device (there is no CPU path)");
-    if (x.ndim != 3 || x.dtype.code != kDLFloat || x.dtype.bits != 32 || x.dtype.lanes != 1)
-        return fail(CTCB_INVALID_VALUE, "logits must be a 3-d float32 tensor");
+    const bool x_f32 = x.dtype.code == kDLFloat && x.dtype.bits == 32, x_bf16 = x.dtype.code == kDLBfloat && x.dtype.bits == 16;
+    if (x.ndim != 3 || !(x_f32 || x_bf16) || x.dtype.lanes != 1)
+        return fail(CTCB_INVALID_VALUE, "logits must be a 3-d float32 or bfloat16 tensor");
+    const int ldt = x_bf16 ? CTCB_BF16 : CTCB_F32;
     if (dl_stride(x, 2) != 1 && x.shape[2] != 1) return fail(CTCB_INVALID_VALUE, "logits need unit stride on the vocabulary axis");
     if (y.ndim != 2) return fail(CTCB_INVALID_VALUE, "labels must be 2-d");
     const bool ntc = (layout_flags & CTCB_LAYOUT_NTC) != 0, tn = (layout_flags & CTCB_LABEL_TN) != 0;
@@ -1408,8 +1468,8 @@ int ctcb_loss_grad_dlpack(const DLManagedTensor* logits, const DLManagedTensor* 
     }
     if (grad) {
         const DLTensor& g = grad->dl_tensor;
-        if (!dl_cuda(g) || g.ndim != 3 || g.dtype.code != kDLFloat || g.dtype.bits != 32)
-            return fail(CTCB_INVALID_VALUE, "grad must be a 3-d float32 CUDA tensor");
+        if (!dl_cuda(g) || g.ndim != 3 || g.dtype.code != x.dtype.code || g.dtype.bits != x.dtype.bits || g.dtype.lanes != 1)
+            return fail(CTCB_INVALID_VALUE, "grad must be a 3-d CUDA tensor of the logits' dtype (%s)", x_bf16 ? "bfloat16" : "float32");
         for (int i = 0; i < 3; ++i)
             if (g.shape[i] != x.shape[i]) return fail(CTCB_INVALID_VALUE, "grad shape differs from logits");
         if (dl_stride(g, 2) != 1 && g.shape[2] != 1) return fail(CTCB_INVALID_VALUE, "grad needs unit stride on the vocabulary axis");
@@ -1422,9 +1482,9 @@ int ctcb_loss_grad_dlpack(const DLManagedTensor* logits, const DLManagedTensor* 
         p.loss_sum = static_cast<double*>(dl_data(s));
     }
     const int phase = (layout_flags >> 8) & 3;   // 0: fused, 1: forward (keep history), 2: backward
-    if (phase == 1) return enqueue(&p, workspace, workspace_bytes, stream, PH_FORWARD, (layout_flags & CTCB_KEEP_FOR_BACKWARD) != 0);
-    if (phase == 2) return enqueue(&p, workspace, workspace_bytes, stream, PH_BACKWARD, true);
-    return enqueue(&p, workspace, workspace_bytes, stream, p.grad ? (PH_FORWARD | PH_BACKWARD) : PH_FORWARD, p.grad != nullptr);
+    if (phase == 1) return enqueue(&p, workspace, workspace_bytes, stream, PH_FORWARD, (layout_flags & CTCB_KEEP_FOR_BACKWARD) != 0, ldt);
+    if (phase == 2) return enqueue(&p, workspace, workspace_bytes, stream, PH_BACKWARD, true, ldt);
+    return enqueue(&p, workspace, workspace_bytes, stream, p.grad ? (PH_FORWARD | PH_BACKWARD) : PH_FORWARD, p.grad != nullptr, ldt);
 }
 
 }  // extern "C"

@@ -23,9 +23,9 @@ namespace ctcb {
 __host__ __device__ inline size_t grad2_smem_bytes(int CH) { return (size_t)4 * 2 * 2 * 32 * CH * 4 + 64 * 8; }
 
 // OCC = 1: 6 CTAs per SM (80 registers); OCC = 0: 7 CTAs per SM (72 registers, a few spilled words)
-template <int VEC, int CH, int OCC>
+template <int VEC, int CH, int OCC, typename LT = float>
 __global__ void __launch_bounds__(128, CH <= 4 ? (OCC ? 6 : 7) : (CH == 8 ? 4 : 2)) k_grad2(GradArgs a) {
-    using V_t = typename VecT<VEC>::type;
+    using V_t = typename LV<LT, VEC>::type;
     constexpr int FPW = kGradFramesPerWarp;               // 2 frames per warp, 4 warps: one frame block per trip
     constexpr int F = CH <= 4 ? FPW : 1;                  // frames in flight per warp
     constexpr int GW = 32 * CH;                           // rank slots per frame
@@ -50,8 +50,8 @@ __global__ void __launch_bounds__(128, CH <= 4 ? (OCC ? 6 : 7) : (CH == 8 ? 4 : 
     __syncthreads();
     auto nan_rows = [&](int t_first, int t_end) {            // a workspace no matching forward call filled: NaN, not a hang
         for (int t = t_first + warp; t < t_end && t < p.T; t += 4) {
-            float* grow = p.grad + b * p.gst_b + (long long)t * p.gst_t;
-            for (int v = lane; v < p.V; v += 32) grow[v] = __int_as_float(0x7fc00000);
+            LT* grow = grad_row<LT>(p, b, t);
+            for (int v = lane; v < p.V; v += 32) stx(grow + v, __int_as_float(0x7fc00000));
         }
     };
     if (!s_ok) { for (int i = 0; i < G; ++i) { const int vi = blockIdx.y * G + i; if (vi < w.NB) nan_rows(vi * kG, vi * kG + kG); } return; }
@@ -168,8 +168,8 @@ __global__ void __launch_bounds__(128, CH <= 4 ? (OCC ? 6 : 7) : (CH == 8 ? 4 : 
         if (blk_live) {
             if (!wait_block(blk)) {
                 for (int t = t_first; t < t_first + kG && t < p.T; ++t) {
-                    float* grow = p.grad + b * p.gst_b + (long long)t * p.gst_t;
-                    for (int v = lane; v < p.V; v += 32) grow[v] = __int_as_float(0x7fc00000);
+                    LT* grow = grad_row<LT>(p, b, t);
+                    for (int v = lane; v < p.V; v += 32) stx(grow + v, __int_as_float(0x7fc00000));
                 }
                 continue;
             }
@@ -197,9 +197,9 @@ __global__ void __launch_bounds__(128, CH <= 4 ? (OCC ? 6 : 7) : (CH == 8 ? 4 : 
                 fr[f] = make_float2(0.0f, 0.0f);
                 if (live[f]) {
                     fr[f] = __ldcg(w.fr + (size_t)b * p.T + tt[f]);
-                    const V_t* xv = reinterpret_cast<const V_t*>(utt_logits(p, b) + (long long)tt[f] * p.st_t);
+                    const V_t* xv = reinterpret_cast<const V_t*>(utt_logits<LT>(p, b) + (long long)tt[f] * p.st_t);
 #pragma unroll
-                    for (int q = 0; q < NXQ; ++q) { const int k = q * 32 + lane; xr[f][q] = k < nvec ? __ldg(xv + k) : vec_fill<VEC>(0.0f); }
+                    for (int q = 0; q < NXQ; ++q) { const int k = q * 32 + lane; xr[f][q] = k < nvec ? __ldg(xv + k) : LV<LT, VEC>::fill(0.0f); }
                     if (CH <= 4) {
                         const int2* A = hA0 + (size_t)(tt[f] - t_first) * pairs + lane;
                         const int2* Bh = hB0 + (size_t)(tt[f] - t_first) * pairs;
@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(128, CH <= 4 ? (OCC ? 6 : 7) : (CH == 8 ? 4 : 
             for (int f = 0; f < F; ++f) {
                 const int t = tt[f];
                 if (t >= p.T) continue;
-                float* grow = p.grad + b * p.gst_b + (long long)t * p.gst_t;
+                LT* grow = grad_row<LT>(p, b, t);
                 if (!live[f]) { zero_row<VEC>(grow, p.V, lane); continue; }
                 float* gbuf = gbuf0 + (size_t)f * GW;                       // gamma of the label states, rank order
                 float* sbuf = gbuf0 + (size_t)(FPW + f) * GW;               // inclusive prefix sums
@@ -245,7 +245,11 @@ __global__ void __launch_bounds__(128, CH <= 4 ? (OCC ? 6 : 7) : (CH == 8 ? 4 : 
                         int2 av[4]; int hb[4], hl[4];
 #pragma unroll
                         for (int k = 0; k < 4; ++k) {
-                            av[k] = __ldcg(A + (c0 + k) * 32); hb[k] = __ldcg(&Bh[ibb[c0 + k]].x); hl[k] = __ldcg(&Bh[ibl[c0 + k]].y);
+                            // lanes past the walkers' 32 * P * NW pairs (8 or 16 chunks cover more) hold no state: a load
+                            // there would read the next frame's row, never written past T_b, and a word with its sign bit
+                            // set wraps to a positive value under the INT_MIN shift of a state beyond the lattice
+                            av[k] = (c0 + k) * 32 + lane < pairs ? __ldcg(A + (c0 + k) * 32) : make_int2(0, 0);
+                            hb[k] = __ldcg(&Bh[ibb[c0 + k]].x); hl[k] = __ldcg(&Bh[ibl[c0 + k]].y);
                         }
 #pragma unroll
                         for (int k = 0; k < 4; ++k) occupancy(av[k], hb[k], hl[k], c0 + k);
@@ -275,7 +279,7 @@ __global__ void __launch_bounds__(128, CH <= 4 ? (OCC ? 6 : 7) : (CH == 8 ? 4 : 
                 for (int q = 0; q < NXQ; ++q) {
                     const int k = q * 32 + lane;
                     if (k < nvec) {
-                        float x[VEC]; vec_get<VEC>(xr[f][q], x);
+                        float x[VEC]; LV<LT, VEC>::get(xr[f][q], x);
                         float y[VEC];
 #pragma unroll
                         for (int j = 0; j < VEC; ++j) {
@@ -285,8 +289,7 @@ __global__ void __launch_bounds__(128, CH <= 4 ? (OCC ? 6 : 7) : (CH == 8 ? 4 : 
                             if (k * VEC + j == p.blank) occ += zb;
                             y[j] = head * (fast_ex2(fmaf(x[j] - fmx, kLog2e, -flz)) - occ * rP);
                         }
-                        V_t o; memcpy(&o, y, sizeof(o));
-                        gv[k] = o;
+                        gv[k] = LV<LT, VEC>::pack(y);
                     }
                 }
                 __syncwarp();

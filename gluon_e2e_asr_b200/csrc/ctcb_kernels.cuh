@@ -26,6 +26,7 @@
 //                        (gamma = alpha*beta'/Z_t), scatter to label columns, fused
 //                        grad = head * (softmax - occupancy) written once, coalesced.
 #pragma once
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -48,9 +49,9 @@ enum : int { DT_I32 = 0, DT_I64 = 1, DT_F32 = 2, DT_F64 = 3 };
 
 struct Problem {          // device view of ctcb_problem_t
     int T, B, V, Lmax, blank, label_pad;
-    const float* logits; long long st_t, st_b;
+    const float* logits; long long st_t, st_b;   // fp32, or bf16 in the kernels instantiated with LT = bf16
     const long long* row_off;        // optional: element offset of utterance b's frame 0 (packed, ragged logits); replaces b*st_b
-    float* grad; long long gst_t, gst_b;
+    float* grad; long long gst_t, gst_b;         // the logits' element type
     const void* labels; int label_dtype; long long lst_b, lst_l;
     const void* data_len; int data_len_dtype;
     const void* label_len; int label_len_dtype;
@@ -108,8 +109,9 @@ __device__ __forceinline__ long long load_as_int(const void* p, int dtype, long 
 }
 
 // frame 0 of utterance b: strided (any T/B strides), or packed -- utterance b's valid frames stored back to back
-__device__ __forceinline__ const float* utt_logits(const Problem& p, int b) {
-    return p.logits + (p.row_off ? __ldg(p.row_off + b) : b * p.st_b);
+template <typename LT = float>
+__device__ __forceinline__ const LT* utt_logits(const Problem& p, int b) {
+    return reinterpret_cast<const LT*>(p.logits) + (p.row_off ? __ldg(p.row_off + b) : b * p.st_b);
 }
 
 __device__ __forceinline__ float fast_ex2(float x) {
@@ -174,6 +176,54 @@ template <> __device__ __forceinline__ float vec_fill<1>(float v) { return v; }
 template <> __device__ __forceinline__ float2 vec_fill<2>(float v) { return make_float2(v, v); }
 template <> __device__ __forceinline__ float4 vec_fill<4>(float v) { return make_float4(v, v, v, v); }
 
+// ---- logits element type (the LT template argument of the kernels that read logits or write the gradient) ----
+// float, or bf16: a bf16 logit is widened to fp32 exactly where it is loaded, everything after that is the fp32 path's
+// arithmetic, and a gradient element is that fp32 value rounded ONCE to bf16 (round to nearest even) where it is stored.
+// Problem::logits / Problem::grad then point at bf16 elements; strides and row offsets stay in elements.
+using bf16 = __nv_bfloat16;
+__device__ __forceinline__ float bf_lo(unsigned u) { return __uint_as_float(u << 16); }          // element 0 of a bf16 pair
+__device__ __forceinline__ float bf_hi(unsigned u) { return __uint_as_float(u & 0xffff0000u); }  // element 1
+__device__ __forceinline__ unsigned bf_rn(float x) { return (unsigned)__bfloat16_as_ushort(__float2bfloat16_rn(x)); }
+__device__ __forceinline__ unsigned bf_pair(float a, float b) { return bf_rn(a) | (bf_rn(b) << 16); }
+
+// VEC consecutive elements of type LT as one load / store: get widens to fp32, pack rounds fp32 values
+template <typename LT, int VEC> struct LV {
+    using type = typename VecT<VEC>::type;
+    static __device__ __forceinline__ void get(const type& v, float (&o)[VEC]) { vec_get<VEC>(v, o); }
+    static __device__ __forceinline__ type fill(float v) { return vec_fill<VEC>(v); }
+    static __device__ __forceinline__ type pack(const float (&y)[VEC]) { type o; memcpy(&o, y, sizeof(o)); return o; }
+};
+template <> struct LV<bf16, 1> {
+    using type = unsigned short;
+    static __device__ __forceinline__ void get(const type& v, float (&o)[1]) { o[0] = bf_lo(v); }
+    static __device__ __forceinline__ type fill(float v) { return (type)bf_rn(v); }
+    static __device__ __forceinline__ type pack(const float (&y)[1]) { return (type)bf_rn(y[0]); }
+};
+template <> struct LV<bf16, 2> {
+    using type = unsigned int;
+    static __device__ __forceinline__ void get(const type& v, float (&o)[2]) { o[0] = bf_lo(v); o[1] = bf_hi(v); }
+    static __device__ __forceinline__ type fill(float v) { return bf_pair(v, v); }
+    static __device__ __forceinline__ type pack(const float (&y)[2]) { return bf_pair(y[0], y[1]); }
+};
+template <> struct LV<bf16, 4> {
+    using type = uint2;
+    static __device__ __forceinline__ void get(const type& v, float (&o)[4]) { o[0] = bf_lo(v.x); o[1] = bf_hi(v.x); o[2] = bf_lo(v.y); o[3] = bf_hi(v.y); }
+    static __device__ __forceinline__ type fill(float v) { return make_uint2(bf_pair(v, v), bf_pair(v, v)); }
+    static __device__ __forceinline__ type pack(const float (&y)[4]) { return make_uint2(bf_pair(y[0], y[1]), bf_pair(y[2], y[3])); }
+};
+// one element: read-only load widened to fp32 / store rounded from fp32
+__device__ __forceinline__ float ldx(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ldx(const bf16* p) { return bf_lo(__ldg(reinterpret_cast<const unsigned short*>(p))); }
+__device__ __forceinline__ void stx(float* p, float v) { *p = v; }
+__device__ __forceinline__ float ldsx(const float* p) { return *p; }             // shared memory
+__device__ __forceinline__ float ldsx(const bf16* p) { return bf_lo(*reinterpret_cast<const unsigned short*>(p)); }
+__device__ __forceinline__ void stx(bf16* p, float v) { *reinterpret_cast<unsigned short*>(p) = (unsigned short)bf_rn(v); }
+// gradient row (b, t) in the element type of the call
+template <typename LT>
+__device__ __forceinline__ LT* grad_row(const Problem& p, int b, int t) {
+    return reinterpret_cast<LT*>(p.grad) + b * p.gst_b + (long long)t * p.gst_t;
+}
+
 __device__ __forceinline__ void st_release_gpu(int* p, int v);
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count);
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes);
@@ -193,9 +243,10 @@ __host__ __device__ inline size_t emit_smem_bytes(int Lp, int staged_V) {
     return staged_V ? emit_slab_bytes(Lp) + (size_t)kG * staged_V * 4 + 64 : (size_t)2 * Lp * sizeof(int);
 }
 
-template <int VEC, int NQ>
+template <int VEC, int NQ, typename LT = float>
 __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspace w) {
-    using V_t = typename VecT<VEC>::type;
+    using V_t = typename LV<LT, VEC>::type;
+    using S_t = typename LV<LT, 4>::type;          // staged rows: four elements per shared-memory load
     // (a programmatic dependent -- the fused projection, ctcb_proj.cuh -- needs nothing from this kernel and may start at once)
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     extern __shared__ __align__(128) int slab[];  // 2*Lp ints: this utterance's labels, metadata scratch
@@ -207,6 +258,7 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
     constexpr int NT = STAGED ? 256 : 128;        // staged rows: 8 warps, one row each
     float* srow = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(slab) + emit_slab_bytes(w.Lp));   // kG rows of V floats
     uint64_t* rbar = reinterpret_cast<uint64_t*>(srow + (size_t)kG * p.V);
+    LT* srowL = reinterpret_cast<LT*>(srow);      // row j at element j * V (bf16 rows fill the first half of the area)
     if (tid == 0) { s_L = p.Lmax; s_rep = 0; s_flags = 0; }
     __syncthreads();
     // operator parameter layer: lengths (trunc + clamp) and labels (trunc + clamp)
@@ -237,8 +289,8 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
         mbar_init(rbar + warp, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         if (t < Tb) {
-            mbar_expect_tx(rbar + warp, (uint32_t)p.V * 4);
-            tma_load_1d(srow + (size_t)warp * p.V, utt_logits(p, b) + (long long)t * p.st_t, (uint32_t)p.V * 4, rbar + warp);
+            mbar_expect_tx(rbar + warp, (uint32_t)p.V * (uint32_t)sizeof(LT));
+            tma_load_1d(srowL + (size_t)warp * p.V, utt_logits<LT>(p, b) + (long long)t * p.st_t, (uint32_t)p.V * (uint32_t)sizeof(LT), rbar + warp);
         }
     }
     __syncwarp();
@@ -262,28 +314,28 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
     const int jbeg = BPC == 4 ? 0 : warp * FPW;
     if (!meta_cta && t0 < Tb) {
         float mxs[kG];
-        const float* rows = utt_logits(p, b) + (long long)t0 * p.st_t;
+        const LT* rows = utt_logits<LT>(p, b) + (long long)t0 * p.st_t;
         if (STAGED) {
             __shared__ float s_mx[kG];
             if (t0 + warp < Tb) {
                 mbar_wait(rbar + warp, 0);
-                const float4* sv = reinterpret_cast<const float4*>(srow + (size_t)warp * p.V);
+                const S_t* sv = reinterpret_cast<const S_t*>(srowL + (size_t)warp * p.V);
                 float m0 = -INFINITY, m1 = -INFINITY;
                 for (int k = lane; k < nvec; k += 64) {
-                    const float4 a = sv[k];
-                    m0 = fmaxf(m0, fmaxf(fmaxf(a.x, a.y), fmaxf(a.z, a.w)));
-                    if (k + 32 < nvec) { const float4 c = sv[k + 32]; m1 = fmaxf(m1, fmaxf(fmaxf(c.x, c.y), fmaxf(c.z, c.w))); }
+                    float a[4]; LV<LT, 4>::get(sv[k], a);
+                    m0 = fmaxf(m0, fmaxf(fmaxf(a[0], a[1]), fmaxf(a[2], a[3])));
+                    if (k + 32 < nvec) { float c[4]; LV<LT, 4>::get(sv[k + 32], c); m1 = fmaxf(m1, fmaxf(fmaxf(c[0], c[1]), fmaxf(c[2], c[3]))); }
                 }
                 const float mx = warp_max(fmaxf(m0, m1));
                 float s0 = 0.0f, s1 = 0.0f;
                 for (int k = lane; k < nvec; k += 64) {
-                    const float4 a = sv[k];
-                    s0 += fast_ex2((a.x - mx) * kLog2e) + fast_ex2((a.y - mx) * kLog2e);
-                    s1 += fast_ex2((a.z - mx) * kLog2e) + fast_ex2((a.w - mx) * kLog2e);
+                    float a[4]; LV<LT, 4>::get(sv[k], a);
+                    s0 += fast_ex2((a[0] - mx) * kLog2e) + fast_ex2((a[1] - mx) * kLog2e);
+                    s1 += fast_ex2((a[2] - mx) * kLog2e) + fast_ex2((a[3] - mx) * kLog2e);
                     if (k + 32 < nvec) {
-                        const float4 c = sv[k + 32];
-                        s0 += fast_ex2((c.x - mx) * kLog2e) + fast_ex2((c.y - mx) * kLog2e);
-                        s1 += fast_ex2((c.z - mx) * kLog2e) + fast_ex2((c.w - mx) * kLog2e);
+                        float c[4]; LV<LT, 4>::get(sv[k + 32], c);
+                        s0 += fast_ex2((c[0] - mx) * kLog2e) + fast_ex2((c[1] - mx) * kLog2e);
+                        s1 += fast_ex2((c[2] - mx) * kLog2e) + fast_ex2((c[3] - mx) * kLog2e);
                     }
                 }
                 const float sum = warp_sum(s0 + s1);
@@ -301,7 +353,7 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
                 double y[kG];
 #pragma unroll
                 for (int j = 0; j < kG; ++j) {
-                    const float l2 = (srow[(size_t)j * p.V + v] - s_mx[j]) * kLog2e;
+                    const float l2 = (ldsx(srowL + (size_t)j * p.V + v) - s_mx[j]) * kLog2e;
                     floored |= j < nval && l2 < kMinLog2;
                     y[j] = j < nval ? (double)fast_ex2(fmaxf(l2, kMinLog2)) : 0.0;
                 }
@@ -320,21 +372,21 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
 #pragma unroll
                 for (int f = 0; f < F; ++f) {                   // every load of F frames in flight
                     const bool valid = t0 + jf + f < Tb;
-                    const float* row = rows + (jf + f) * p.st_t;
+                    const LT* row = rows + (jf + f) * p.st_t;
                     const V_t* rowv = reinterpret_cast<const V_t*>(row);
 #pragma unroll
                     for (int q = 0; q < NQ1; ++q) {
                         const int k = q * 32 + lane;
-                        x[f][q] = (valid && k < nvec) ? __ldg(rowv + k) : vec_fill<VEC>(-INFINITY);
+                        x[f][q] = (valid && k < nvec) ? __ldg(rowv + k) : LV<LT, VEC>::fill(-INFINITY);
                     }
-                    xt[f] = (VEC > 1 && valid && nvec * VEC + lane < p.V) ? __ldg(row + nvec * VEC + lane) : -INFINITY;
+                    xt[f] = (VEC > 1 && valid && nvec * VEC + lane < p.V) ? ldx(row + nvec * VEC + lane) : -INFINITY;
                 }
                 float mx[F], sum[F];
 #pragma unroll
                 for (int f = 0; f < F; ++f) {
                     float m = xt[f];
 #pragma unroll
-                    for (int q = 0; q < NQ1; ++q) { float e[VEC]; vec_get<VEC>(x[f][q], e);
+                    for (int q = 0; q < NQ1; ++q) { float e[VEC]; LV<LT, VEC>::get(x[f][q], e);
 #pragma unroll
                         for (int i = 0; i < VEC; ++i) m = fmaxf(m, e[i]); }
                     mx[f] = m;
@@ -347,7 +399,7 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
                 for (int f = 0; f < F; ++f) {
                     float sacc = fast_ex2((xt[f] - mx[f]) * kLog2e);          // ex2(-inf) = 0 for absent elements
 #pragma unroll
-                    for (int q = 0; q < NQ1; ++q) { float e[VEC]; vec_get<VEC>(x[f][q], e);
+                    for (int q = 0; q < NQ1; ++q) { float e[VEC]; LV<LT, VEC>::get(x[f][q], e);
 #pragma unroll
                         for (int i = 0; i < VEC; ++i) sacc += fast_ex2((e[i] - mx[f]) * kLog2e); }
                     sum[f] = sacc;
@@ -371,7 +423,7 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
 #pragma unroll
                         for (int f = 0; f < F; ++f) {
                             const bool valid = t0 + jf + f < Tb;
-                            const float xv = valid ? __ldg(rows + (jf + f) * p.st_t + v) : 0.0f;
+                            const float xv = valid ? ldx(rows + (jf + f) * p.st_t + v) : 0.0f;
                             if (valid && (xv - mx[f]) * kLog2e < kMinLog2 && p.status) atomicOr(p.status + b, UTT_WIDE_LOGITS);
                             eblk[(size_t)col * kEC + jf + f] = valid ? (double)fast_ex2(fmaxf((xv - mx[f]) * kLog2e, kMinLog2)) : 0.0;
                         }
@@ -384,23 +436,23 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
                 const int t = t0 + j;
                 mxs[j] = 0.0f;
                 if (t >= Tb) continue;
-                const float* row = rows + j * p.st_t;
+                const LT* row = rows + j * p.st_t;
                 const V_t* rowv = reinterpret_cast<const V_t*>(row);
                 float mx = -INFINITY;
                 for (int k = lane; k < nvec; k += 32) {
-                    float x[VEC]; vec_get<VEC>(__ldg(rowv + k), x);
+                    float x[VEC]; LV<LT, VEC>::get(__ldg(rowv + k), x);
 #pragma unroll
                     for (int i = 0; i < VEC; ++i) mx = fmaxf(mx, x[i]);
                 }
-                for (int v = nvec * VEC + lane; v < p.V; v += 32) mx = fmaxf(mx, __ldg(row + v));
+                for (int v = nvec * VEC + lane; v < p.V; v += 32) mx = fmaxf(mx, ldx(row + v));
                 mx = warp_max(mx);
                 float sum = 0.0f;
                 for (int k = lane; k < nvec; k += 32) {          // second pass hits L1/L2
-                    float x[VEC]; vec_get<VEC>(__ldg(rowv + k), x);
+                    float x[VEC]; LV<LT, VEC>::get(__ldg(rowv + k), x);
 #pragma unroll
                     for (int i = 0; i < VEC; ++i) sum += fast_ex2((x[i] - mx) * kLog2e);
                 }
-                for (int v = nvec * VEC + lane; v < p.V; v += 32) sum += fast_ex2((__ldg(row + v) - mx) * kLog2e);
+                for (int v = nvec * VEC + lane; v < p.V; v += 32) sum += fast_ex2((ldx(row + v) - mx) * kLog2e);
                 sum = warp_sum(sum);
                 if (lane == 0) w.fr[(size_t)b * p.T + t] = make_float2(mx, log2f(sum));
                 mxs[j] = mx;
@@ -412,7 +464,7 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
             const int v = w.dense ? col : (col == 0 ? p.blank : slab[col - 1]);
             float xv[kG];
 #pragma unroll
-            for (int j = 0; j < kG; ++j) xv[j] = t0 + j < Tb ? __ldg(rows + j * p.st_t + v) : 0.0f;
+            for (int j = 0; j < kG; ++j) xv[j] = t0 + j < Tb ? ldx(rows + j * p.st_t + v) : 0.0f;
             double2* dst = reinterpret_cast<double2*>(eblk + (size_t)col * kEC);
 #pragma unroll
             for (int j = 0; j < kG; j += 2) {
@@ -636,7 +688,7 @@ __host__ __device__ inline size_t walk_smem_bytes(int W, int NW, int stages, int
            (size_t)NW * sizeof(int) + 64 + (fused_Lp ? 16 + kFusedProducers * 64 + (size_t)fused_Lp * sizeof(int) : 0);
 }
 
-template <int P, int NW, int DIR, bool HIST, bool FUSED>
+template <int P, int NW, int DIR, bool HIST, bool FUSED, typename LT = float>
 __device__ __forceinline__ void walk_dir(const WalkArgs& a, unsigned char* smem_raw, int Tb, int Lb, int uflags) {
     constexpr int PW = 32 * P;
     constexpr unsigned FULL = 0xffffffffu;
@@ -685,14 +737,14 @@ __device__ __forceinline__ void walk_dir(const WalkArgs& a, unsigned char* smem_
         const int q = warp - NW, V = p.V;
         const int fj = lane >> 2, qk = lane & 3;                       // frame of the block, quarter of the row
         const int cpl = (V + 3) >> 2, col0 = qk * cpl;                 // this lane's columns [col0, col0 + cpl) below V
-        const float* base = utt_logits(p, b);
+        const LT* base = utt_logits<LT>(p, b);
         const float kMinProb = 7.888609052210118e-31f;                 // 2^kMinLog2
         auto load_blk = [&](int n, float (&x)[CPL]) {
             const int t = (DIR ? NQ - 1 - n : n) * kG + fj;
-            const float* row = base + (long long)t * p.st_t + col0;
+            const LT* row = base + (long long)t * p.st_t + col0;
             const bool valid = t < Tb;
 #pragma unroll
-            for (int i = 0; i < CPL; ++i) x[i] = (valid && i < cpl && col0 + i < V) ? __ldg(row + i) : -INFINITY;
+            for (int i = 0; i < CPL; ++i) x[i] = (valid && i < cpl && col0 + i < V) ? ldx(row + i) : -INFINITY;
         };
         float cur[CPL], nxt[CPL];
         double ls = 0.0;
@@ -1201,7 +1253,7 @@ __device__ __forceinline__ void walk_dir(const WalkArgs& a, unsigned char* smem_
     }
 }
 
-template <int P, int NW, bool HIST, bool FUSED>
+template <int P, int NW, bool HIST, bool FUSED, typename LT = float>
 __global__ void __launch_bounds__((NW + (FUSED ? kFusedProducers + 1 : 1)) * 32) k_walk(WalkArgs a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     if (a.pdl_wait) asm volatile("griddepcontrol.wait;" ::: "memory");   // everything enqueued before this kernel is complete and visible
@@ -1295,8 +1347,8 @@ __global__ void __launch_bounds__((NW + (FUSED ? kFusedProducers + 1 : 1)) * 32)
         }
     }
     if (flags & UTT_INFEASIBLE) return;
-    if (blockIdx.y == 0) walk_dir<P, NW, 0, HIST, true>(a, smem_raw, Tb, L, flags);
-    else                 walk_dir<P, NW, 1, HIST, true>(a, smem_raw, Tb, L, flags);
+    if (blockIdx.y == 0) walk_dir<P, NW, 0, HIST, true, LT>(a, smem_raw, Tb, L, flags);
+    else                 walk_dir<P, NW, 1, HIST, true, LT>(a, smem_raw, Tb, L, flags);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1403,14 +1455,14 @@ __global__ void __launch_bounds__(32) k_mailbox_exchange(const MailboxDev* m, do
 // ---------------------------------------------------------------------------------------
 struct GradArgs { Problem p; Workspace w; };
 
-template <int VEC>
-__device__ __forceinline__ void zero_row(float* row, int V, int lane) {
-    using V_t = typename VecT<VEC>::type;
+template <int VEC, typename LT>
+__device__ __forceinline__ void zero_row(LT* row, int V, int lane) {
+    using V_t = typename LV<LT, VEC>::type;
     const int nvec = V / VEC;
     V_t z; memset(&z, 0, sizeof(z));
     V_t* rv = reinterpret_cast<V_t*>(row);
     for (int k = lane; k < nvec; k += 32) rv[k] = z;
-    for (int v = nvec * VEC + lane; v < V; v += 32) row[v] = 0.0f;
+    for (int v = nvec * VEC + lane; v < V; v += 32) stx(row + v, 0.0f);
 }
 
 constexpr int kNoState = INT_MIN / 2;
@@ -1443,9 +1495,9 @@ __host__ __device__ inline size_t grad_smem_bytes(int Lp, int pairs_cap, int sta
 // OCC = 1: registers capped at 64 (8 CTAs per SM instead of 7, a few spilled words) for batches
 // that run after the walkers: measured -14 % at cfg5, but +5 % on the overlapped cfg2 step, where
 // the kernel shares the GPU with the walkers and its tail is what counts -- hence a variant.
-template <int VEC, int CH, int XQ, int OCC = 0>
+template <int VEC, int CH, int XQ, int OCC = 0, typename LT = float>
 __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3) : ((CH == 0 || CH == 8) ? 5 : (CH <= 4 ? (OCC ? 8 : 1) : 3))) k_grad(GradArgs a) {
-    using V_t = typename VecT<VEC>::type;
+    using V_t = typename LV<LT, VEC>::type;
     constexpr int NCH = CH > 0 ? CH : 1, NXQ = XQ > 0 ? XQ : 1;
     // staged rows: 8 warps, one frame each (the compute phase is latency-bound: twice the warps per SM)
     constexpr int FPW = XQ < 0 ? 1 : kGradFramesPerWarp, NT = XQ < 0 ? 256 : 128;
@@ -1487,8 +1539,8 @@ __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3
         for (int j = warp; j < kG; j += (XQ < 0 ? 8 : 4)) {
             const int t = blockIdx.y * kG + j;
             if (t < p.T) {
-                float* grow = p.grad + b * p.gst_b + (long long)t * p.gst_t;
-                for (int v = lane; v < p.V; v += 32) grow[v] = __int_as_float(0x7fc00000);
+                LT* grow = grad_row<LT>(p, b, t);
+                for (int v = lane; v < p.V; v += 32) stx(grow + v, __int_as_float(0x7fc00000));
             }
         }
         return;
@@ -1516,8 +1568,10 @@ __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3
         for (int f = 0; f < FPW; ++f) {
             const int j = warp * FPW + f, t = t_first + j;
             if (t < Tb) {
-                mbar_expect_tx(rbar + j, (uint32_t)p.V * 4);
-                tma_load_1d(srow + (size_t)j * p.V, utt_logits(p, b) + (long long)t * p.st_t, (uint32_t)p.V * 4, rbar + j);
+                // a bf16 row lands in the upper half of its fp32 slot and is widened in place (below)
+                mbar_expect_tx(rbar + j, (uint32_t)p.V * (uint32_t)sizeof(LT));
+                tma_load_1d(reinterpret_cast<LT*>(srow + (size_t)j * p.V) + (sizeof(LT) == 4 ? 0 : p.V),
+                            utt_logits<LT>(p, b) + (long long)t * p.st_t, (uint32_t)p.V * (uint32_t)sizeof(LT), rbar + j);
             }
         }
     }
@@ -1553,8 +1607,8 @@ __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3
         for (int j = warp; j < kG; j += NT / 32) {
             const int t = t_first + j;
             if (t < p.T) {
-                float* grow = p.grad + b * p.gst_b + (long long)t * p.gst_t;
-                for (int v = lane; v < p.V; v += 32) grow[v] = __int_as_float(0x7fc00000);
+                LT* grow = grad_row<LT>(p, b, t);
+                for (int v = lane; v < p.V; v += 32) stx(grow + v, __int_as_float(0x7fc00000));
             }
         }
         return;
@@ -1636,11 +1690,11 @@ __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3
             fr[f] = make_float2(0.0f, 0.0f);
             if (live[f]) {
                 fr[f] = __ldcg(w.fr + (size_t)b * p.T + tt[f]);
-                const float* xrow = utt_logits(p, b) + (long long)tt[f] * p.st_t;
+                const LT* xrow = utt_logits<LT>(p, b) + (long long)tt[f] * p.st_t;
                 if (XQ > 0) {
                     const V_t* xv = reinterpret_cast<const V_t*>(xrow);
 #pragma unroll
-                    for (int q = 0; q < NXQ; ++q) { const int k = q * 32 + lane; xr[f][q] = k < nvec ? __ldg(xv + k) : vec_fill<VEC>(0.0f); }
+                    for (int q = 0; q < NXQ; ++q) { const int k = q * 32 + lane; xr[f][q] = k < nvec ? __ldg(xv + k) : LV<LT, VEC>::fill(0.0f); }
                 }
                 if (CH > 0) {
                     const int2* A = hA0 + (size_t)(tt[f] - t_first) * pairs + lane;
@@ -1660,9 +1714,9 @@ __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3
         for (int f = 0; f < F; ++f) {
             const int t = tt[f];
             if (t >= p.T) continue;
-            float* grow = p.grad + b * p.gst_b + (long long)t * p.gst_t;
+            LT* grow = grad_row<LT>(p, b, t);
             if (!live[f]) { zero_row<VEC>(grow, p.V, lane); continue; }
-            const float* xrow = utt_logits(p, b) + (long long)t * p.st_t;
+            const LT* xrow = utt_logits<LT>(p, b) + (long long)t * p.st_t;
             float* gbuf = gbuf0 + (size_t)(r * F + f) * GW;
             float zb = 0.0f, zl = 0.0f;
             if (CH > 0) {
@@ -1722,7 +1776,7 @@ __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3
                 for (int q = 0; q < NXQ; ++q) {
                     const int k = q * 32 + lane;
                     if (k < nvec) {
-                        float x[VEC]; vec_get<VEC>(xr[f][q], x);
+                        float x[VEC]; LV<LT, VEC>::get(xr[f][q], x);
                         float y[VEC];
 #pragma unroll
                         for (int j = 0; j < VEC; ++j) {
@@ -1730,8 +1784,7 @@ __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3
                             if (k * VEC + j == p.blank) y[j] -= gblank;
                             y[j] *= head;
                         }
-                        V_t o; memcpy(&o, y, sizeof(o));
-                        gv[k] = o;
+                        gv[k] = LV<LT, VEC>::pack(y);
                     }
                 }
             } else if (STAGED) {
@@ -1739,13 +1792,29 @@ __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3
                 float* sr = srow + (size_t)(warp * FPW + r * F + f) * p.V;
                 mbar_wait(rbar + warp * FPW + r * F + f, 0);
                 float4* sv = reinterpret_cast<float4*>(sr);
-                for (int k = lane; k < nvec; k += 32) {
-                    float4 v = sv[k];
-                    v.x = head * fast_ex2(fmaf(v.x - fmx, kLog2e, -flz));
-                    v.y = head * fast_ex2(fmaf(v.y - fmx, kLog2e, -flz));
-                    v.z = head * fast_ex2(fmaf(v.z - fmx, kLog2e, -flz));
-                    v.w = head * fast_ex2(fmaf(v.w - fmx, kLog2e, -flz));
-                    sv[k] = v;
+                if constexpr (sizeof(LT) == 4) {
+                    for (int k = lane; k < nvec; k += 32) {
+                        float4 v = sv[k];
+                        v.x = head * fast_ex2(fmaf(v.x - fmx, kLog2e, -flz));
+                        v.y = head * fast_ex2(fmaf(v.y - fmx, kLog2e, -flz));
+                        v.z = head * fast_ex2(fmaf(v.z - fmx, kLog2e, -flz));
+                        v.w = head * fast_ex2(fmaf(v.w - fmx, kLog2e, -flz));
+                        sv[k] = v;
+                    }
+                } else {
+                    // bf16 row in the upper half of the slot, widened in place to the fp32 row head * y: the fp32 elements
+                    // 4k..4k+3 overwrite bf16 elements <= 4k+3 only, which this step (all loads before the warp's stores)
+                    // or an earlier one has read.  From here to the packing below the row is the fp32 path's, bit for bit.
+                    const uint2* sb = reinterpret_cast<const uint2*>(reinterpret_cast<const LT*>(sr) + p.V);
+                    for (int k0 = 0; k0 < nvec; k0 += 32) {
+                        const int k = k0 + lane;
+                        float x[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+                        if (k < nvec) LV<LT, 4>::get(sb[k], x);
+                        __syncwarp();
+                        if (k < nvec)
+                            sv[k] = make_float4(head * fast_ex2(fmaf(x[0] - fmx, kLog2e, -flz)), head * fast_ex2(fmaf(x[1] - fmx, kLog2e, -flz)),
+                                                head * fast_ex2(fmaf(x[2] - fmx, kLog2e, -flz)), head * fast_ex2(fmaf(x[3] - fmx, kLog2e, -flz)));
+                    }
                 }
                 __syncwarp();
                 // sr[v] now holds head * y_v: the corrections subtract head * occupancy.  Blank first, then
@@ -1761,7 +1830,20 @@ __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3
                     sr[e.x] = fmaf(-hz, occ, sr[e.x]);
                 }
                 __syncwarp();
-                if (lane == 0) tma_store_1d(grow, sr, (uint32_t)p.V * 4);
+                if constexpr (sizeof(LT) != 4) {
+                    // every element rounded once into the lower half: bf16 elements 4k..4k+3 overwrite fp32 elements 2k, 2k+1,
+                    // read in this step or an earlier one
+                    uint2* so = reinterpret_cast<uint2*>(sr);
+                    for (int k0 = 0; k0 < nvec; k0 += 32) {
+                        const int k = k0 + lane;
+                        float4 v = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+                        if (k < nvec) v = sv[k];
+                        __syncwarp();
+                        if (k < nvec) so[k] = make_uint2(bf_pair(v.x, v.y), bf_pair(v.z, v.w));
+                    }
+                    __syncwarp();
+                }
+                if (lane == 0) tma_store_1d(grow, sr, (uint32_t)p.V * (uint32_t)sizeof(LT));
                 continue;
             } else {
                 // wide rows: four vector loads in flight per lane; the blank column is fixed afterwards
@@ -1769,31 +1851,30 @@ __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3
                 for (int k0 = lane; k0 < nvec; k0 += 128) {
                     V_t xq[4];
 #pragma unroll
-                    for (int u = 0; u < 4; ++u) { const int k = k0 + 32 * u; xq[u] = k < nvec ? __ldg(xv + k) : vec_fill<VEC>(0.0f); }
+                    for (int u = 0; u < 4; ++u) { const int k = k0 + 32 * u; xq[u] = k < nvec ? __ldg(xv + k) : LV<LT, VEC>::fill(0.0f); }
 #pragma unroll
                     for (int u = 0; u < 4; ++u) {
                         const int k = k0 + 32 * u;
                         if (k < nvec) {
-                            float x[VEC]; vec_get<VEC>(xq[u], x);
+                            float x[VEC]; LV<LT, VEC>::get(xq[u], x);
                             float y[VEC];
 #pragma unroll
                             for (int j = 0; j < VEC; ++j) y[j] = head * fast_ex2(fmaf(x[j] - fmx, kLog2e, -flz));
-                            V_t o; memcpy(&o, y, sizeof(o));
-                            gv[k] = o;
+                            gv[k] = LV<LT, VEC>::pack(y);
                         }
                     }
                 }
             }
             for (int v = nvec * VEC + lane; v < p.V; v += 32) {
-                float y = fast_ex2(fmaf(__ldg(xrow + v) - fmx, kLog2e, -flz));
+                float y = fast_ex2(fmaf(ldx(xrow + v) - fmx, kLog2e, -flz));
                 if (v == p.blank) y -= gblank;
-                grow[v] = y * head;
+                stx(grow + v, y * head);
             }
             __syncwarp();
             if (XQ == 0) {
                 if (lane == 0 && p.blank < nvec * VEC) {
-                    const float y = fast_ex2(fmaf(__ldg(xrow + p.blank) - fmx, kLog2e, -flz));
-                    grow[p.blank] = head * (y - gblank);
+                    const float y = fast_ex2(fmaf(ldx(xrow + p.blank) - fmx, kLog2e, -flz));
+                    stx(grow + p.blank, head * (y - gblank));
                 }
                 __syncwarp();
             }
@@ -1805,8 +1886,8 @@ __global__ void __launch_bounds__(XQ < 0 ? 256 : 128, XQ < 0 ? (CH == 16 ? 2 : 3
                 float occ = 0.0f;
                 for (int k = e.y; k < end; ++k) occ += gbuf[k];
                 if (e.x == p.blank) occ += zb;                       // invalid input (label == blank): keep both
-                const float y = fast_ex2(fmaf(__ldg(xrow + e.x) - fmx, kLog2e, -flz));
-                grow[e.x] = head * (y - occ * rZ);
+                const float y = fast_ex2(fmaf(ldx(xrow + e.x) - fmx, kLog2e, -flz));
+                stx(grow + e.x, head * (y - occ * rZ));
             }
         }
     }
@@ -1848,7 +1929,8 @@ __device__ __forceinline__ void top2_push(Top2& t, float v, int i) {
     else if (better(v, i, t.v2, t.i2)) { t.v2 = v; t.i2 = i; }
 }
 #ifndef CTCB_NO_PLAIN_KERNELS   // non-template kernels: defined in ctcb.cu's translation unit only
-__global__ void __launch_bounds__(256) k_greedy_decode(const float* logits, long long st_t, long long st_b,
+template <typename LT = float>
+__global__ void __launch_bounds__(256) k_greedy_decode(const LT* logits, long long st_t, long long st_b,
                                                        const void* data_len, int dl_dtype, int T, int B, int V,
                                                        int blank, int unk, int* out_tokens, int* out_len) {
     extern __shared__ int path[];                 // T ints: the raw best symbol; T more: the symbol after the <unk> rule
@@ -1858,9 +1940,9 @@ __global__ void __launch_bounds__(256) k_greedy_decode(const float* logits, long
     const int n = (int)(n64 < 0 ? 0 : (n64 > T ? T : n64));
     int* sym = path + T;
     for (int t = warp; t < n; t += 8) {
-        const float* row = logits + b * st_b + t * st_t;
+        const LT* row = logits + b * st_b + t * st_t;
         Top2 tp{-INFINITY, 0x7fffffff, -INFINITY, 0x7fffffff};
-        for (int v = lane; v < V; v += 32) top2_push(tp, __ldg(row + v), v);
+        for (int v = lane; v < V; v += 32) top2_push(tp, ldx(row + v), v);
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
             const float ov1 = __shfl_xor_sync(0xffffffffu, tp.v1, o), ov2 = __shfl_xor_sync(0xffffffffu, tp.v2, o);

@@ -21,6 +21,8 @@ from . import _lib
 __all__ = ["ctc_loss", "CTCLoss", "ctc_loss_and_grad", "greedy_decode", "workspace_bytes"]
 
 _DT = {torch.int32: _lib.DT_I32, torch.int64: _lib.DT_I64, torch.float32: _lib.DT_F32, torch.float64: _lib.DT_F64}
+# logits element types: float32, and bfloat16 (a mixed-precision model's logits; loss fp32, gradient bf16 -- include/ctcb.h)
+_DT_LOGITS = {torch.float32: _lib.DT_F32, torch.bfloat16: _lib.DT_BF16}
 _HANDOFF = os.environ.get("CTCB_HANDOFF", "dlpack")
 
 _PyCapsule_GetPointer = ctypes.pythonapi.PyCapsule_GetPointer
@@ -82,8 +84,9 @@ def _check_data(data):
         raise RuntimeError("gluon_e2e_asr_b200.ctc_loss has no CPU path: data must be a CUDA tensor")
     if data.dim() != 3:
         raise ValueError("data must be 3-d, got shape %s" % (tuple(data.shape),))
-    if data.dtype != torch.float32:
-        raise TypeError("data must be float32 (the reference's logits dtype), got %s" % data.dtype)
+    if data.dtype not in _DT_LOGITS:
+        raise TypeError("data must be float32 (the reference's logits dtype) or bfloat16, got %s "
+                        "(float16 logits are not supported: cast them to bfloat16 or float32)" % data.dtype)
     if data.shape[2] > 1 and data.stride(2) != 1:
         data = data.contiguous()
     return data
@@ -94,6 +97,7 @@ class _Call:
 
     def __init__(self, data, label, data_lengths, label_lengths, blank_last, ntc, tn):
         self.data = data
+        self.ldt = _DT_LOGITS[data.dtype]          # element type of the logits and of the gradient
         self.ntc, self.tn, self.blank_last = ntc, tn, blank_last
         dev = data.device
         self.label = _as_index_tensor(label, dev, "label")
@@ -169,11 +173,11 @@ class _Call:
             else:
                 p = self.problem(loss, grad, head, loss_sum, status)
                 if phase == _lib.PHASE_FORWARD:
-                    rc = lib.ctcb_forward(ctypes.byref(p), 1 if keep else 0, ws.data_ptr(), ws.numel(), stream)
+                    rc = lib.ctcb_forward_typed(ctypes.byref(p), self.ldt, 1 if keep else 0, ws.data_ptr(), ws.numel(), stream)
                 elif phase == _lib.PHASE_BACKWARD:
-                    rc = lib.ctcb_backward(ctypes.byref(p), ws.data_ptr(), ws.numel(), stream)
+                    rc = lib.ctcb_backward_typed(ctypes.byref(p), self.ldt, ws.data_ptr(), ws.numel(), stream)
                 else:
-                    rc = lib.ctcb_loss_grad(ctypes.byref(p), ws.data_ptr(), ws.numel(), stream)
+                    rc = lib.ctcb_loss_grad_typed(ctypes.byref(p), self.ldt, ws.data_ptr(), ws.numel(), stream)
         _lib.check(rc)
 
 
@@ -185,7 +189,8 @@ def _alloc_ws(call, need_grad):
 # Forward of a differentiable call: small problems run the fused forward+gradient once (the
 # gradient is stored like MXNet's operator stores it, SURVEY 8a row a8) and Backward only scales
 # it by the head gradient; large ones keep the alpha/beta history and write head*G once in
-# Backward, which saves a pass over the (T,B,V) gradient.
+# Backward, which saves a pass over the (T,B,V) gradient.  bfloat16 logits always take the second
+# branch: scaling a stored bf16 gradient would round every element twice.
 _FUSE_IN_FORWARD_MAX_ELEMS = 8 * 1024 * 1024
 
 
@@ -196,7 +201,7 @@ class _CtcLossFn(torch.autograd.Function):
         need = ctx.needs_input_grad[0]
         loss = torch.empty((call.B,), dtype=torch.float32, device=data.device)
         ctx.call = call
-        if need and data.numel() <= _FUSE_IN_FORWARD_MAX_ELEMS:
+        if need and data.dtype == torch.float32 and data.numel() <= _FUSE_IN_FORWARD_MAX_ELEMS:
             grad = torch.empty_like(data)           # same layout as the logits: no swapaxes backward
             call.run(_lib.PHASE_FUSED, _cached_ws(call, data.device), loss, grad=grad)
             ctx.grad, ctx.ws = grad, None
@@ -238,7 +243,8 @@ def ctc_loss(data, label, data_lengths=None, label_lengths=None, use_data_length
              use_label_lengths=False, blank_label="first"):
     """``mx.nd.contrib.ctc_loss`` as called at scripts/swbd/loss.py:134-139.
 
-    data (T, B, V) float32 CUDA logits (softmax is inside); label (B, Lmax) any numeric dtype,
+    data (T, B, V) float32 or bfloat16 CUDA logits (softmax is inside; bf16: fp32 loss, bf16 gradient);
+    label (B, Lmax) any numeric dtype,
     truncated to int; lengths (B,) used only when the matching ``use_*`` flag is set
     (otherwise T, resp. the first padding value: 0 for blank_label='first', -1 for 'last').
     Returns the per-utterance negative log-likelihood (B,); differentiable w.r.t. ``data``.
@@ -282,9 +288,12 @@ def ctc_loss_and_grad(pred, label, pred_lengths=None, label_lengths=None, head_g
 
     ``head_grad`` (B,) is the upstream gradient of each loss (``1/B`` for the reference's
     ``.mean().backward()``, train_ctc_ce.py:363-366); ``loss_sum`` an optional float64 device
-    scalar accumulated in place.  The workspace is cached per (device, stream, shape).
+    scalar accumulated in place.  The workspace is cached per (device, stream, shape).  bfloat16
+    ``pred``: the loss is float32 and the gradient bfloat16 (``out_grad`` must then be bfloat16).
     """
     pred = _check_data(pred)
+    if out_grad is not None and out_grad.dtype != pred.dtype:
+        raise TypeError("out_grad must have the logits' dtype %s, got %s" % (pred.dtype, out_grad.dtype))
     call = _Call(pred, label, pred_lengths, label_lengths, _blank_last(blank_label),
                  layout == "NTC", label_layout == "TN")
     dev = pred.device
@@ -302,7 +311,8 @@ def greedy_decode(pred, pred_lengths=None, blank=0, layout="NTC", unk=None):
     """Greedy CTC decode of train_ctc_ce.py:149-160: argmax over V, collapse repeats, drop
     blank.  ``unk`` (the index of ``<unk>``): decode_ctc.py:120-140's rule -- a frame whose best symbol
     is ``unk`` takes its second best; the repeat test still compares with the raw best symbol of the
-    previous frame.  Returns (tokens (B,T) int32 -- prefix valid, lengths (B,) int32) on pred's device."""
+    previous frame.  ``pred`` float32 or bfloat16.  Returns (tokens (B,T) int32 -- prefix valid, lengths (B,) int32) on
+    pred's device."""
     pred = _check_data(pred)
     ta, ba = (1, 0) if layout == "NTC" else (0, 1)
     T, B, V = pred.shape[ta], pred.shape[ba], pred.shape[2]
@@ -313,7 +323,7 @@ def greedy_decode(pred, pred_lengths=None, blank=0, layout="NTC", unk=None):
     lens = torch.empty((B,), dtype=torch.int32, device=pred.device)
     lib = _lib.load()
     with _on_device(pred.device):
-        rc = lib.ctcb_greedy_decode_unk(pred.data_ptr(), pred.stride(ta), pred.stride(ba),
+        rc = lib.ctcb_greedy_decode_typed(pred.data_ptr(), _DT_LOGITS[pred.dtype], pred.stride(ta), pred.stride(ba),
                                         pl.data_ptr() if pl is not None else None,
                                         _DT[pl.dtype] if pl is not None else 0, T, B, V, blank,
                                         -1 if unk is None else int(unk),

@@ -131,6 +131,7 @@ class _MetaLogits:
     def __init__(self, t, dev):
         self._t, self.device = t, dev
         self.shape = t.shape
+        self.dtype = torch.float32          # the projection writes fp32 logits
 
     def stride(self, i):
         return self._t.stride(i)

@@ -42,8 +42,10 @@ typedef enum {
 
 /* element types accepted for labels and lengths: the reference's data pipeline delivers
  * float32 for all three (reader_kaldi_io.py:33-35, gluonE2EASR/data/batchify.py:78-82);
- * values are truncated toward zero like the operator's own cast. */
-typedef enum { CTCB_I32 = 0, CTCB_I64 = 1, CTCB_F32 = 2, CTCB_F64 = 3 } ctcb_dtype_t;
+ * values are truncated toward zero like the operator's own cast.
+ * CTCB_BF16 is a LOGITS type only (the *_typed entries below); labels and lengths in bfloat16 are refused (integers
+ * above 256 are not exact in bfloat16). */
+typedef enum { CTCB_I32 = 0, CTCB_I64 = 1, CTCB_F32 = 2, CTCB_F64 = 3, CTCB_BF16 = 4 } ctcb_dtype_t;
 
 /* per-utterance status bits written to ctcb_problem_t.status (optional) */
 /* The parameter layer, identical on every kernel path.  Lengths are truncated toward zero, then clamped to [0, T] and
@@ -72,9 +74,9 @@ typedef struct ctcb_problem {
     int32_t blank;                  /* 0 for blank_label='first' (loss.py:139), V-1 for 'last' */
     int32_t label_pad;              /* padding value that ends a label row when label_lengths
                                        is NULL: 0 for 'first', -1 for 'last' (row a3) */
-    const float* logits;            /* unnormalised activations, fp32 */
+    const float* logits;            /* unnormalised activations, fp32 (bf16 through the *_typed entries) */
     int64_t logits_stride_t, logits_stride_b;
-    float* grad;                    /* d(sum_b head[b]*loss[b])/d logits; NULL = forward only */
+    float* grad;                    /* d(sum_b head[b]*loss[b])/d logits, the logits' type; NULL = forward only */
     int64_t grad_stride_t, grad_stride_b;
     const void* labels;             /* (B, Lmax), label_dtype */
     int32_t label_dtype;            /* ctcb_dtype_t */
@@ -125,6 +127,29 @@ int ctcb_forward(const ctcb_problem_t* p, int32_t keep_for_backward, void* works
                  size_t workspace_bytes, void* stream);
 int ctcb_backward(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes,
                   void* stream);
+
+/* The same three entries with the logits' element type: logits_dtype CTCB_F32 (exactly the entries above, which are these
+ * with CTCB_F32) or CTCB_BF16 (a mixed-precision model's logits, read without an upcast pass).  p->logits and p->grad are
+ * then read as that type (strides and logits_row_offsets stay in elements); the gradient has the logits' type.
+ * The bfloat16 contract:
+ *   - a bf16 logit is converted to fp32 exactly when it is loaded; after the load every operation is the fp32 path's, in
+ *     the same order, and the kernels selected are those of the fp32 call on the upcast logits (same launches, gradient
+ *     kernel and walker configuration).  One exception: the bulk-copy (staged) variants of the wide-vocabulary kernels
+ *     need 16-byte aligned rows of a multiple of 16 bytes, so a bf16 call with V % 8 != 0 (or strides not multiples of
+ *     8 elements) takes the register variants where the fp32 call with V % 4 == 0 is staged -- same results, other kernels;
+ *   - loss (fp32), head_grad (fp32), loss_sum (fp64) and the status word are unchanged: the loss and the status word are
+ *     bit-identical to the fp32 call on the upcast logits, CTCB_UTT_WIDE_LOGITS included;
+ *   - each gradient element is the fp32 path's value rounded ONCE to bfloat16 (round to nearest even); padded frames and
+ *     infeasible utterances are exact zeros, rows a missing forward call leaves are NaN;
+ *   - the opt-in one-kernel path ("meet" option) is fp32-only: bf16 calls take the two-kernel path.
+ * Any other logits_dtype (fp16 included) is CTCB_INVALID_VALUE.  The host entries, ctcb_pipe_*, ctcb_loss_grad_timed and
+ * ctcb_proj_* are fp32-only.  A binding detects the feature by looking these symbols up. */
+int ctcb_loss_grad_typed(const ctcb_problem_t* p, int32_t logits_dtype, void* workspace, size_t workspace_bytes,
+                         void* stream);
+int ctcb_forward_typed(const ctcb_problem_t* p, int32_t logits_dtype, int32_t keep_for_backward, void* workspace,
+                       size_t workspace_bytes, void* stream);
+int ctcb_backward_typed(const ctcb_problem_t* p, int32_t logits_dtype, void* workspace, size_t workspace_bytes,
+                        void* stream);
 
 /* Measurement aid (bench.py's roofline leg): ctcb_loss_grad with a CUDA event recorded on
  * `stream` after every kernel; synchronises and returns the per-kernel device times in launch
@@ -194,6 +219,12 @@ int ctcb_greedy_decode_unk(const float* logits, int64_t stride_t, int64_t stride
                            const void* data_lengths, int32_t data_lengths_dtype,
                            int32_t T, int32_t B, int32_t V, int32_t blank, int32_t unk,
                            int32_t* out_tokens, int32_t* out_lengths, void* stream);
+/* ctcb_greedy_decode_unk for logits of type logits_dtype (CTCB_F32 or CTCB_BF16; bf16 values are compared after an exact
+ * widening, ties -- frequent in bf16 -- still go to the lowest index). */
+int ctcb_greedy_decode_typed(const void* logits, int32_t logits_dtype, int64_t stride_t, int64_t stride_b,
+                             const void* data_lengths, int32_t data_lengths_dtype,
+                             int32_t T, int32_t B, int32_t V, int32_t blank, int32_t unk,
+                             int32_t* out_tokens, int32_t* out_lengths, void* stream);
 
 /* Edit distance of each (reference, hypothesis) token pair of a batch: scripts/swbd/wer.py:45-68
  * (`_edit_distance`; next-row scope, SURVEY 8f rank 4).  ref (B, max_ref) / hyp (B, max_hyp)

@@ -52,13 +52,13 @@ typedef struct DLManagedTensor {
 
 /* mx.nd.contrib.ctc_loss(data, label, data_lengths, label_lengths, use_data_lengths,
  * use_label_lengths, blank_label) (loss.py:134-139) on DLPack tensors.
- *   logits        fp32 CUDA, 3-d, unit stride on the last axis, any T/B strides
+ *   logits        fp32 or bfloat16 CUDA, 3-d, unit stride on the last axis, any T/B strides (bf16: ctcb.h, *_typed)
  *   labels        2-d, int32/int64/float32/float64, CUDA
  *   data_lengths  1-d (B,) or NULL  == use_data_lengths=False
  *   label_lengths 1-d (B,) or NULL  == use_label_lengths=False
  *   head_grad     1-d (B,) fp32 or NULL (= ones)
  *   loss          1-d (B,) fp32, written
- *   grad          same shape as logits, fp32, written; NULL = forward only
+ *   grad          same shape and dtype as logits, written; NULL = forward only
  *   loss_sum      0/1-d float64 scalar accumulated in place, or NULL
  *   blank_last    0: blank_label='first' (the reference, loss.py:139), 1: 'last'
  */
