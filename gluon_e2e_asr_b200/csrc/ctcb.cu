@@ -53,6 +53,8 @@ bool launch_pending_xchg(cudaStream_t stream, bool programmatic = false) {
     return true;
 }
 thread_local const ctcb_proj_t* g_proj = nullptr;      // ctcb_proj_*: the projection whose epilogue replaces k_emit in this call
+struct DecodeRequest { int32_t* tokens; int32_t* lengths; int unk; };
+thread_local const DecodeRequest* g_decode = nullptr;  // ctcb_proj_forward_decode: the greedy decode the projection's epilogue adds
 thread_local cudaEvent_t* g_prof_events = nullptr;   // when set: one event recorded after every launch
 thread_local int g_prof_count = 0;
 
@@ -416,7 +418,7 @@ int launch_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const ctcb::Prob
         return fail(CTCB_INVALID_VALUE, "projection: hidden / weight / bias must be CUDA device memory");
     // CTA pairs (tcgen05 cta_group::2: 256 frames per pair, each CTA stages half of the vocabulary tile) or single CTAs
     const int ctas = opt(OPT_PROJ_CTAS) == 1 ? 1 : 2;            // measured: pairs 186 us, single CTAs 190 us per fused forward (cfg3, H = 512)
-    const size_t smem = ctcb::proj_smem_bytes(p->Lmax, lay.Lp, p->logits != nullptr, (p->V + ctcb::kPN - 1) / ctcb::kPN, ctas);
+    const size_t smem = ctcb::proj_smem_bytes(p->Lmax, lay.Lp, p->logits != nullptr, (p->V + ctcb::kPN - 1) / ctcb::kPN, ctas, g_decode != nullptr);
     if (smem > 232448 - 64) return fail(CTCB_UNSUPPORTED, "projection: Lmax=%d label columns do not fit the kernel's shared memory", p->Lmax);
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return fail(CTCB_UNSUPPORTED, "cuTensorMapEncodeTiled is not available from this driver");
@@ -448,6 +450,8 @@ int launch_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const ctcb::Prob
     pa.ctas = ctas;
     pa.dbg = opt(OPT_PROJ_DBG) > 0 ? opt(OPT_PROJ_DBG) : 0;
     pa.vec4 = (p->V % 4 == 0 && reinterpret_cast<uintptr_t>(pj->bias) % 16 == 0) ? 1 : 0;
+    pa.tok = g_decode ? g_decode->tokens : nullptr;
+    pa.unk = g_decode ? g_decode->unk : -1;
     // the logits (kept for the gradient kernel) leave through TMA stores when their rows allow a tensor map
     CUtensorMap tmC = tmA;
     pa.store = 0;
@@ -489,6 +493,8 @@ int launch_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const ctcb::Prob
         mark(stream);
         return CTCB_OK;
     }
+    // decoding: k_greedy_collapse acquires the tile flags, which a previous call on this workspace may have left set
+    if (g_decode) CUDA_TRY(cudaMemsetAsync(w.tflag, 0, sizeof(int) * (size_t)p->B * w.ntile, stream));
     CUDA_TRY(ctcb::launch_proj_emit(tmA, tmB, tmC, pa, pgrid, smem, stream, false));
     mark(stream);
     // the metadata kernel as the projection kernel's programmatic dependent -- it starts at once and runs beside it (it
@@ -653,6 +659,14 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
             if (int rc = launch_proj(g_proj, p, dp, w, lay, stream, beside)) return rc;
         } else if (!lay.fused) { if (int rc = launch_emit()) return rc; }
         if (int rc = launch_walk((xchg && lay.fused != 0) || beside, beside)) return rc;
+        if (g_decode) {
+            // the hypotheses from the projection's per-frame words (an ordinary launch: it acquires the tile flags itself)
+            const size_t dsm = 2 * sizeof(int) * (size_t)p->T;
+            if (dsm > 48 * 1024) CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(ctcb::k_greedy_collapse), dsm));
+            ctcb::k_greedy_collapse<<<p->B, 256, dsm, stream>>>(w.tflag, w.ntile, p->data_lengths, p->data_lengths_dtype, p->T, p->blank,
+                                                                g_decode->unk, g_decode->tokens, g_decode->lengths);
+            mark(stream);
+        }
     }
     if (phases & PH_BACKWARD) {
         ctcb::GradArgs ga{dp, w};
@@ -808,6 +822,19 @@ int ctcb_proj_forward(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t 
     g_proj = proj;
     const int rc = enqueue(p, workspace, workspace_bytes, stream, PH_FORWARD, keep_for_backward != 0);
     g_proj = nullptr;
+    return rc;
+}
+
+int ctcb_proj_forward_decode(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t keep_for_backward, int32_t unk,
+                             int32_t* out_tokens, int32_t* out_lengths, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!out_tokens || !out_lengths) return fail(CTCB_INVALID_VALUE, "NULL argument");
+    if (p && unk >= p->V) return fail(CTCB_INVALID_VALUE, "unk %d outside the vocabulary (V=%d; -1 = no <unk> rule)", unk, p->V);
+    if (p && p->T > 0 && 2 * sizeof(int) * (size_t)p->T > 200 * 1024) return fail(CTCB_UNSUPPORTED, "T=%d too long for the decode kernel", p->T);
+    if (!is_device_ptr(out_tokens) || !is_device_ptr(out_lengths)) return fail(CTCB_INVALID_VALUE, "buffers must be CUDA device memory");
+    const DecodeRequest req{out_tokens, out_lengths, unk < 0 ? -1 : unk};
+    g_decode = &req;
+    const int rc = ctcb_proj_forward(proj, p, keep_for_backward, workspace, workspace_bytes, stream);
+    g_decode = nullptr;
     return rc;
 }
 

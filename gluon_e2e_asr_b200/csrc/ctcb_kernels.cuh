@@ -1929,6 +1929,34 @@ __device__ __forceinline__ void top2_push(Top2& t, float v, int i) {
     else if (better(v, i, t.v2, t.i2)) { t.v2 = v; t.i2 = i; }
 }
 #ifndef CTCB_NO_PLAIN_KERNELS   // non-template kernels: defined in ctcb.cu's translation unit only
+// the collapse of frames 0..n-1 by a block of 256 threads: keep[t] = sym[t] != blank && (t == 0 || sym[t] != path[t-1]),
+// compacted in order into out[0..len).  Returns len (in every thread); s_scan: 8 ints of shared memory
+__device__ __forceinline__ int greedy_collapse(const int* path, const int* sym, int n, int blank, int* out, int* s_scan) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int chunk = (n + 255) / 256;
+    const int lo = min(tid * chunk, n), hi = min(lo + chunk, n);
+    int cnt = 0;
+    for (int t = lo; t < hi; ++t) {
+        const int c = sym[t];
+        cnt += (c != blank && (t == 0 || c != path[t - 1]));
+    }
+    int incl = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += v; }
+    if (lane == 31) s_scan[warp] = incl;
+    __syncthreads();
+    int base = 0;
+    for (int k = 0; k < warp; ++k) base += s_scan[k];
+    int pos = base + incl - cnt;
+    for (int t = lo; t < hi; ++t) {
+        const int c = sym[t];
+        if (c != blank && (t == 0 || c != path[t - 1])) out[pos++] = c;
+    }
+    int len = 0;
+    for (int k = 0; k < 8; ++k) len += s_scan[k];
+    return len;
+}
+
 template <typename LT = float>
 __global__ void __launch_bounds__(256) k_greedy_decode(const LT* logits, long long st_t, long long st_b,
                                                        const void* data_len, int dl_dtype, int T, int B, int V,
@@ -1953,28 +1981,40 @@ __global__ void __launch_bounds__(256) k_greedy_decode(const LT* logits, long lo
         if (lane == 0) { path[t] = tp.i1; sym[t] = (unk >= 0 && tp.i1 == unk && tp.i2 != 0x7fffffff) ? tp.i2 : tp.i1; }
     }
     __syncthreads();
-    // keep[t] = sym[t] != blank && (t == 0 || sym[t] != path[t-1]); compact in order
-    const int chunk = (n + 255) / 256;
-    const int lo = min(tid * chunk, n), hi = min(lo + chunk, n);
-    int cnt = 0;
-    for (int t = lo; t < hi; ++t) {
-        const int c = sym[t];
-        cnt += (c != blank && (t == 0 || c != path[t - 1]));
+    const int len = greedy_collapse(path, sym, n, blank, out_tokens + (size_t)b * T, s_scan);
+    if (tid == 255) out_len[b] = len;
+}
+
+// ---------------------------------------------------------------------------------------
+// k_greedy_collapse: grid B, block 256.  The second half of k_greedy_decode for the fused projection's decode epilogue
+// (ctcb_proj.cuh, DECODE), which leaves one word per valid frame in out_tokens: the frame's symbol after the <unk> rule,
+// bit 31 set when its raw best symbol is `unk`.  An ordinary launch behind the recursion kernel, which may have run beside
+// the projection without waiting for it: the utterance's tile flags are acquired here.  Writes the hypothesis, zeros
+// after it (ctcb_greedy_decode's output on a zeroed buffer) and the length.
+// ---------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) k_greedy_collapse(const int* tflag, int ntile, const void* data_len, int dl_dtype, int T,
+                                                         int blank, int unk, int* out_tokens, int* out_len) {
+    extern __shared__ int path[];                 // T ints: the raw best symbol; T more: the symbol after the <unk> rule
+    __shared__ int s_scan[8];
+    const int b = blockIdx.x, tid = threadIdx.x;
+    long long n64 = data_len ? load_as_int(data_len, dl_dtype, b) : T;
+    const int n = (int)(n64 < 0 ? 0 : (n64 > T ? T : n64));
+    int* sym = path + T;
+    for (int k = tid; k * 128 < n; k += 256) {    // the 128-frame tiles that hold valid frames
+        const long long t0 = clock64();           // bounded: a projection that never ran gives garbage, not a hang
+        while (ld_acquire_gpu(tflag + (size_t)b * ntile + k) == 0 && clock64() - t0 < kSpinLimit) __nanosleep(256);
     }
-    int incl = cnt;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += v; }
-    if (lane == 31) s_scan[warp] = incl;
     __syncthreads();
-    int base = 0;
-    for (int k = 0; k < warp; ++k) base += s_scan[k];
-    int pos = base + incl - cnt;
-    int* out = out_tokens + (size_t)b * T;
-    for (int t = lo; t < hi; ++t) {
-        const int c = sym[t];
-        if (c != blank && (t == 0 || c != path[t - 1])) out[pos++] = c;
+    int* row = out_tokens + (size_t)b * T;
+    for (int t = tid; t < n; t += 256) {
+        const int v = row[t];
+        sym[t] = v & 0x7fffffff;
+        path[t] = v < 0 ? unk : (v & 0x7fffffff);
     }
-    if (tid == 255) out_len[b] = base + incl;
+    __syncthreads();                              // the row is staged before the hypothesis overwrites it
+    const int len = greedy_collapse(path, sym, n, blank, row, s_scan);
+    for (int t = len + tid; t < T; t += 256) row[t] = 0;
+    if (tid == 255) out_len[b] = len;
 }
 #endif
 

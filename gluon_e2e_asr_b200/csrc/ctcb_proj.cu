@@ -9,13 +9,14 @@ cudaError_t launch_proj_emit(const CUtensorMap& tmA, const CUtensorMap& tmB, con
                              cudaStream_t stream, bool programmatic) {
     // the opt-in shared-memory size is a per-device function attribute: raised when a launch needs more than any before
     static thread_local int done_dev = -1;
-    static thread_local size_t done_bytes[4] = {0, 0, 0, 0};
+    static thread_local size_t done_bytes[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     int dev = 0;
     cudaGetDevice(&dev);
-    if (done_dev != dev) { done_dev = dev; done_bytes[0] = done_bytes[1] = done_bytes[2] = done_bytes[3] = 0; }
-    const int pair = a.ctas == 2 ? 1 : 0, bf = a.bf16 ? 1 : 0, which = pair * 2 + bf;
+    if (done_dev != dev) { done_dev = dev; for (size_t& d : done_bytes) d = 0; }
+    const int pair = a.ctas == 2 ? 1 : 0, bf = a.bf16 ? 1 : 0, dec = a.tok ? 1 : 0, which = dec * 4 + pair * 2 + bf;
     using Fn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, ProjArgs);
-    static const Fn fns[4] = {k_proj_emit<1, false>, k_proj_emit<1, true>, k_proj_emit<2, false>, k_proj_emit<2, true>};
+    static const Fn fns[8] = {k_proj_emit<1, false, false>, k_proj_emit<1, true, false>, k_proj_emit<2, false, false>, k_proj_emit<2, true, false>,
+                              k_proj_emit<1, false, true>, k_proj_emit<1, true, true>, k_proj_emit<2, false, true>, k_proj_emit<2, true, true>};
     const Fn fn = fns[which];
     if (done_bytes[which] < smem) {
         const cudaError_t rc = cudaFuncSetAttribute(reinterpret_cast<const void*>(fn), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -65,6 +65,9 @@ struct ProjArgs {
     int ctas;                // 1: one CTA per tile; 2: CTA pairs (tcgen05 cta_group::2) over 256 frames
     int bf16;                // operands are bfloat16 (64 values per 128-byte K block, kind::f16) instead of fp32 (32, kind::tf32)
     int dbg;                 // measurement only (option proj_dbg): 1 = the epilogue skips its arithmetic (results are garbage)
+    int* tok;                // DECODE: (B, T) one word per valid frame -- the symbol after the <unk> rule, bit 31 set when the
+                             //   raw best symbol is `unk` -- collapsed into the hypothesis by k_greedy_collapse
+    int unk;                 // DECODE: the <unk> index, or -1 for no <unk> rule
 };
 
 constexpr uint32_t kPStageTile = 32 * 32 * 4;    // one warp's 32 frames x 32 columns on their way to the logits tensor
@@ -75,9 +78,11 @@ __host__ __device__ inline size_t proj_side_bytes(int Lmax, bool store) {
     if (store) return (size_t)kPEpiWarps * 2 * kPStageTile;
     return proj_smem_stash(Lmax, store) ? (size_t)(Lmax + 1) * kPM * sizeof(float) : 0;
 }
-__host__ __device__ inline size_t proj_smem_bytes(int Lmax, int Lp, bool store, int NT, int ctas) {
+// decode: + the upper column halves' top-2 lists, where the two halves of a row meet
+__host__ __device__ inline size_t proj_smem_bytes(int Lmax, int Lp, bool store, int NT, int ctas, bool decode = false) {
     return 1024 + (size_t)proj_stages(ctas) * proj_stage_bytes(ctas) + proj_side_bytes(Lmax, store) +
-           (size_t)Lp * sizeof(int) + 128 + 2 * kPM * sizeof(float2) + (size_t)(Lp + 4) * sizeof(int) + (size_t)(2 * NT + 4) * sizeof(int);
+           (size_t)Lp * sizeof(int) + 128 + 2 * kPM * sizeof(float2) + (size_t)(Lp + 4) * sizeof(int) + (size_t)(2 * NT + 4) * sizeof(int) +
+           (decode ? kPM * sizeof(Top2) : 0);
 }
 
 // (a.ctas == 2: grid.x even, launched as clusters of two CTAs along x)
@@ -216,7 +221,10 @@ constexpr uint32_t kPIdescBfPair = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32
 
 __device__ __forceinline__ void bar_sync_epilogue() { asm volatile("bar.sync 1, %0;" ::"n"(32 * kPEpiWarps) : "memory"); }
 
-template <int CTAS, bool BF16>
+// DECODE: the epilogue also reduces each frame's row to its best and second best symbol (k_greedy_decode's order: greater
+// value, ties to the lower index) and writes the frame's word of ProjArgs::tok -- the greedy decode of the logits that
+// are never stored.  A compile-time switch: a run-time branch in this kernel was measured at +17 us (DESIGN.md section 5)
+template <int CTAS, bool BF16, bool DECODE>
 __global__ void __launch_bounds__(kPThreads, 1)
 k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmC,
             ProjArgs a) {
@@ -384,6 +392,7 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         const uint32_t sbuf = sC + (uint32_t)(warp - 2) * 2 * kPStageTile;
         int nstored = 0;
         float mx = -INFINITY, sum = 0.0f;
+        Top2 tp{-INFINITY, 0x7fffffff, -INFINITY, 0x7fffffff};   // DECODE: the best two of this thread's columns
         for (int n = 0; n < a.NT; ++n) {
             const int as = n & 1;
             mbar_wait(tfull + as, ((uint32_t)n >> 1) & 1u);
@@ -454,6 +463,16 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                     sp[3] += fast_ex2(fmaf(x[i + 3], kLog2e, -ms));
                 }
                 sum += (sp[0] + sp[1]) + (sp[2] + sp[3]);
+                if constexpr (DECODE) {
+                    // a thread visits its columns in increasing order: a chunk whose maximum only ties the second best
+                    // holds higher indices and cannot displace it (one compare per 32 columns in the common case).
+                    // Columns >= V are never pushed
+                    if (cmx > tp.v2 || tp.i2 == 0x7fffffff) {
+#pragma unroll
+                        for (int i = 0; i < 32; ++i)
+                            if (FULLC || col0 + i < p.V) top2_push(tp, x[i], col0 + i);
+                    }
+                }
             };
 #pragma unroll
             for (int c = 0; c < HC / 32; ++c) {
@@ -476,12 +495,26 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         }
         // ---- the two column halves of a row meet: row max and normaliser ----
         part[hsel * kPM + r] = make_float2(mx, sum);
+        Top2* htop = reinterpret_cast<Top2*>(hstart + 2 * a.NT + 4);      // DECODE: [128] the upper halves' top-2 lists
+        if constexpr (DECODE) { if (hsel == 1) htop[r] = tp; }
         bar_sync_epilogue();
         {
             const float2 o = part[(hsel ^ 1) * kPM + r];
             const float m2 = fmaxf(mx, o.x);           // a half without columns holds {-inf, 0}: ex2(-inf) = 0
             sum = sum * fast_ex2((mx - m2) * kLog2e) + o.y * fast_ex2((o.x - m2) * kLog2e);
             mx = m2;
+        }
+        if constexpr (DECODE) {
+            // the frame's word: the best symbol, or the second best when the best is `unk` (k_greedy_decode's rule and
+            // fallback); bit 31 keeps the raw best for the repeat test of the next frame, whatever V is
+            if (hsel == 0 && valid) {
+                const Top2 o = htop[r];
+                top2_push(tp, o.v1, o.i1);
+                top2_push(tp, o.v2, o.i2);
+                const bool is_unk = a.unk >= 0 && tp.i1 == a.unk;
+                const int sym = (is_unk && tp.i2 != 0x7fffffff) ? tp.i2 : tp.i1;
+                a.tok[(size_t)b * p.T + t] = sym | (is_unk ? (int)0x80000000 : 0);
+            }
         }
         // ---- the frame's outputs: {row max, log2 normaliser}; the parked columns (each thread finishes the ones it
         // parked itself) become softmax numerators relative to the final row maximum ----

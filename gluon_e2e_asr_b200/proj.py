@@ -21,7 +21,7 @@ import torch
 from . import _lib
 from .ops import _Call, _alloc_ws, _blank_last, _on_device, _stream_ptr
 
-__all__ = ["proj_ctc_loss", "ProjCtcLoss"]
+__all__ = ["proj_ctc_loss", "proj_ctc_eval", "ProjCtcLoss"]
 
 
 def _proj_struct(hidden, weight, bias):
@@ -157,6 +157,42 @@ def proj_ctc_loss(hidden, weight, bias, label, pred_lengths=None, label_lengths=
                                 label_layout == "TN", (not needs_grad) or bool(fused_training))
 
 
+def proj_ctc_eval(hidden, weight, bias, label, pred_lengths=None, label_lengths=None, blank_label="first",
+                  label_layout="NT", unk=None):
+    """The validation pass from the encoder output (train_ctc_ce.py:143-160): ``(loss (B,), tokens (B,T) int32,
+    lengths (B,) int32)`` of ``hidden @ weight.T + bias`` without the logits ever reaching HBM.
+
+    ``loss`` is bit-identical to ``proj_ctc_loss`` under ``torch.no_grad()``.  ``tokens`` / ``lengths`` are
+    ``greedy_decode(logits, pred_lengths, blank, unk=unk)`` of the logits the fused product forms (blank 0, or V - 1 for
+    ``blank_label="last"``): the projection's epilogue keeps each frame's best two symbols while it reduces the row, and a
+    small kernel collapses repeats and blanks.  The outputs go straight into ``edit_distance``.  fp32 (tf32 product) or
+    bfloat16 operands; no autograd graph."""
+    _check_inputs(hidden, weight, bias)
+    if hidden.stride(2) != 1:
+        hidden = hidden.contiguous()
+    weight = weight.detach().contiguous()
+    bias = bias.detach().contiguous() if bias is not None else None
+    B, T, K = hidden.shape
+    V = weight.shape[0]
+    dev = hidden.device
+    meta = torch.empty((B, T, V), dtype=torch.float32, device="meta")
+    call = _Call(_MetaLogits(meta, dev), label, pred_lengths, label_lengths, _blank_last(blank_label), True,
+                 label_layout == "TN")
+    loss = torch.empty((B,), dtype=torch.float32, device=dev)
+    tokens = torch.empty((B, T), dtype=torch.int32, device=dev)
+    lengths = torch.empty((B,), dtype=torch.int32, device=dev)
+    ws = _alloc_ws(call, False)
+    p = call.problem(loss)
+    p.logits = None
+    pj = _proj_struct(hidden, weight, bias)
+    with _on_device(dev):
+        rc = _lib.load().ctcb_proj_forward_decode(ctypes.byref(pj), ctypes.byref(p), 0, -1 if unk is None else int(unk),
+                                                  tokens.data_ptr(), lengths.data_ptr(), ws.data_ptr(), ws.numel(),
+                                                  _stream_ptr(dev))
+    _lib.check(rc)
+    return loss, tokens, lengths
+
+
 class ProjCtcLoss(torch.nn.Module):
     """``tgt_proj`` + ``CtcLoss`` as one block: holds the Dense parameters (units=V, in_units=K) in gluon's layout."""
 
@@ -170,3 +206,8 @@ class ProjCtcLoss(torch.nn.Module):
     def forward(self, hidden, label, pred_lengths=None, label_lengths=None, fused_training=False):
         return proj_ctc_loss(hidden, self.weight, self.bias, label, pred_lengths, label_lengths, self.blank_label,
                              self.label_layout, fused_training)
+
+    def evaluate(self, hidden, label, pred_lengths=None, label_lengths=None, unk=None):
+        """``proj_ctc_eval`` with this block's parameters: (loss, tokens, lengths), the logits never stored."""
+        return proj_ctc_eval(hidden, self.weight, self.bias, label, pred_lengths, label_lengths, self.blank_label,
+                             self.label_layout, unk)

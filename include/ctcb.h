@@ -335,6 +335,16 @@ typedef struct ctcb_proj {
  * walkers' fused producers read them once anyway) and for label rows too long for the kernel's shared memory. */
 int ctcb_proj_forward(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t keep_for_backward, void* workspace,
                       size_t workspace_bytes, void* stream);
+/* ctcb_proj_forward plus the greedy decode of ctcb_greedy_decode_unk on the logits the projection forms
+ * (train_ctc_ce.py:143-160): blank = p->blank, frame counts = p->data_lengths (clamped like the parameter layer),
+ * unk = -1 for no <unk> rule.  out_tokens (B, T) int32, hypothesis prefix then zeros; out_lengths (B,) int32.  Tokens and
+ * lengths are those of ctcb_greedy_decode_unk on the logits the projection writes with keep_for_backward = 1 (bit for bit:
+ * the epilogue compares the values it would store, in the same order).  Device buffers; out_tokens also serves as the
+ * per-frame scratch between the projection and the collapse kernel.  CTCB_UNSUPPORTED for T too long for the collapse
+ * kernel's shared memory (2 T ints <= 200 KB).  Detected by symbol, like the *_typed entries. */
+int ctcb_proj_forward_decode(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t keep_for_backward, int32_t unk,
+                             int32_t* out_tokens, int32_t* out_lengths, void* workspace, size_t workspace_bytes,
+                             void* stream);
 /* ctcb_proj_forward(keep_for_backward=1) followed by ctcb_backward in one call: loss, p->logits and p->grad. */
 int ctcb_proj_loss_grad(const ctcb_proj_t* proj, const ctcb_problem_t* p, void* workspace, size_t workspace_bytes,
                         void* stream);
