@@ -9,7 +9,7 @@ from .loss import CtcLoss
 from .batch import PinnedBatch
 from .pipeline import HostPipeline
 from .ops import CTCLoss, ctc_loss, ctc_loss_and_grad, edit_distance, greedy_decode, workspace_bytes
-from .proj import ProjCtcLoss, proj_ctc_eval, proj_ctc_loss
+from .proj import ProjCtcLoss, proj_ctc_eval, proj_ctc_loss, proj_greedy_decode
 from .sampler import FixedBucketSampler, SortedBucketSampler, SortedSampler
 from .sharding import (PeerLossSum, balanced_assignment, loss_sum_allreduce, shard_for_rank,
                        split_and_load, split_slices)
@@ -17,4 +17,4 @@ from .sharding import (PeerLossSum, balanced_assignment, loss_sum_allreduce, sha
 __all__ = ["CtcLoss", "CTCLoss", "ctc_loss", "ctc_loss_and_grad", "greedy_decode",
            "workspace_bytes", "split_and_load", "split_slices", "balanced_assignment",
            "shard_for_rank", "loss_sum_allreduce", "PeerLossSum", "edit_distance", "PinnedBatch", "HostPipeline", "FixedBucketSampler",
-           "SortedBucketSampler", "SortedSampler", "ProjCtcLoss", "proj_ctc_loss", "proj_ctc_eval"]
+           "SortedBucketSampler", "SortedSampler", "ProjCtcLoss", "proj_ctc_loss", "proj_ctc_eval", "proj_greedy_decode"]

@@ -397,6 +397,67 @@ EncodeTiledFn encode_tiled() {
     return fn;
 }
 
+// the projection's operands (hidden, weight, bias): element type, 16-byte strides and bases, device memory
+int check_proj_operands(const ctcb_proj_t* pj) {
+    if (pj->operand_dtype != CTCB_PROJ_F32 && pj->operand_dtype != CTCB_PROJ_BF16)
+        return fail(CTCB_INVALID_VALUE, "projection: operand_dtype %d is neither CTCB_PROJ_F32 nor CTCB_PROJ_BF16", pj->operand_dtype);
+    const int per16 = pj->operand_dtype == CTCB_PROJ_BF16 ? 8 : 4;
+    if (pj->K % per16 || pj->hidden_stride_t % per16 || pj->hidden_stride_b % per16 || reinterpret_cast<uintptr_t>(pj->hidden) % 16 ||
+        reinterpret_cast<uintptr_t>(pj->weight) % 16)
+        return fail(CTCB_INVALID_VALUE, "projection: K and the hidden strides must be multiples of 16 bytes, bases 16-byte aligned");
+    if (!is_device_ptr(pj->hidden) || !is_device_ptr(pj->weight) || !is_device_ptr(pj->bias))
+        return fail(CTCB_INVALID_VALUE, "projection: hidden / weight / bias must be CUDA device memory");
+    return CTCB_OK;
+}
+
+// the TMA maps of the projection's operands: hidden (K, T, B) in boxes of one 128-byte K block x kPM frames, weight (K, V) in
+// boxes of one K block x the CTA's share of a vocabulary tile
+int encode_proj_maps(const ctcb_proj_t* pj, int T, int B, int V, int ctas, CUtensorMap* tmA, CUtensorMap* tmB) {
+    EncodeTiledFn enc = encode_tiled();
+    if (!enc) return fail(CTCB_UNSUPPORTED, "cuTensorMapEncodeTiled is not available from this driver");
+    const bool bf = pj->operand_dtype == CTCB_PROJ_BF16;
+    const int esz = bf ? 2 : 4;
+    {
+        const cuuint64_t gdim[3] = {(cuuint64_t)pj->K, (cuuint64_t)T, (cuuint64_t)B};
+        const cuuint64_t gstr[2] = {(cuuint64_t)pj->hidden_stride_t * esz, (cuuint64_t)pj->hidden_stride_b * esz};
+        const cuuint32_t box[3] = {(cuuint32_t)(128 / esz), (cuuint32_t)ctcb::kPM, 1};
+        const cuuint32_t est[3] = {1, 1, 1};
+        const CUresult r = enc(tmA, bf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(pj->hidden), gdim, gstr, box, est,
+                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) return fail(CTCB_INVALID_VALUE, "cuTensorMapEncodeTiled(hidden) failed: %d", (int)r);
+    }
+    {
+        const cuuint64_t gdim[2] = {(cuuint64_t)pj->K, (cuuint64_t)V};
+        const cuuint64_t gstr[1] = {(cuuint64_t)pj->K * esz};
+        const cuuint32_t box[2] = {(cuuint32_t)(128 / esz), (cuuint32_t)(ctcb::kPN / ctas)};
+        const cuuint32_t est[2] = {1, 1};
+        const CUresult r = enc(tmB, bf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(pj->weight), gdim, gstr, box, est,
+                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) return fail(CTCB_INVALID_VALUE, "cuTensorMapEncodeTiled(weight) failed: %d", (int)r);
+    }
+    return CTCB_OK;
+}
+
+// the launch fields that depend on the projection alone (the caller adds the problem, workspace and outputs)
+ctcb::ProjArgs proj_args(const ctcb_proj_t* pj, int V, int ctas) {
+    const int esz = pj->operand_dtype == CTCB_PROJ_BF16 ? 2 : 4;
+    ctcb::ProjArgs pa{};
+    pa.bias = pj->bias;
+    pa.K = pj->K; pa.NT = (V + ctcb::kPN - 1) / ctcb::kPN; pa.KB = (pj->K + 128 / esz - 1) / (128 / esz);
+    pa.bf16 = esz == 2 ? 1 : 0;
+    pa.ctas = ctas;
+    pa.dbg = opt(OPT_PROJ_DBG) > 0 ? opt(OPT_PROJ_DBG) : 0;
+    pa.vec4 = (V % 4 == 0 && reinterpret_cast<uintptr_t>(pj->bias) % 16 == 0) ? 1 : 0;
+    pa.unk = -1;
+    return pa;
+}
+
+// CTA pairs (tcgen05 cta_group::2: 256 frames per pair, each CTA stages half of the vocabulary tile) or single CTAs
+// (measured: pairs 186 us, single CTAs 190 us per fused forward at cfg3, H = 512)
+inline int proj_ctas() { return opt(OPT_PROJ_CTAS) == 1 ? 1 : 2; }
+
 // the projection kernel (ctcb_proj.cuh) in k_emit's place: {row max, normaliser} and the emission table from the
 // encoder output, then the metadata CTAs of k_emit (one per utterance)
 // beside: the recursion kernel will be launched as the projection's programmatic dependent and follow its tiles (loss
@@ -407,49 +468,14 @@ int launch_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const ctcb::Prob
     if (lay.fused || lay.dense)
         return fail(CTCB_UNSUPPORTED, "projection fused with the loss needs V > 64 and V > Lmax + 1 (V=%d, Lmax=%d)", p->V, p->Lmax);
     if (p->logits_row_offsets) return fail(CTCB_UNSUPPORTED, "projection: packed logits are not supported");
-    if (pj->operand_dtype != CTCB_PROJ_F32 && pj->operand_dtype != CTCB_PROJ_BF16)
-        return fail(CTCB_INVALID_VALUE, "projection: operand_dtype %d is neither CTCB_PROJ_F32 nor CTCB_PROJ_BF16", pj->operand_dtype);
-    const bool bf = pj->operand_dtype == CTCB_PROJ_BF16;
-    const int esz = bf ? 2 : 4, per16 = 16 / esz;
-    if (pj->K % per16 || pj->hidden_stride_t % per16 || pj->hidden_stride_b % per16 || reinterpret_cast<uintptr_t>(pj->hidden) % 16 ||
-        reinterpret_cast<uintptr_t>(pj->weight) % 16)
-        return fail(CTCB_INVALID_VALUE, "projection: K and the hidden strides must be multiples of 16 bytes, bases 16-byte aligned");
-    if (!is_device_ptr(pj->hidden) || !is_device_ptr(pj->weight) || !is_device_ptr(pj->bias))
-        return fail(CTCB_INVALID_VALUE, "projection: hidden / weight / bias must be CUDA device memory");
-    // CTA pairs (tcgen05 cta_group::2: 256 frames per pair, each CTA stages half of the vocabulary tile) or single CTAs
-    const int ctas = opt(OPT_PROJ_CTAS) == 1 ? 1 : 2;            // measured: pairs 186 us, single CTAs 190 us per fused forward (cfg3, H = 512)
+    if (int rc = check_proj_operands(pj)) return rc;
+    const int ctas = proj_ctas();
     const size_t smem = ctcb::proj_smem_bytes(p->Lmax, lay.Lp, p->logits != nullptr, (p->V + ctcb::kPN - 1) / ctcb::kPN, ctas, g_decode != nullptr);
     if (smem > 232448 - 64) return fail(CTCB_UNSUPPORTED, "projection: Lmax=%d label columns do not fit the kernel's shared memory", p->Lmax);
-    EncodeTiledFn enc = encode_tiled();
-    if (!enc) return fail(CTCB_UNSUPPORTED, "cuTensorMapEncodeTiled is not available from this driver");
     CUtensorMap tmA, tmB;
-    {
-        const cuuint64_t gdim[3] = {(cuuint64_t)pj->K, (cuuint64_t)p->T, (cuuint64_t)p->B};
-        const cuuint64_t gstr[2] = {(cuuint64_t)pj->hidden_stride_t * esz, (cuuint64_t)pj->hidden_stride_b * esz};
-        const cuuint32_t box[3] = {(cuuint32_t)(128 / esz), (cuuint32_t)ctcb::kPM, 1};
-        const cuuint32_t est[3] = {1, 1, 1};
-        const CUresult r = enc(&tmA, bf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(pj->hidden), gdim, gstr, box, est,
-                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail(CTCB_INVALID_VALUE, "cuTensorMapEncodeTiled(hidden) failed: %d", (int)r);
-    }
-    {
-        const cuuint64_t gdim[2] = {(cuuint64_t)pj->K, (cuuint64_t)p->V};
-        const cuuint64_t gstr[1] = {(cuuint64_t)pj->K * esz};
-        const cuuint32_t box[2] = {(cuuint32_t)(128 / esz), (cuuint32_t)(ctcb::kPN / ctas)};
-        const cuuint32_t est[2] = {1, 1};
-        const CUresult r = enc(&tmB, bf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(pj->weight), gdim, gstr, box, est,
-                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail(CTCB_INVALID_VALUE, "cuTensorMapEncodeTiled(weight) failed: %d", (int)r);
-    }
-    ctcb::ProjArgs pa{};
-    pa.p = dp; pa.w = w; pa.bias = pj->bias; pa.logits = const_cast<float*>(p->logits);
-    pa.K = pj->K; pa.NT = (p->V + ctcb::kPN - 1) / ctcb::kPN; pa.KB = (pj->K + 128 / esz - 1) / (128 / esz);
-    pa.bf16 = bf ? 1 : 0;
-    pa.ctas = ctas;
-    pa.dbg = opt(OPT_PROJ_DBG) > 0 ? opt(OPT_PROJ_DBG) : 0;
-    pa.vec4 = (p->V % 4 == 0 && reinterpret_cast<uintptr_t>(pj->bias) % 16 == 0) ? 1 : 0;
+    if (int rc = encode_proj_maps(pj, p->T, p->B, p->V, ctas, &tmA, &tmB)) return rc;
+    ctcb::ProjArgs pa = proj_args(pj, p->V, ctas);
+    pa.p = dp; pa.w = w; pa.logits = const_cast<float*>(p->logits);
     pa.tok = g_decode ? g_decode->tokens : nullptr;
     pa.unk = g_decode ? g_decode->unk : -1;
     // the logits (kept for the gradient kernel) leave through TMA stores when their rows allow a tensor map
@@ -464,7 +490,7 @@ int launch_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const ctcb::Prob
             const cuuint32_t box[3] = {32, 32, 1};
             const cuuint32_t est[3] = {1, 1, 1};
             // a (T,B,V) buffer has the batch stride below the frame stride: the map's dimensions stay (V, T, B), strides say the rest
-            const CUresult r = enc(&tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(p->logits), gdim, gstr, box, est,
+            const CUresult r = encode_tiled()(&tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(p->logits), gdim, gstr, box, est,
                                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
                                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
             if (r == CUDA_SUCCESS) pa.store = 1;
@@ -472,6 +498,7 @@ int launch_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const ctcb::Prob
     }
     const int mtiles = (p->T + ctcb::kPM - 1) / ctcb::kPM;
     const dim3 pgrid(ctas, p->B, (mtiles + ctas - 1) / ctas);
+    const int mode = g_decode ? ctcb::kProjLossDecode : ctcb::kProjLoss;
     auto launch_meta = [&](bool programmatic) -> int {
         // per-utterance metadata: k_emit's extra CTA alone (grid.x = 1: every CTA is the metadata CTA)
         cudaLaunchConfig_t cfg{};
@@ -489,13 +516,13 @@ int launch_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const ctcb::Prob
         CUDA_TRY(cudaMemsetAsync(w.tflag, 0, sizeof(int) * (size_t)p->B * w.ntile, stream));
         CUDA_TRY(cudaMemsetAsync(w.gprog, 0, sizeof(int) * 4 * (size_t)p->B, stream));
         if (int rc = launch_meta(false)) return rc;
-        CUDA_TRY(ctcb::launch_proj_emit(tmA, tmB, tmC, pa, pgrid, smem, stream, true));    // programmatic: beside the metadata kernel
+        CUDA_TRY(ctcb::launch_proj_emit(tmA, tmB, tmC, pa, mode, pgrid, smem, stream, true));    // programmatic: beside the metadata kernel
         mark(stream);
         return CTCB_OK;
     }
     // decoding: k_greedy_collapse acquires the tile flags, which a previous call on this workspace may have left set
     if (g_decode) CUDA_TRY(cudaMemsetAsync(w.tflag, 0, sizeof(int) * (size_t)p->B * w.ntile, stream));
-    CUDA_TRY(ctcb::launch_proj_emit(tmA, tmB, tmC, pa, pgrid, smem, stream, false));
+    CUDA_TRY(ctcb::launch_proj_emit(tmA, tmB, tmC, pa, mode, pgrid, smem, stream, false));
     mark(stream);
     // the metadata kernel as the projection kernel's programmatic dependent -- it starts at once and runs beside it (it
     // reads nothing the projection writes); the recursion kernel that follows is an ordinary launch and waits for both
@@ -836,6 +863,44 @@ int ctcb_proj_forward_decode(const ctcb_proj_t* proj, const ctcb_problem_t* p, i
     const int rc = ctcb_proj_forward(proj, p, keep_for_backward, workspace, workspace_bytes, stream);
     g_decode = nullptr;
     return rc;
+}
+
+int ctcb_proj_greedy_decode(const ctcb_proj_t* proj, int32_t T, int32_t B, int32_t V, const void* data_lengths,
+                            int32_t data_lengths_dtype, int32_t blank, int32_t unk, int32_t* out_tokens, int32_t* out_lengths,
+                            void* stream) {
+    g_launches = 0;
+    if (!proj || !out_tokens || !out_lengths) return fail(CTCB_INVALID_VALUE, "NULL argument");
+    if (T <= 0 || B <= 0 || V <= 0) return fail(CTCB_INVALID_VALUE, "bad shape");
+    if (unk >= V) return fail(CTCB_INVALID_VALUE, "unk %d outside the vocabulary (V=%d; -1 = no <unk> rule)", unk, V);
+    if (data_lengths && (data_lengths_dtype < CTCB_I32 || data_lengths_dtype > CTCB_F64))
+        return fail(CTCB_INVALID_VALUE, "unsupported length dtype %d", data_lengths_dtype);
+    const size_t dsm = 2 * sizeof(int) * (size_t)T;
+    if (dsm > 200 * 1024) return fail(CTCB_UNSUPPORTED, "T=%d too long for the decode kernel", T);
+    if (!proj->hidden || !proj->weight || proj->K <= 0) return fail(CTCB_INVALID_VALUE, "projection: hidden / weight is NULL or K <= 0");
+    if (int rc = check_proj_operands(proj)) return rc;
+    if (!is_device_ptr(out_tokens) || !is_device_ptr(out_lengths) || !is_device_ptr(data_lengths))
+        return fail(CTCB_INVALID_VALUE, "buffers must be CUDA device memory");
+    const int ctas = proj_ctas();
+    const int NT = (V + ctcb::kPN - 1) / ctcb::kPN;
+    CUtensorMap tmA, tmB;
+    if (int rc = encode_proj_maps(proj, T, B, V, ctas, &tmA, &tmB)) return rc;
+    // no labels and no workspace: of the problem the decode-only epilogue reads the shape and the frame counts
+    ctcb::ProjArgs pa = proj_args(proj, V, ctas);
+    pa.p.T = T; pa.p.B = B; pa.p.V = V; pa.p.blank = blank;
+    pa.p.data_len = data_lengths; pa.p.data_len_dtype = data_lengths_dtype;
+    pa.tok = out_tokens;
+    pa.unk = unk < 0 ? -1 : unk;
+    const int mtiles = (T + ctcb::kPM - 1) / ctcb::kPM;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    CUDA_TRY(ctcb::launch_proj_emit(tmA, tmB, tmA, pa, ctcb::kProjDecode, dim3(ctas, B, (mtiles + ctas - 1) / ctas),
+                                    ctcb::proj_smem_bytes(0, 0, false, NT, ctas, true), st, false));
+    mark(st);
+    // the collapse right behind the projection: stream order, no tile flags
+    if (dsm > 48 * 1024) CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(ctcb::k_greedy_collapse), dsm));
+    ctcb::k_greedy_collapse<<<B, 256, dsm, st>>>(nullptr, 0, data_lengths, data_lengths_dtype, T, blank, pa.unk, out_tokens, out_lengths);
+    CUDA_TRY(cudaGetLastError());
+    mark(st);
+    return CTCB_OK;
 }
 
 int ctcb_proj_loss_grad(const ctcb_proj_t* proj, const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream) {

@@ -1989,8 +1989,9 @@ __global__ void __launch_bounds__(256) k_greedy_decode(const LT* logits, long lo
 // k_greedy_collapse: grid B, block 256.  The second half of k_greedy_decode for the fused projection's decode epilogue
 // (ctcb_proj.cuh, DECODE), which leaves one word per valid frame in out_tokens: the frame's symbol after the <unk> rule,
 // bit 31 set when its raw best symbol is `unk`.  An ordinary launch behind the recursion kernel, which may have run beside
-// the projection without waiting for it: the utterance's tile flags are acquired here.  Writes the hypothesis, zeros
-// after it (ctcb_greedy_decode's output on a zeroed buffer) and the length.
+// the projection without waiting for it: the utterance's tile flags are acquired here.  tflag == nullptr: an ordinary
+// launch right behind the projection (ctcb_proj_greedy_decode, no walkers), stream order is enough.  Writes the
+// hypothesis, zeros after it (ctcb_greedy_decode's output on a zeroed buffer) and the length.
 // ---------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_greedy_collapse(const int* tflag, int ntile, const void* data_len, int dl_dtype, int T,
                                                          int blank, int unk, int* out_tokens, int* out_len) {
@@ -2000,7 +2001,7 @@ __global__ void __launch_bounds__(256) k_greedy_collapse(const int* tflag, int n
     long long n64 = data_len ? load_as_int(data_len, dl_dtype, b) : T;
     const int n = (int)(n64 < 0 ? 0 : (n64 > T ? T : n64));
     int* sym = path + T;
-    for (int k = tid; k * 128 < n; k += 256) {    // the 128-frame tiles that hold valid frames
+    for (int k = tid; tflag && k * 128 < n; k += 256) {    // the 128-frame tiles that hold valid frames
         const long long t0 = clock64();           // bounded: a projection that never ran gives garbage, not a hang
         while (ld_acquire_gpu(tflag + (size_t)b * ntile + k) == 0 && clock64() - t0 < kSpinLimit) __nanosleep(256);
     }

@@ -5,18 +5,19 @@
 
 namespace ctcb {
 
-cudaError_t launch_proj_emit(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC, const ProjArgs& a, dim3 grid, size_t smem,
-                             cudaStream_t stream, bool programmatic) {
+cudaError_t launch_proj_emit(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC, const ProjArgs& a, int mode, dim3 grid,
+                             size_t smem, cudaStream_t stream, bool programmatic) {
     // the opt-in shared-memory size is a per-device function attribute: raised when a launch needs more than any before
     static thread_local int done_dev = -1;
-    static thread_local size_t done_bytes[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    static thread_local size_t done_bytes[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
     int dev = 0;
     cudaGetDevice(&dev);
     if (done_dev != dev) { done_dev = dev; for (size_t& d : done_bytes) d = 0; }
-    const int pair = a.ctas == 2 ? 1 : 0, bf = a.bf16 ? 1 : 0, dec = a.tok ? 1 : 0, which = dec * 4 + pair * 2 + bf;
+    const int pair = a.ctas == 2 ? 1 : 0, bf = a.bf16 ? 1 : 0, which = mode * 4 + pair * 2 + bf;
     using Fn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, ProjArgs);
-    static const Fn fns[8] = {k_proj_emit<1, false, false>, k_proj_emit<1, true, false>, k_proj_emit<2, false, false>, k_proj_emit<2, true, false>,
-                              k_proj_emit<1, false, true>, k_proj_emit<1, true, true>, k_proj_emit<2, false, true>, k_proj_emit<2, true, true>};
+#define PROJ_MODE(M_) k_proj_emit<1, false, M_>, k_proj_emit<1, true, M_>, k_proj_emit<2, false, M_>, k_proj_emit<2, true, M_>
+    static const Fn fns[12] = {PROJ_MODE(kProjLoss), PROJ_MODE(kProjLossDecode), PROJ_MODE(kProjDecode)};
+#undef PROJ_MODE
     const Fn fn = fns[which];
     if (done_bytes[which] < smem) {
         const cudaError_t rc = cudaFuncSetAttribute(reinterpret_cast<const void*>(fn), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -85,11 +85,15 @@ __host__ __device__ inline size_t proj_smem_bytes(int Lmax, int Lp, bool store, 
            (decode ? kPM * sizeof(Top2) : 0);
 }
 
+// what k_proj_emit's epilogue computes (its MODE, see there)
+enum : int { kProjLoss = 0, kProjLossDecode = 1, kProjDecode = 2 };
+
 // (a.ctas == 2: grid.x even, launched as clusters of two CTAs along x)
 // host-side launcher, defined in ctcb_proj.cu (its own translation unit: the kernel below is compiled there only)
+// mode: kProjLoss, kProjLossDecode or kProjDecode (what the epilogue computes, see k_proj_emit)
 // programmatic: launched with programmatic stream serialization (it starts beside the kernel enqueued before it)
-cudaError_t launch_proj_emit(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC, const ProjArgs& a, dim3 grid, size_t smem,
-                             cudaStream_t stream, bool programmatic);
+cudaError_t launch_proj_emit(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC, const ProjArgs& a, int mode, dim3 grid,
+                             size_t smem, cudaStream_t stream, bool programmatic);
 
 #ifdef CTCB_PROJ_IMPL
 // ---- tcgen05 / TMA wrappers -------------------------------------------------------------------------------------
@@ -221,13 +225,19 @@ constexpr uint32_t kPIdescBfPair = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32
 
 __device__ __forceinline__ void bar_sync_epilogue() { asm volatile("bar.sync 1, %0;" ::"n"(32 * kPEpiWarps) : "memory"); }
 
-// DECODE: the epilogue also reduces each frame's row to its best and second best symbol (k_greedy_decode's order: greater
-// value, ties to the lower index) and writes the frame's word of ProjArgs::tok -- the greedy decode of the logits that
-// are never stored.  A compile-time switch: a run-time branch in this kernel was measured at +17 us (DESIGN.md section 5)
-template <int CTAS, bool BF16, bool DECODE>
+// What the epilogue makes of the tiles (MODE):
+//   kProjLoss        the loss's inputs: {row max, normaliser} in `fr`, the label columns in E, the tile flags;
+//   kProjLossDecode  the same, and each frame's row is also reduced to its best and second best symbol (k_greedy_decode's
+//                    order: greater value, ties to the lower index) for the frame's word of ProjArgs::tok -- the greedy
+//                    decode of the logits that are never stored;
+//   kProjDecode      the frame's word only (ctcb_proj_greedy_decode: no labels): label parsing, the label columns, the
+//                    normaliser, `fr`, E and the tile flags are compiled out, the word is the kProjLossDecode one.
+// A compile-time switch: a run-time branch in this kernel was measured at +17 us (DESIGN.md section 5)
+template <int CTAS, bool BF16, int MODE>
 __global__ void __launch_bounds__(kPThreads, 1)
 k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmC,
             ProjArgs a) {
+    constexpr bool LOSS = MODE != kProjDecode, DECODE = MODE != kProjLoss;
     extern __shared__ unsigned char proj_raw[];
     __shared__ int s_L;
     const Problem& p = a.p;
@@ -345,45 +355,47 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         const int hsel = (warp - 2) >> 2;             // which half of the tile's columns
         const int r = q * 32 + lane;                  // accumulator row = frame within the tile
         const int t = m0 + r;
-        // labels (the rest of the parameter layer; bad labels are clamped here and reported by the metadata CTA)
-        int L;
-        if (p.label_len) {
-            long long l64 = load_as_int(p.label_len, p.label_len_dtype, b);
-            l64 = l64 < 0 ? 0 : (l64 > p.Lmax ? p.Lmax : l64);
-            L = (int)l64;
-        } else {
-            for (int j = etid; j < p.Lmax; j += NE)
-                if (load_as_int(p.labels, p.label_dtype, b * p.lst_b + j * p.lst_l) == p.label_pad) atomicMin(&s_L, j);
-            bar_sync_epilogue();
-            L = s_L;
-        }
-        for (int j = etid; j < L; j += NE) {
-            const long long v = load_as_int(p.labels, p.label_dtype, b * p.lst_b + j * p.lst_l);
-            labs[j] = (int)(v < 0 ? 0 : (v >= p.V ? p.V - 1 : v));
-        }
-        bar_sync_epilogue();
-        // the lattice's columns (0 = blank, j = label j) bucketed by the half tile (128 symbols) their symbol lies in, the
-        // buckets of the lower column halves first (key = half * NT + tile): an epilogue warp visits exactly its own
-        // columns of a tile, and all the columns a thread parks are one contiguous range of `order`
-        for (int h = etid; h <= 2 * a.NT; h += NE) {
-            int c = 0;
-            for (int j = 0; j <= L; ++j) { const int hb = (j == 0 ? p.blank : labs[j - 1]) >> 7; c += ((hb & 1) * a.NT + (hb >> 1)) < h; }
-            hstart[h] = c;
-        }
-        for (int j = etid; j <= L; j += NE) {
-            const int hb = (j == 0 ? p.blank : labs[j - 1]) >> 7;
-            const int key = (hb & 1) * a.NT + (hb >> 1);
-            int pos = 0;
-            for (int k = 0; k <= L; ++k) {
-                const int hk = (k == 0 ? p.blank : labs[k - 1]) >> 7;
-                const int kk = (hk & 1) * a.NT + (hk >> 1);
-                pos += (kk < key) | ((kk == key) & (k < j));
+        if constexpr (LOSS) {
+            // labels (the rest of the parameter layer; bad labels are clamped here and reported by the metadata CTA)
+            int L;
+            if (p.label_len) {
+                long long l64 = load_as_int(p.label_len, p.label_len_dtype, b);
+                l64 = l64 < 0 ? 0 : (l64 > p.Lmax ? p.Lmax : l64);
+                L = (int)l64;
+            } else {
+                for (int j = etid; j < p.Lmax; j += NE)
+                    if (load_as_int(p.labels, p.label_dtype, b * p.lst_b + j * p.lst_l) == p.label_pad) atomicMin(&s_L, j);
+                bar_sync_epilogue();
+                L = s_L;
             }
-            order[pos] = j;
+            for (int j = etid; j < L; j += NE) {
+                const long long v = load_as_int(p.labels, p.label_dtype, b * p.lst_b + j * p.lst_l);
+                labs[j] = (int)(v < 0 ? 0 : (v >= p.V ? p.V - 1 : v));
+            }
+            bar_sync_epilogue();
+            // the lattice's columns (0 = blank, j = label j) bucketed by the half tile (128 symbols) their symbol lies in, the
+            // buckets of the lower column halves first (key = half * NT + tile): an epilogue warp visits exactly its own
+            // columns of a tile, and all the columns a thread parks are one contiguous range of `order`
+            for (int h = etid; h <= 2 * a.NT; h += NE) {
+                int c = 0;
+                for (int j = 0; j <= L; ++j) { const int hb = (j == 0 ? p.blank : labs[j - 1]) >> 7; c += ((hb & 1) * a.NT + (hb >> 1)) < h; }
+                hstart[h] = c;
+            }
+            for (int j = etid; j <= L; j += NE) {
+                const int hb = (j == 0 ? p.blank : labs[j - 1]) >> 7;
+                const int key = (hb & 1) * a.NT + (hb >> 1);
+                int pos = 0;
+                for (int k = 0; k <= L; ++k) {
+                    const int hk = (k == 0 ? p.blank : labs[k - 1]) >> 7;
+                    const int kk = (hk & 1) * a.NT + (hk >> 1);
+                    pos += (kk < key) | ((kk == key) & (k < j));
+                }
+                order[pos] = j;
+            }
+            bar_sync_epilogue();
         }
-        bar_sync_epilogue();
 
-        float* lrow = (a.store == 2 && t < p.T) ? a.logits + (long long)b * p.st_b + (long long)t * p.st_t : nullptr;
+        float* lrow = (LOSS && a.store == 2 && t < p.T) ? a.logits + (long long)b * p.st_b + (long long)t * p.st_t : nullptr;
         // this frame's slots of the emission table (block of 8 frames, frame-minor): parked raw, finished below
         const int blk = t >> 3;
         const bool eblock = blk < w.NB && blk * kG < Tb;
@@ -426,7 +438,7 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                         x[i] = in ? __uint_as_float(v[c & 1][i]) + (a.bias ? __ldg(a.bias + col0 + i) : 0.0f) : -INFINITY;
                     }
                 }
-                if (a.store == 1 && !(a.dbg & 2)) {
+                if (LOSS && a.store == 1 && !(a.dbg & 2)) {
                     // 32 frames x 32 columns through a swizzled staging tile: row = lane, 16-byte chunk i at (i ^ row % 8)
                     const uint32_t tile = sbuf + (uint32_t)(nstored & 1) * kPStageTile;
                     if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");   // the store that read this tile two chunks ago
@@ -452,6 +464,7 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                     cm[2] = fmaxf(cm[2], x[i + 2]); cm[3] = fmaxf(cm[3], x[i + 3]);
                 }
                 const float cmx = fmaxf(fmaxf(cm[0], cm[1]), fmaxf(cm[2], cm[3]));
+                // the normaliser (kProjDecode: mx and sum are never read, and the compiler drops this)
                 if (cmx > mx) { sum *= fast_ex2((mx - cmx) * kLog2e); mx = cmx; }     // first chunk: mx = -inf -> sum (0) * 0
                 const float ms = mx * kLog2e;
                 float sp[4] = {0.0f, 0.0f, 0.0f, 0.0f};
@@ -481,24 +494,26 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                 else if (col0 < p.V) chunk(std::false_type{}, c, col0);
             }
             // the utterance's own columns in this half tile (blank, l_1..l_L): column index uniform over the warp
-            for (int k = hstart[hsel * a.NT + n]; k < hstart[hsel * a.NT + n + 1]; ++k) {
-                const int j = order[k];
-                const int vj = j == 0 ? p.blank : labs[j - 1];
-                const uint32_t raw1 = tmem_ld1(trow + (uint32_t)(vj & (HC - 1)));
-                tmem_ld_wait();
-                const float xv = __uint_as_float(raw1) + (a.bias ? __ldg(a.bias + vj) : 0.0f);
-                if (a.smem_stash) stash[j * kPM + r] = xv;
-                else if (eblock && !(a.dbg & 4)) ecol[(size_t)j * kEC] = valid ? (double)xv : 0.0;
+            if constexpr (LOSS) {
+                for (int k = hstart[hsel * a.NT + n]; k < hstart[hsel * a.NT + n + 1]; ++k) {
+                    const int j = order[k];
+                    const int vj = j == 0 ? p.blank : labs[j - 1];
+                    const uint32_t raw1 = tmem_ld1(trow + (uint32_t)(vj & (HC - 1)));
+                    tmem_ld_wait();
+                    const float xv = __uint_as_float(raw1) + (a.bias ? __ldg(a.bias + vj) : 0.0f);
+                    if (a.smem_stash) stash[j * kPM + r] = xv;
+                    else if (eblock && !(a.dbg & 4)) ecol[(size_t)j * kEC] = valid ? (double)xv : 0.0;
+                }
             }
             tc_fence_before();
             if (CTAS == 2) mbar_arrive_leader(tempty + as); else mbar_arrive(tempty + as);
         }
         // ---- the two column halves of a row meet: row max and normaliser ----
-        part[hsel * kPM + r] = make_float2(mx, sum);
+        if constexpr (LOSS) part[hsel * kPM + r] = make_float2(mx, sum);
         Top2* htop = reinterpret_cast<Top2*>(hstart + 2 * a.NT + 4);      // DECODE: [128] the upper halves' top-2 lists
         if constexpr (DECODE) { if (hsel == 1) htop[r] = tp; }
         bar_sync_epilogue();
-        {
+        if constexpr (LOSS) {
             const float2 o = part[(hsel ^ 1) * kPM + r];
             const float m2 = fmaxf(mx, o.x);           // a half without columns holds {-inf, 0}: ex2(-inf) = 0
             sum = sum * fast_ex2((mx - m2) * kLog2e) + o.y * fast_ex2((o.x - m2) * kLog2e);
@@ -516,43 +531,45 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                 a.tok[(size_t)b * p.T + t] = sym | (is_unk ? (int)0x80000000 : 0);
             }
         }
-        // ---- the frame's outputs: {row max, log2 normaliser}; the parked columns (each thread finishes the ones it
-        // parked itself) become softmax numerators relative to the final row maximum ----
-        if (hsel == 0 && valid) w.fr[(size_t)b * p.T + t] = make_float2(mx, log2f(sum));
-        if (a.smem_stash) {
-            if (eblock) {
+        if constexpr (LOSS) {
+            // ---- the frame's outputs: {row max, log2 normaliser}; the parked columns (each thread finishes the ones it
+            // parked itself) become softmax numerators relative to the final row maximum ----
+            if (hsel == 0 && valid) w.fr[(size_t)b * p.T + t] = make_float2(mx, log2f(sum));
+            if (a.smem_stash) {
+                if (eblock) {
+                    bool floored = false;
+                    for (int k = hstart[hsel * a.NT]; k < hstart[(hsel + 1) * a.NT]; ++k) {
+                        const int j = order[k];
+                        const float l2 = (stash[j * kPM + r] - mx) * kLog2e;
+                        floored |= valid && l2 < kMinLog2;
+                        ecol[(size_t)j * kEC] = valid ? (double)fast_ex2(fmaxf(l2, kMinLog2)) : 0.0;
+                    }
+                    if (floored && p.status) atomicOr(p.status + b, UTT_WIDE_LOGITS);
+                }
+            } else if (eblock && valid && !(a.dbg & 4)) {
                 bool floored = false;
-                for (int k = hstart[hsel * a.NT]; k < hstart[(hsel + 1) * a.NT]; ++k) {
-                    const int j = order[k];
-                    const float l2 = (stash[j * kPM + r] - mx) * kLog2e;
-                    floored |= valid && l2 < kMinLog2;
-                    ecol[(size_t)j * kEC] = valid ? (double)fast_ex2(fmaxf(l2, kMinLog2)) : 0.0;
+                const int k1 = hstart[(hsel + 1) * a.NT];
+                for (int k0 = hstart[hsel * a.NT]; k0 < k1; k0 += 8) {          // eight independent round trips to L2 at a time
+                    double raw[8];
+#pragma unroll
+                    for (int i = 0; i < 8; ++i)
+                        if (k0 + i < k1) raw[i] = ecol[(size_t)order[k0 + i] * kEC];
+#pragma unroll
+                    for (int i = 0; i < 8; ++i)
+                        if (k0 + i < k1) {
+                            const float l2 = ((float)raw[i] - mx) * kLog2e;
+                            floored |= l2 < kMinLog2;
+                            ecol[(size_t)order[k0 + i] * kEC] = (double)fast_ex2(fmaxf(l2, kMinLog2));
+                        }
                 }
                 if (floored && p.status) atomicOr(p.status + b, UTT_WIDE_LOGITS);
             }
-        } else if (eblock && valid && !(a.dbg & 4)) {
-            bool floored = false;
-            const int k1 = hstart[(hsel + 1) * a.NT];
-            for (int k0 = hstart[hsel * a.NT]; k0 < k1; k0 += 8) {          // eight independent round trips to L2 at a time
-                double raw[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i)
-                    if (k0 + i < k1) raw[i] = ecol[(size_t)order[k0 + i] * kEC];
-#pragma unroll
-                for (int i = 0; i < 8; ++i)
-                    if (k0 + i < k1) {
-                        const float l2 = ((float)raw[i] - mx) * kLog2e;
-                        floored |= l2 < kMinLog2;
-                        ecol[(size_t)order[k0 + i] * kEC] = (double)fast_ex2(fmaxf(l2, kMinLog2));
-                    }
-            }
-            if (floored && p.status) atomicOr(p.status + b, UTT_WIDE_LOGITS);
+            if (a.store == 1 && lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // staging tiles are read before the CTA exits
+            // this tile's rows of `fr` and E are written: tell a recursion kernel that runs beside this one
+            __threadfence();
+            bar_sync_epilogue();
+            if (etid == 0) st_release_gpu(w.tflag + (size_t)b * w.ntile + mt, 1);
         }
-        if (a.store == 1 && lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // staging tiles are read before the CTA exits
-        // this tile's rows of `fr` and E are written: tell a recursion kernel that runs beside this one
-        __threadfence();
-        bar_sync_epilogue();
-        if (etid == 0) st_release_gpu(w.tflag + (size_t)b * w.ntile + mt, 1);
     }
     tc_fence_before();
     if (CTAS == 2) cluster_sync_all(); else __syncthreads();      // a pair: nobody leaves while its peer may still signal it

@@ -19,9 +19,9 @@ import ctypes
 import torch
 
 from . import _lib
-from .ops import _Call, _alloc_ws, _blank_last, _on_device, _stream_ptr
+from .ops import _DT, _Call, _alloc_ws, _as_index_tensor, _blank_last, _on_device, _stream_ptr
 
-__all__ = ["proj_ctc_loss", "proj_ctc_eval", "ProjCtcLoss"]
+__all__ = ["proj_ctc_loss", "proj_ctc_eval", "proj_greedy_decode", "ProjCtcLoss"]
 
 
 def _proj_struct(hidden, weight, bias):
@@ -193,6 +193,40 @@ def proj_ctc_eval(hidden, weight, bias, label, pred_lengths=None, label_lengths=
     return loss, tokens, lengths
 
 
+def proj_greedy_decode(hidden, weight, bias, pred_lengths=None, blank=0, unk=None):
+    """Greedy decode from the encoder output without labels (decode_ctc.py:118-140: ``tgt_proj``, then the argmax with the
+    ``<unk>`` rule): ``(tokens (B,T) int32, lengths (B,) int32)`` of ``hidden @ weight.T + bias``, the logits never stored.
+
+    ``ctcb_proj_greedy_decode``: the projection's epilogue keeps each frame's best two symbols, a small kernel collapses
+    repeats and ``blank``.  ``unk``: a frame whose best symbol is ``unk`` takes its second best (``greedy_decode``'s rule).
+    Tokens and lengths are bit-identical to those of ``proj_ctc_eval`` for the same operands, lengths, blank and ``unk``,
+    whatever its labels.  Any vocabulary size (no lattice, so no V > 64 condition).  fp32 (tf32 product) or bfloat16
+    operands; no autograd graph.  The outputs go straight into ``edit_distance``."""
+    _check_inputs(hidden, weight, bias)
+    if hidden.stride(2) != 1:
+        hidden = hidden.contiguous()
+    weight = weight.detach().contiguous()
+    bias = bias.detach().contiguous() if bias is not None else None
+    B, T, _ = hidden.shape
+    V = weight.shape[0]
+    dev = hidden.device
+    pl = _as_index_tensor(pred_lengths, dev, "pred_lengths")
+    if pl is not None:
+        if pl.dim() != 1 or pl.shape[0] != B:
+            raise ValueError("pred_lengths must have shape (%d,)" % B)
+        pl = pl.contiguous()
+    tokens = torch.empty((B, T), dtype=torch.int32, device=dev)
+    lengths = torch.empty((B,), dtype=torch.int32, device=dev)
+    pj = _proj_struct(hidden, weight, bias)
+    with _on_device(dev):
+        rc = _lib.load().ctcb_proj_greedy_decode(ctypes.byref(pj), T, B, V, pl.data_ptr() if pl is not None else None,
+                                                 _DT[pl.dtype] if pl is not None else 0, int(blank),
+                                                 -1 if unk is None else int(unk), tokens.data_ptr(), lengths.data_ptr(),
+                                                 _stream_ptr(dev))
+    _lib.check(rc)
+    return tokens, lengths
+
+
 class ProjCtcLoss(torch.nn.Module):
     """``tgt_proj`` + ``CtcLoss`` as one block: holds the Dense parameters (units=V, in_units=K) in gluon's layout."""
 
@@ -211,3 +245,9 @@ class ProjCtcLoss(torch.nn.Module):
         """``proj_ctc_eval`` with this block's parameters: (loss, tokens, lengths), the logits never stored."""
         return proj_ctc_eval(hidden, self.weight, self.bias, label, pred_lengths, label_lengths, self.blank_label,
                              self.label_layout, unk)
+
+    def decode(self, hidden, pred_lengths=None, unk=None):
+        """``proj_greedy_decode`` with this block's parameters and blank (0, or V - 1 for ``blank_label="last"``):
+        (tokens, lengths) without labels, the logits never stored."""
+        blank = self.weight.shape[0] - 1 if _blank_last(self.blank_label) else 0
+        return proj_greedy_decode(hidden, self.weight, self.bias, pred_lengths, blank, unk)

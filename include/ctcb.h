@@ -345,6 +345,18 @@ int ctcb_proj_forward(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t 
 int ctcb_proj_forward_decode(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t keep_for_backward, int32_t unk,
                              int32_t* out_tokens, int32_t* out_lengths, void* workspace, size_t workspace_bytes,
                              void* stream);
+/* Greedy decode from the encoder output WITHOUT labels (decode_ctc.py:118-140: `tgt_proj`, then the argmax with the <unk>
+ * rule): ctcb_greedy_decode_typed's arguments with the projection in place of the logits.  The projection's epilogue keeps
+ * each frame's best and second best symbol of the logits it forms, a second kernel collapses repeats and blanks; the logits
+ * never reach HBM, no workspace, 2 launches.  Frame counts = data_lengths (data_lengths_dtype; truncated and clamped to
+ * [0, T]) or T when NULL; unk = -1 (or below) for no <unk> rule.  out_tokens (B, T) int32, hypothesis prefix then zeros;
+ * out_lengths (B,) int32.  Tokens and lengths are bit-identical to ctcb_proj_forward_decode's for the same projection,
+ * lengths, blank and unk, whatever its labels (the same tiles in the same K order), hence to ctcb_greedy_decode_unk on the
+ * logits ctcb_proj_forward stores.  Any V >= 1: no V > 64 / Lmax restriction (there is no lattice).  Device buffers;
+ * CTCB_UNSUPPORTED for T too long for the collapse kernel (2 T ints <= 200 KB).  Detected by symbol. */
+int ctcb_proj_greedy_decode(const ctcb_proj_t* proj, int32_t T, int32_t B, int32_t V,
+                            const void* data_lengths, int32_t data_lengths_dtype,
+                            int32_t blank, int32_t unk, int32_t* out_tokens, int32_t* out_lengths, void* stream);
 /* ctcb_proj_forward(keep_for_backward=1) followed by ctcb_backward in one call: loss, p->logits and p->grad. */
 int ctcb_proj_loss_grad(const ctcb_proj_t* proj, const ctcb_problem_t* p, void* workspace, size_t workspace_bytes,
                         void* stream);
