@@ -30,7 +30,7 @@ EXPORTS = (
     "ctcb_set_option", "ctcb_get_option", "ctcb_greedy_decode_unk", "ctcb_last_grad_kernel",
     "ctcb_proj_forward", "ctcb_proj_loss_grad",
     "ctcb_loss_grad_typed", "ctcb_forward_typed", "ctcb_backward_typed", "ctcb_greedy_decode_typed",
-    "ctcb_proj_forward_decode", "ctcb_proj_greedy_decode",
+    "ctcb_proj_forward_decode", "ctcb_proj_greedy_decode", "ctcb_proj_backward",
 )
 
 
@@ -113,6 +113,7 @@ def load():
     lib.ctcb_loss_grad_dlpack.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, vp, sz, vp]
     lib.ctcb_proj_forward.argtypes = [ctypes.POINTER(Proj), PP, i32, vp, sz, vp]
     lib.ctcb_proj_loss_grad.argtypes = [ctypes.POINTER(Proj), PP, vp, sz, vp]
+    lib.ctcb_proj_backward.argtypes = [ctypes.POINTER(Proj), PP, vp, sz, vp]
     lib.ctcb_proj_forward_decode.argtypes = [ctypes.POINTER(Proj), PP, i32, i32, vp, vp, vp, sz, vp]
     lib.ctcb_proj_greedy_decode.argtypes = [ctypes.POINTER(Proj), i32, i32, i32, vp, i32, i32, i32, vp, vp, vp]
     lib.ctcb_set_option.argtypes = [ctypes.c_char_p, i32]

@@ -55,6 +55,7 @@ bool launch_pending_xchg(cudaStream_t stream, bool programmatic = false) {
 thread_local const ctcb_proj_t* g_proj = nullptr;      // ctcb_proj_*: the projection whose epilogue replaces k_emit in this call
 struct DecodeRequest { int32_t* tokens; int32_t* lengths; int unk; };
 thread_local const DecodeRequest* g_decode = nullptr;  // ctcb_proj_forward_decode: the greedy decode the projection's epilogue adds
+thread_local bool g_recompute = false;                 // ctcb_proj_forward(keep_for_backward, no logits): the occupancy table follows
 thread_local cudaEvent_t* g_prof_events = nullptr;   // when set: one event recorded after every launch
 thread_local int g_prof_count = 0;
 
@@ -686,6 +687,11 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
             if (int rc = launch_proj(g_proj, p, dp, w, lay, stream, beside)) return rc;
         } else if (!lay.fused) { if (int rc = launch_emit()) return rc; }
         if (int rc = launch_walk((xchg && lay.fused != 0) || beside, beside)) return rc;
+        if (g_recompute) {
+            // the recomputing training forward: the history becomes the occupancy table O that ctcb_proj_backward reads
+            CUDA_TRY(ctcb::launch_proj_occ(dp, w, stream));
+            mark(stream);
+        }
         if (g_decode) {
             // the hypotheses from the projection's per-frame words (an ordinary launch: it acquires the tile flags itself)
             const size_t dsm = 2 * sizeof(int) * (size_t)p->T;
@@ -843,12 +849,14 @@ int ctcb_backward_typed(const ctcb_problem_t* p, int32_t logits_dtype, void* wor
 int ctcb_proj_forward(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t keep_for_backward, void* workspace,
                       size_t workspace_bytes, void* stream) {
     if (!proj) return fail(CTCB_INVALID_VALUE, "proj is NULL");
-    if (keep_for_backward && p && !p->logits)
-        return fail(CTCB_INVALID_VALUE, "keep_for_backward needs p->logits (the gradient kernel reads the projection's output)");
     g_launches = 0;
     g_proj = proj;
+    // keep_for_backward without a logits buffer: the history is kept and turned into the occupancy table, the logits are
+    // never stored, and ctcb_proj_backward forms the product again
+    g_recompute = keep_for_backward && p && !p->logits;
     const int rc = enqueue(p, workspace, workspace_bytes, stream, PH_FORWARD, keep_for_backward != 0);
     g_proj = nullptr;
+    g_recompute = false;
     return rc;
 }
 
@@ -911,6 +919,55 @@ int ctcb_proj_loss_grad(const ctcb_proj_t* proj, const ctcb_problem_t* p, void* 
     const int rc = enqueue(p, workspace, workspace_bytes, stream, PH_FORWARD | PH_BACKWARD, true);
     g_proj = nullptr;
     return rc;
+}
+
+int ctcb_proj_backward(const ctcb_proj_t* proj, const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream_) {
+    g_launches = 0;
+    if (!proj) return fail(CTCB_INVALID_VALUE, "proj is NULL");
+    g_proj = proj;                                  // validate: the logits pointer is not needed
+    const int vrc = validate(p);
+    g_proj = nullptr;
+    if (vrc) return vrc;
+    if (!p->grad) return fail(CTCB_INVALID_VALUE, "grad is NULL");
+    const Layout lay = make_layout(p->T, p->B, p->V, p->Lmax, 1);
+    if (lay.fused || lay.dense)
+        return fail(CTCB_UNSUPPORTED, "projection fused with the loss needs V > 64 and V > Lmax + 1 (V=%d, Lmax=%d)", p->V, p->Lmax);
+    if (p->logits_row_offsets) return fail(CTCB_UNSUPPORTED, "projection: packed logits are not supported");
+    if (!workspace) return fail(CTCB_INVALID_VALUE, "workspace is NULL");
+    if (workspace_bytes < lay.total)
+        return fail(CTCB_WORKSPACE_TOO_SMALL, "workspace %zu < required %zu bytes", workspace_bytes, lay.total);
+    if (reinterpret_cast<uintptr_t>(workspace) % 256) return fail(CTCB_INVALID_VALUE, "workspace must be 256-byte aligned");
+    if (!is_device_ptr(workspace) || !is_device_ptr(p->grad) || !is_device_ptr(p->labels) || !is_device_ptr(p->head_grad))
+        return fail(CTCB_INVALID_VALUE, "labels/grad/head_grad/workspace must be CUDA device memory (there is no CPU path)");
+    if (!proj->hidden || !proj->weight || proj->K <= 0) return fail(CTCB_INVALID_VALUE, "projection: hidden / weight is NULL or K <= 0");
+    if (int rc = check_proj_operands(proj)) return rc;
+    const int ctas = proj_ctas();
+    const int NT = (p->V + ctcb::kPN - 1) / ctcb::kPN;
+    const size_t smem = ctcb::proj_smem_bytes(p->Lmax, lay.Lp, true, NT, ctas);
+    if (smem > 232448 - 64) return fail(CTCB_UNSUPPORTED, "projection: Lmax=%d label columns do not fit the kernel's shared memory", p->Lmax);
+    CUtensorMap tmA, tmB;
+    if (int rc = encode_proj_maps(proj, p->T, p->B, p->V, ctas, &tmA, &tmB)) return rc;
+    ctcb::ProjArgs pa = proj_args(proj, p->V, ctas);
+    pa.p = to_device_problem(p);
+    pa.w = carve(lay, workspace);
+    // G leaves through TMA tile stores when its rows allow a tensor map, else as coalesced rows from the staging tiles
+    CUtensorMap tmC = tmA;
+    pa.store = 2;
+    if (p->grad_stride_t % 4 == 0 && p->grad_stride_b % 4 == 0 && reinterpret_cast<uintptr_t>(p->grad) % 16 == 0) {
+        const cuuint64_t gdim[3] = {(cuuint64_t)p->V, (cuuint64_t)p->T, (cuuint64_t)p->B};
+        const cuuint64_t gstr[2] = {(cuuint64_t)p->grad_stride_t * 4, (cuuint64_t)p->grad_stride_b * 4};
+        const cuuint32_t box[3] = {32, 32, 1};
+        const cuuint32_t est[3] = {1, 1, 1};
+        const CUresult r = encode_tiled()(&tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, p->grad, gdim, gstr, box, est,
+                                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r == CUDA_SUCCESS) pa.store = 1;
+    }
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    const int mtiles = (p->T + ctcb::kPM - 1) / ctcb::kPM;
+    CUDA_TRY(ctcb::launch_proj_emit(tmA, tmB, tmC, pa, ctcb::kProjGrad, dim3(ctas, p->B, (mtiles + ctas - 1) / ctas), smem, stream, false));
+    mark(stream);
+    return CTCB_OK;
 }
 
 // ---- host-buffer entry ------------------------------------------------------------------

@@ -9,14 +9,14 @@ cudaError_t launch_proj_emit(const CUtensorMap& tmA, const CUtensorMap& tmB, con
                              size_t smem, cudaStream_t stream, bool programmatic) {
     // the opt-in shared-memory size is a per-device function attribute: raised when a launch needs more than any before
     static thread_local int done_dev = -1;
-    static thread_local size_t done_bytes[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    static thread_local size_t done_bytes[16] = {};
     int dev = 0;
     cudaGetDevice(&dev);
     if (done_dev != dev) { done_dev = dev; for (size_t& d : done_bytes) d = 0; }
     const int pair = a.ctas == 2 ? 1 : 0, bf = a.bf16 ? 1 : 0, which = mode * 4 + pair * 2 + bf;
     using Fn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, ProjArgs);
 #define PROJ_MODE(M_) k_proj_emit<1, false, M_>, k_proj_emit<1, true, M_>, k_proj_emit<2, false, M_>, k_proj_emit<2, true, M_>
-    static const Fn fns[12] = {PROJ_MODE(kProjLoss), PROJ_MODE(kProjLossDecode), PROJ_MODE(kProjDecode)};
+    static const Fn fns[16] = {PROJ_MODE(kProjLoss), PROJ_MODE(kProjLossDecode), PROJ_MODE(kProjDecode), PROJ_MODE(kProjGrad)};
 #undef PROJ_MODE
     const Fn fn = fns[which];
     if (done_bytes[which] < smem) {
@@ -41,6 +41,12 @@ cudaError_t launch_proj_emit(const CUtensorMap& tmA, const CUtensorMap& tmB, con
     cfg.attrs = attr; cfg.numAttrs = na;
     const cudaError_t rc = cudaLaunchKernelEx(&cfg, fn, tmA, tmB, tmC, a);
     if (rc != cudaSuccess) return rc;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_proj_occ(const Problem& p, const Workspace& w, cudaStream_t stream) {
+    const dim3 grid(p.B, (w.NB + kOccBlocksPerCta - 1) / kOccBlocksPerCta);
+    k_proj_occ<<<grid, kOccThreads, 0, stream>>>(p, w);
     return cudaGetLastError();
 }
 

@@ -61,6 +61,7 @@ struct ProjArgs {
     int K, NT, KB;           // hidden units, vocabulary tiles, K blocks
     int vec4;                // bias allows 16-byte loads
     int store;               // 0: logits not stored; 1: TMA store through the staging tiles; 2: direct scalar stores
+                             //   (kProjGrad: the gradient, 1 = TMA store, 2 = coalesced row stores from the staging tiles)
     int smem_stash;          // the label columns are parked in shared memory (store == 0 and they fit), else in E
     int ctas;                // 1: one CTA per tile; 2: CTA pairs (tcgen05 cta_group::2) over 256 frames
     int bf16;                // operands are bfloat16 (64 values per 128-byte K block, kind::f16) instead of fp32 (32, kind::tf32)
@@ -86,7 +87,17 @@ __host__ __device__ inline size_t proj_smem_bytes(int Lmax, int Lp, bool store, 
 }
 
 // what k_proj_emit's epilogue computes (its MODE, see there)
-enum : int { kProjLoss = 0, kProjLossDecode = 1, kProjDecode = 2 };
+enum : int { kProjLoss = 0, kProjLossDecode = 1, kProjDecode = 2, kProjGrad = 3 };
+
+// The occupancy table O of the recomputing training path (ctcb_proj_forward with keep_for_backward and no logits buffer):
+// gamma_t(j) = sum over the lattice states of column j (0 = blank, j = label j) of alpha_t(s) beta'_t(s) / P(l|x), fp32, in
+// E's frame-minor (B, NB, W, kEC) index space.  It lives in E's region: the walkers are the last readers of E, and the
+// occupancy kernel runs after them in stream order.  Written by k_proj_occ, read by k_proj_emit<..., kProjGrad>.
+__host__ __device__ inline float* proj_occ_table(const Workspace& w) { return reinterpret_cast<float*>(w.E); }
+// frame blocks per CTA of k_proj_occ (each CTA forms P(l|x) once for all of them)
+constexpr int kOccBlocksPerCta = 16;
+constexpr int kOccThreads = 256;
+constexpr int kGradOcc = 8;               // kProjGrad: occupancies of a chunk's label columns in flight per round trip
 
 // (a.ctas == 2: grid.x even, launched as clusters of two CTAs along x)
 // host-side launcher, defined in ctcb_proj.cu (its own translation unit: the kernel below is compiled there only)
@@ -94,6 +105,8 @@ enum : int { kProjLoss = 0, kProjLossDecode = 1, kProjDecode = 2 };
 // programmatic: launched with programmatic stream serialization (it starts beside the kernel enqueued before it)
 cudaError_t launch_proj_emit(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC, const ProjArgs& a, int mode, dim3 grid,
                              size_t smem, cudaStream_t stream, bool programmatic);
+// k_proj_occ over the batch (an ordinary launch: the walkers before it in the stream have completed)
+cudaError_t launch_proj_occ(const Problem& p, const Workspace& w, cudaStream_t stream);
 
 #ifdef CTCB_PROJ_IMPL
 // ---- tcgen05 / TMA wrappers -------------------------------------------------------------------------------------
@@ -231,13 +244,22 @@ __device__ __forceinline__ void bar_sync_epilogue() { asm volatile("bar.sync 1, 
 //                    order: greater value, ties to the lower index) for the frame's word of ProjArgs::tok -- the greedy
 //                    decode of the logits that are never stored;
 //   kProjDecode      the frame's word only (ctcb_proj_greedy_decode: no labels): label parsing, the label columns, the
-//                    normaliser, `fr`, E and the tile flags are compiled out, the word is the kProjLossDecode one.
+//                    normaliser, `fr`, E and the tile flags are compiled out, the word is the kProjLossDecode one;
+//   kProjGrad        d loss / d logits of the recomputing training path (ctcb_proj_backward): the product is formed again,
+//                    tile by tile, and each element becomes  head[b] * (softmax - occupancy)  with the forward's `fr` row and
+//                    the occupancy table O (proj_occ_table) -- the logits are never written or read.  The label columns of a
+//                    half tile are sorted by symbol, so those of one 32-column chunk are a contiguous run; their
+//                    occupancies are fetched while the chunk's softmax is formed and subtracted, in fp32, in the staging
+//                    tile before it leaves (TMA tile store into p.grad, or coalesced row stores when p.grad's rows do
+//                    not allow a tensor map).  Tiles of padded frames, infeasible utterances and a workspace that no
+//                    matching forward filled skip the product: zeros (NaN for the last) are written instead.
 // A compile-time switch: a run-time branch in this kernel was measured at +17 us (DESIGN.md section 5)
 template <int CTAS, bool BF16, int MODE>
 __global__ void __launch_bounds__(kPThreads, 1)
 k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmC,
             ProjArgs a) {
-    constexpr bool LOSS = MODE != kProjDecode, DECODE = MODE != kProjLoss;
+    constexpr bool LOSS = MODE == kProjLoss || MODE == kProjLossDecode, DECODE = MODE == kProjLossDecode || MODE == kProjDecode;
+    constexpr bool GRAD = MODE == kProjGrad, LABELS = LOSS || GRAD;
     extern __shared__ unsigned char proj_raw[];
     __shared__ int s_L;
     const Problem& p = a.p;
@@ -256,6 +278,24 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         long long t64 = load_as_int(p.data_len, p.data_len_dtype, b);
         t64 = t64 < 0 ? 0 : (t64 > p.T ? p.T : t64);
         Tb = (int)t64;
+    }
+    if constexpr (GRAD) {
+        // rows without a product: the tile (pair) lies beyond Tb, the utterance is infeasible (G = 0), or no matching forward
+        // filled the workspace (G = NaN, never a wait).  The words read are the utterance's, so both CTAs of a pair agree
+        const bool filled = __ldcg(w.gprog + 4 * b + 2) == w.stamp && __ldcg(w.gprog + 4 * b + 3) == w.stamp;
+        const bool zero = !filled || (CTAS == 2 ? (int)blockIdx.z * 2 * kPM : m0) >= Tb || (__ldcg(w.flags + b) & UTT_INFEASIBLE);
+        if (zero) {
+            if (warp < 2) return;
+            // the epilogue warps: a quadrant's two warps take alternate rows of its 32, all V columns, coalesced
+            const float fill = filled ? 0.0f : __int_as_float(0x7fc00000);
+            for (int rr = (warp - 2) >> 2; rr < 32; rr += 2) {
+                const int t = m0 + (warp & 3) * 32 + rr;
+                if (t >= p.T) break;
+                float* grow = p.grad + (long long)b * p.gst_b + (long long)t * p.gst_t;
+                for (int v = lane; v < p.V; v += 32) grow[v] = fill;
+            }
+            return;
+        }
     }
     // a tile of padded frames: nothing of it is ever read (a pair leaves together: its second CTA stages half of B)
     if ((CTAS == 2 ? (int)blockIdx.z * 2 * kPM : m0) >= Tb) return;
@@ -355,7 +395,7 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         const int hsel = (warp - 2) >> 2;             // which half of the tile's columns
         const int r = q * 32 + lane;                  // accumulator row = frame within the tile
         const int t = m0 + r;
-        if constexpr (LOSS) {
+        if constexpr (LABELS) {
             // labels (the rest of the parameter layer; bad labels are clamped here and reported by the metadata CTA)
             int L;
             if (p.label_len) {
@@ -382,18 +422,30 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                 hstart[h] = c;
             }
             for (int j = etid; j <= L; j += NE) {
-                const int hb = (j == 0 ? p.blank : labs[j - 1]) >> 7;
+                const int sj = j == 0 ? p.blank : labs[j - 1], hb = sj >> 7;
                 const int key = (hb & 1) * a.NT + (hb >> 1);
                 int pos = 0;
                 for (int k = 0; k <= L; ++k) {
-                    const int hk = (k == 0 ? p.blank : labs[k - 1]) >> 7;
+                    const int sk = k == 0 ? p.blank : labs[k - 1], hk = sk >> 7;
                     const int kk = (hk & 1) * a.NT + (hk >> 1);
-                    pos += (kk < key) | ((kk == key) & (k < j));
+                    // GRAD: within a bucket by symbol, then position (a chunk's columns are one run of `order`)
+                    if constexpr (GRAD) pos += (kk < key) | ((kk == key) & ((sk < sj) | ((sk == sj) & (k < j))));
+                    else pos += (kk < key) | ((kk == key) & (k < j));
                 }
                 order[pos] = j;
             }
             bar_sync_epilogue();
         }
+        // GRAD: this frame's softmax row ({row max, log2 normaliser} of the forward), head, and its slots of O
+        float2 gfr = make_float2(0.0f, 0.0f);
+        float ghead = 1.0f;
+        const float* ocol = nullptr;
+        if constexpr (GRAD) {
+            if (t < Tb) gfr = __ldcg(w.fr + (size_t)b * p.T + t);
+            ghead = p.head ? __ldg(p.head + b) : 1.0f;
+            ocol = proj_occ_table(w) + ((size_t)b * w.NB + (t < Tb ? (t >> 3) : 0)) * w.W * kEC + (t & 7);
+        }
+        int gk = 0;                                   // GRAD: the next of this half tile's label columns in `order`
 
         float* lrow = (LOSS && a.store == 2 && t < p.T) ? a.logits + (long long)b * p.st_b + (long long)t * p.st_t : nullptr;
         // this frame's slots of the emission table (block of 8 frames, frame-minor): parked raw, finished below
@@ -414,6 +466,8 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
             uint32_t v[2][32];
             if (a.dbg & 1) { tc_fence_before(); if (CTAS == 2) mbar_arrive_leader(tempty + as); else mbar_arrive(tempty + as); continue; }
             if (cbase < p.V) tmem_ld32(trow, v[0]);
+            const int gend = GRAD ? hstart[hsel * a.NT + n + 1] : 0;
+            if constexpr (GRAD) gk = hstart[hsel * a.NT + n];
             // one chunk of 32 columns; FULLC: every column lies below V (no bounds checks: all but the vocabulary's last chunks)
             auto chunk = [&](auto full_tag, const int c, const int col0) {
                 constexpr bool FULLC = decltype(full_tag)::value;
@@ -437,6 +491,61 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                         const bool in = FULLC || col0 + i < p.V;
                         x[i] = in ? __uint_as_float(v[c & 1][i]) + (a.bias ? __ldg(a.bias + col0 + i) : 0.0f) : -INFINITY;
                     }
+                }
+                if constexpr (GRAD) {
+                    // the chunk's label columns are order[gk, gk1): their occupancies travel while the softmax is formed
+                    auto sym = [&](int j) { return j == 0 ? p.blank : labs[j - 1]; };
+                    int gk1 = gk;
+                    while (gk1 < gend && sym(order[gk1]) < col0 + 32) ++gk1;
+                    float ov[kGradOcc];
+#pragma unroll
+                    for (int i = 0; i < kGradOcc; ++i) ov[i] = (valid && gk + i < gk1) ? __ldcg(ocol + (size_t)order[gk + i] * kEC) : 0.0f;
+                    // head * softmax, k_grad's arithmetic (padded rows: 0; columns >= V: ex2(-inf) = 0)
+#pragma unroll
+                    for (int i = 0; i < 32; ++i) x[i] = valid ? ghead * fast_ex2(fmaf(x[i] - gfr.x, kLog2e, -gfr.y)) : 0.0f;
+                    const uint32_t tile = sbuf + (uint32_t)(nstored & 1) * kPStageTile;
+                    if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");   // the store that read this tile two chunks ago
+                    __syncwarp();
+#pragma unroll
+                    for (int i = 0; i < 8; ++i)
+                        asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};"
+                                     ::"r"(tile + (uint32_t)lane * 128u + (uint32_t)((i ^ (lane & 7)) << 4)),
+                                       "f"(x[4 * i]), "f"(x[4 * i + 1]), "f"(x[4 * i + 2]), "f"(x[4 * i + 3]) : "memory");
+                    // minus head * occupancy in the thread's own row (a repeated symbol: once per lattice column)
+                    float* trowp = reinterpret_cast<float*>(gbase + (tile - base)) + lane * 32;
+                    for (int k0 = gk; k0 < gk1; k0 += kGradOcc) {
+                        if (k0 != gk) {
+#pragma unroll
+                            for (int i = 0; i < kGradOcc; ++i) ov[i] = (valid && k0 + i < gk1) ? __ldcg(ocol + (size_t)order[k0 + i] * kEC) : 0.0f;
+                        }
+#pragma unroll
+                        for (int i = 0; i < kGradOcc; ++i)
+                            if (k0 + i < gk1) {
+                                const int ci = sym(order[k0 + i]) - col0;
+                                float* e = trowp + (((ci >> 2) ^ (lane & 7)) << 2) + (ci & 3);
+                                *e = fmaf(-ghead, ov[i], *e);
+                            }
+                    }
+                    gk = gk1;
+                    if (a.store == 1) {
+                        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                        __syncwarp();
+                        if (lane == 0) tma_store_3d(&tmC, tile, col0, m0 + q * 32, b);
+                    } else {
+                        // rows whose strides allow no tensor map: the warp writes the tile row by row, 128 bytes at a time
+                        __syncwarp();
+                        const float* tf = reinterpret_cast<const float*>(gbase + (tile - base));
+                        for (int rr = 0; rr < 32; ++rr) {
+                            const int t2 = m0 + q * 32 + rr;
+                            if (t2 >= p.T) break;
+                            if (FULLC || col0 + lane < p.V)
+                                p.grad[(long long)b * p.gst_b + (long long)t2 * p.gst_t + col0 + lane] =
+                                    tf[rr * 32 + ((((lane >> 2) ^ (rr & 7))) << 2) + (lane & 3)];
+                        }
+                        __syncwarp();
+                    }
+                    ++nstored;
+                    return;
                 }
                 if (LOSS && a.store == 1 && !(a.dbg & 2)) {
                     // 32 frames x 32 columns through a swizzled staging tile: row = lane, 16-byte chunk i at (i ^ row % 8)
@@ -508,6 +617,7 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
             tc_fence_before();
             if (CTAS == 2) mbar_arrive_leader(tempty + as); else mbar_arrive(tempty + as);
         }
+        if constexpr (GRAD) { if (a.store == 1 && lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }   // tiles read before exit
         // ---- the two column halves of a row meet: row max and normaliser ----
         if constexpr (LOSS) part[hsel * kPM + r] = make_float2(mx, sum);
         Top2* htop = reinterpret_cast<Top2*>(hstart + 2 * a.NT + 4);      // DECODE: [128] the upper halves' top-2 lists
@@ -574,6 +684,130 @@ k_proj_emit(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     tc_fence_before();
     if (CTAS == 2) cluster_sync_all(); else __syncthreads();      // a pair: nobody leaves while its peer may still signal it
     if (warp == 1) { if (CTAS == 2) tmem_dealloc_pair(tmem, kPTmemCols); else tmem_dealloc(tmem, kPTmemCols); }
+}
+
+// k_proj_occ: the occupancy table O (proj_occ_table) from the walkers' α/β' history, the last kernel of the recomputing
+// training forward.  grid (B, ceil(NB / kOccBlocksPerCta)), kOccThreads threads; it runs after the walkers in stream order.
+// k_grad2's normalisation, with one prologue per CTA instead of one per frame block: warp 0 forms P(l|x) from the
+// utterance's frame 0 (exact integer exponents, fp64 sum) as {exponent EP, 1 / mantissa}; a state's occupancy is then
+// its stored alpha high word with the block's exponent shift (both walkers' offsets minus EP) added as an integer, one DMUL
+// with beta's high word, times 1 / mantissa.  A warp takes whole frame blocks: lane g holds state pair g -- the blank state
+// 2g, summed over the warp into column 0, and the label state 2g+1, column g+1 -- forms the pair's shift once per block and
+// then covers the block's kG frames with all their history loads in flight.  Padded frames, columns beyond the utterance's
+// labels and infeasible utterances get zeros.  The CTA of the first blocks stamps gprog word 3 (zeroed by every forward's
+// metadata kernel) for ctcb_proj_backward.
+__global__ void __launch_bounds__(kOccThreads) k_proj_occ(Problem p, Workspace w) {
+    constexpr unsigned FULL = 0xffffffffu;
+    const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    __shared__ int s_EP;
+    __shared__ float s_rP;
+    float* O = proj_occ_table(w);
+    const int Tb = __ldcg(w.Tb + b), Lb = __ldcg(w.Lb + b);
+    const bool infeasible = (__ldcg(w.flags + b) & UTT_INFEASIBLE) != 0;
+    const int NQ = infeasible ? 0 : (Tb + kG - 1) / kG;
+    const int pairs = 32 * w.P * w.NW;
+    const int blk0 = (int)blockIdx.y * kOccBlocksPerCta, blk1 = min(blk0 + kOccBlocksPerCta, w.NB);
+    if (warp == 0 && blk0 < NQ) {
+        // ---- P(l|x) = sum_s alpha_0(s) beta'_0(s), k_grad2's prologue over any number of state pairs ----
+        const int2* hA0 = w.hA + (size_t)b * w.NB * kG * pairs;
+        const int2* hB0 = w.hB + (size_t)b * w.NB * kG * pairs;
+        const int2* oA = w.oA + (size_t)b * w.NB * pairs;
+        const int2* oB = w.oB + (size_t)b * w.NB * pairs;
+        auto term = [&](int g, int& exb, float& mb, int& exl, float& ml) {
+            const int ib = Lb - g, il = max(Lb - 1 - g, 0);
+            const int2 av = __ldcg(hA0 + g), oa = __ldcg(oA + g);
+            const int hb = __ldcg(&hB0[ib].x), hl = __ldcg(&hB0[il].y);
+            const int ob = __ldcg(&oB[ib].x), ol = __ldcg(&oB[il].y);
+            const bool vb = av.x != 0 && hb != 0, vl = g < Lb && av.y != 0 && hl != 0;
+            exb = vb ? (av.x >> 20) + (hb >> 20) - 2046 + oa.x + ob : INT_MIN / 2;
+            exl = vl ? (av.y >> 20) + (hl >> 20) - 2046 + oa.y + ol : INT_MIN / 2;
+            mb = vb ? hw_mant(av.x) * hw_mant(hb) : 0.0f;
+            ml = vl ? hw_mant(av.y) * hw_mant(hl) : 0.0f;
+        };
+        int emax = INT_MIN / 2;
+        for (int g = lane; g <= Lb; g += 32) {
+            int eb, el; float mb, ml;
+            term(g, eb, mb, el, ml);
+            emax = max(emax, max(eb, el));
+        }
+        emax = __reduce_max_sync(FULL, emax);
+        double s = 0.0;
+        for (int g = lane; g <= Lb; g += 32) {
+            int eb, el; float mb, ml;
+            term(g, eb, mb, el, ml);
+            s += (double)mb * pow2c(max(eb - emax, -2000));
+            s += (double)ml * pow2c(max(el - emax, -2000));
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1)
+            s += __hiloint2double(__shfl_xor_sync(FULL, __double2hiint(s), o), __shfl_xor_sync(FULL, __double2loint(s), o));
+        if (lane == 0) { s_EP = emax + dexp(s); s_rP = (float)(1.0 / dmant(s)); }
+    }
+    __syncthreads();
+    const int EP = s_EP;
+    const float rP = s_rP;
+#pragma unroll 1
+    for (int blk = blk0 + warp; blk < blk1; blk += kOccThreads / 32) {
+        float* ob = O + ((size_t)b * w.NB + blk) * w.W * kEC;
+        if (blk >= NQ) {
+            for (int j = lane; j < w.W; j += 32)
+#pragma unroll
+                for (int f = 0; f < kG; ++f) ob[(size_t)j * kEC + f] = 0.0f;
+            continue;
+        }
+        const size_t blkoff = (size_t)b * w.NB + blk;
+        const int2* hA0 = w.hA + blkoff * kG * pairs;
+        const int2* hB0 = w.hB + blkoff * kG * pairs;
+        const int2* oA = w.oA + blkoff * pairs;
+        const int2* oB = w.oB + blkoff * pairs;
+        const int t_first = blk * kG;
+        float zb[kG];
+#pragma unroll
+        for (int f = 0; f < kG; ++f) zb[f] = 0.0f;
+        for (int g = lane; g < w.W; g += 32) {
+            float zl[kG];
+#pragma unroll
+            for (int f = 0; f < kG; ++f) zl[f] = 0.0f;
+            if (g <= Lb) {
+                const int ib = Lb - g, il = max(Lb - 1 - g, 0);
+                const int2 oa = __ldcg(oA + g);
+                const int db = min(max(oa.x + __ldcg(&oB[ib].x) - EP, -2047), 2047);
+                const int dl = min(max(oa.y + __ldcg(&oB[il].y) - EP, -2047), 2047);
+                const int dsb = db * (1 << 20), dsl = g < Lb ? dl * (1 << 20) : INT_MIN;
+                int2 av[kG]; int hb[kG], hl[kG];
+#pragma unroll
+                for (int f = 0; f < kG; ++f) {
+                    const bool live = t_first + f < Tb;
+                    av[f] = live ? __ldcg(hA0 + (size_t)f * pairs + g) : make_int2(0, 0);
+                    hb[f] = live ? __ldcg(&hB0[(size_t)f * pairs + ib].x) : 0;
+                    hl[f] = live ? __ldcg(&hB0[(size_t)f * pairs + il].y) : 0;
+                }
+#pragma unroll
+                for (int f = 0; f < kG; ++f) {
+                    // k_grad2's occupancy: an exact zero stays zero, a value that leaves the normal range is flushed
+                    int tb = av[f].x != 0 ? (int)((unsigned)av[f].x + (unsigned)dsb) : 0;
+                    int tl = av[f].y != 0 ? (int)((unsigned)av[f].y + (unsigned)dsl) : 0;
+                    tb = tb < (1 << 20) ? 0 : tb; tl = tl < (1 << 20) ? 0 : tl;
+                    zb[f] += (float)(__hiloint2double(tb, 0) * __hiloint2double(tb ? hb[f] : 0, 0));
+                    zl[f] = (float)(__hiloint2double(tl, 0) * __hiloint2double(tl ? hl[f] : 0, 0)) * rP;
+                }
+            }
+            if (g + 1 < w.W) {
+#pragma unroll
+                for (int f = 0; f < kG; ++f) ob[(size_t)(g + 1) * kEC + f] = zl[f];
+            }
+        }
+#pragma unroll
+        for (int f = 0; f < kG; ++f) zb[f] = warp_sum(zb[f]);
+        if (lane == 0) {
+#pragma unroll
+            for (int f = 0; f < kG; ++f) ob[f] = zb[f] * rP;
+        }
+    }
+    if (blockIdx.y == 0 && tid == 0) {
+        __threadfence();
+        st_release_gpu(w.gprog + 4 * b + 3, w.stamp);
+    }
 }
 
 #endif  // CTCB_PROJ_IMPL

@@ -11,6 +11,11 @@ epilogue produces what the lattice recursion reads; the logits are written once 
 gradient is needed and NOT AT ALL otherwise (``torch.no_grad()`` / validation).  The backward forms
 d loss / d logits with ``ctcb_backward`` and then the three plain contractions (d hidden = G W, d weight = G^T hidden,
 d bias = sum G) with torch.matmul -- library GEMMs, plumbing.  No CPU path.
+
+``fused_training="recompute"`` trains without the logits: the forward keeps the lattice history and turns it into a
+table of label-column occupancies (no logits buffer), and the backward's ``ctcb_proj_backward`` forms the product again
+on the tensor cores and writes G directly from it -- the logits are never written or read.  The same three
+contractions follow.
 """
 from __future__ import annotations
 
@@ -64,6 +69,7 @@ class _tf32_matmul:
 class _ProjCtcLossFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, hidden, weight, bias, label, pred_lengths, label_lengths, blank_last, tn, fused=True):
+        # fused: False (library product + CtcLoss), True (fused forward with a logits store) or "recompute"
         _check_inputs(hidden, weight, bias)
         if hidden.stride(2) != 1:
             hidden = hidden.contiguous()
@@ -73,14 +79,15 @@ class _ProjCtcLossFn(torch.autograd.Function):
         V = weight.shape[0]
         dev = hidden.device
         need = any(ctx.needs_input_grad[:3])
+        recompute = need and fused == "recompute"        # no logits: the backward forms the product again
         # the logits buffer exists only when a gradient will be asked for (NTC, like the model's output)
-        if hidden.dtype == torch.bfloat16:
+        if hidden.dtype == torch.bfloat16 and not recompute:
             fused = True              # no library GEMM gives fp32 logits from bfloat16 operands without a rounding in between
         if need and not fused:
             with _tf32_matmul():      # the library product, written once: what the gradient kernel reads
                 logits = torch.nn.functional.linear(hidden, weight, bias)
         else:
-            logits = torch.empty((B, T, V), dtype=torch.float32, device=dev) if need else None
+            logits = torch.empty((B, T, V), dtype=torch.float32, device=dev) if need and not recompute else None
         shape_only = logits if logits is not None else torch.empty((B, T, V), dtype=torch.float32, device="meta")
         call = _Call(_MetaLogits(shape_only, dev), label, pred_lengths, label_lengths, blank_last, True, tn)
         loss = torch.empty((B,), dtype=torch.float32, device=dev)
@@ -97,21 +104,33 @@ class _ProjCtcLossFn(torch.autograd.Function):
                                                    _stream_ptr(dev))
         _lib.check(rc)
         ctx.call, ctx.ws, ctx.logits = call, (ws if need else None), logits
-        ctx.save_for_backward(hidden, weight)
+        ctx.recompute = recompute
+        ctx.save_for_backward(hidden, weight, bias)
         ctx.has_bias = bias is not None
         return loss
 
     @staticmethod
     def backward(ctx, head):
-        hidden, weight = ctx.saved_tensors
+        hidden, weight, bias = ctx.saved_tensors
         call, ws, logits = ctx.call, ctx.ws, ctx.logits
         if ws is None:
             raise RuntimeError("proj_ctc_loss: backward needs a forward that ran with gradients enabled (and runs once)")
         head = head.to(torch.float32).contiguous()
-        G = torch.empty_like(logits)
         scratch = torch.empty((call.B,), dtype=torch.float32, device=head.device)
-        call.data = logits
-        call.run(_lib.PHASE_BACKWARD, ws, scratch, grad=G, head=head, handoff="pointer")
+        if ctx.recompute:
+            # the product again, straight into G: head * (softmax - occupancy), the logits never stored
+            G = torch.empty((call.B, call.T, call.V), dtype=torch.float32, device=head.device)
+            p = call.problem(scratch, grad=G, head=head)
+            p.logits = None
+            pj = _proj_struct(hidden, weight, bias)
+            with _on_device(head.device):
+                rc = _lib.load().ctcb_proj_backward(ctypes.byref(pj), ctypes.byref(p), ws.data_ptr(), ws.numel(),
+                                                    _stream_ptr(head.device))
+            _lib.check(rc)
+        else:
+            G = torch.empty_like(logits)
+            call.data = logits
+            call.run(_lib.PHASE_BACKWARD, ws, scratch, grad=G, head=head, handoff="pointer")
         ctx.ws = ctx.logits = None
         G2 = G.view(-1, G.shape[2])
         dh = dw = db = None
@@ -151,10 +170,19 @@ def proj_ctc_loss(hidden, weight, bias, label, pred_lengths=None, label_lengths=
     With a gradient the logits have to exist for the gradient kernel; measured on B200 (scripts/proj_bench.py, cfg3
     shape, H = 512) a 2-SM 256x256 library GEMM writes them faster than the fused epilogue does (forward with logits
     kept: 211 us against 251), so by default the training call is the library product followed by ``CtcLoss``;
-    ``fused_training=True`` forces the fused kernel (``ctcb_proj_forward`` with a logits buffer)."""
+    ``fused_training=True`` forces the fused kernel (``ctcb_proj_forward`` with a logits buffer).
+
+    ``fused_training="recompute"``: the fused forward without a logits buffer (it keeps a table of the label columns'
+    occupancies instead), and a backward that forms the product again on the tensor cores and writes d loss / d logits
+    straight from it (``ctcb_proj_backward``): the logits are never written or read.  Losses bit-identical to
+    ``fused_training=True``; fp32 (tf32 product) or bfloat16 operands.  Measured against the other two arms in
+    scripts/proj_train_bench.py (README)."""
+    if isinstance(fused_training, str) and fused_training != "recompute":
+        raise ValueError("fused_training must be False, True or 'recompute', got %r" % (fused_training,))
     needs_grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (hidden, weight, bias))
+    fused = True if not needs_grad else (fused_training if fused_training == "recompute" else bool(fused_training))
     return _ProjCtcLossFn.apply(hidden, weight, bias, label, pred_lengths, label_lengths, _blank_last(blank_label),
-                                label_layout == "TN", (not needs_grad) or bool(fused_training))
+                                label_layout == "TN", fused)
 
 
 def proj_ctc_eval(hidden, weight, bias, label, pred_lengths=None, label_lengths=None, blank_label="first",
@@ -238,6 +266,7 @@ class ProjCtcLoss(torch.nn.Module):
         self.blank_label, self.label_layout = blank_label, label_layout
 
     def forward(self, hidden, label, pred_lengths=None, label_lengths=None, fused_training=False):
+        """``proj_ctc_loss`` with this block's parameters; ``fused_training``: False, True or "recompute" (see there)."""
         return proj_ctc_loss(hidden, self.weight, self.bias, label, pred_lengths, label_lengths, self.blank_label,
                              self.label_layout, fused_training)
 

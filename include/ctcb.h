@@ -330,7 +330,8 @@ typedef struct ctcb_proj {
  * validation pass, train_ctc_ce.py:143); otherwise the (T,B,V) buffer (p->logits_stride_*) the projection is written to,
  * once, for the gradient kernel.  keep_for_backward as in ctcb_forward: with it (and p->logits) a following
  * ctcb_backward(p, ...) writes d loss / d logits into p->grad, from which d hidden = G . weight, d weight = G^T . hidden
- * and d bias = sum G are plain library GEMMs (gluon_e2e_asr_b200/proj.py).  p->logits_row_offsets is not supported.
+ * and d bias = sum G are plain library GEMMs (gluon_e2e_asr_b200/proj.py).  keep_for_backward with p->logits = NULL: no
+ * logits are stored, the gradient comes from ctcb_proj_backward (below).  p->logits_row_offsets is not supported.
  * CTCB_UNSUPPORTED for V <= 64 or V <= Lmax + 1 (there the logits are a few per cent of the projection's traffic and the
  * walkers' fused producers read them once anyway) and for label rows too long for the kernel's shared memory. */
 int ctcb_proj_forward(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t keep_for_backward, void* workspace,
@@ -360,6 +361,17 @@ int ctcb_proj_greedy_decode(const ctcb_proj_t* proj, int32_t T, int32_t B, int32
 /* ctcb_proj_forward(keep_for_backward=1) followed by ctcb_backward in one call: loss, p->logits and p->grad. */
 int ctcb_proj_loss_grad(const ctcb_proj_t* proj, const ctcb_problem_t* p, void* workspace, size_t workspace_bytes,
                         void* stream);
+/* The training call without the logits: ctcb_proj_forward(keep_for_backward=1) with p->logits = NULL keeps the walkers'
+ * history and turns it into a table of normalised lattice occupancies in the workspace (one more launch, no logits
+ * written); this entry then forms the product again on the tensor cores, tile by tile, and writes
+ * p->grad = head_grad[b] * (softmax(logits) - occupancy) -- d loss / d logits, fp32, (B,T,V) in p->grad_stride_* -- without
+ * the logits ever reaching HBM.  Same proj and problem as the forward (the same workspace, need_grad = 1 size of
+ * ctcb_workspace_bytes); p->logits is ignored, p->head_grad NULL = 1.  Padded frames and infeasible utterances get zero
+ * rows; a workspace that no such forward filled gets NaN rows (no wait, no hang).  Validation as ctcb_proj_loss_grad;
+ * CTCB_UNSUPPORTED where ctcb_proj_forward is (V <= 64, V <= Lmax + 1, label rows too long for shared memory).  Detected
+ * by symbol, like the *_typed entries. */
+int ctcb_proj_backward(const ctcb_proj_t* proj, const ctcb_problem_t* p, void* workspace, size_t workspace_bytes,
+                       void* stream);
 
 #ifdef __cplusplus
 }
