@@ -9,6 +9,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <initializer_list>
 #include <mutex>
 #include <new>
 #include <utility>
@@ -41,23 +42,35 @@ thread_local PendingXchg g_xchg;                      // ctcb_mailbox_exchange_w
 // programmatic dependent of the kernel launched just before it (the step's gradient kernel).
 bool launch_pending_xchg(cudaStream_t stream, bool programmatic = false) {
     if (!g_xchg.mb) return false;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(1); cfg.blockDim = dim3(32); cfg.dynamicSmemBytes = 0; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = programmatic ? 1 : 0;
     const ctcb::MailboxDev* md = g_xchg.mb->dev_d;
-    cudaLaunchKernelEx(&cfg, ctcb::k_mailbox_exchange, md, g_xchg.values, g_xchg.count, g_xchg.out, 0);
+    ctcb::launch_ex(ctcb::k_mailbox_exchange, dim3(1), dim3(32), 0, stream, programmatic, 1, md, g_xchg.values, g_xchg.count,
+                    g_xchg.out, 0);
     g_xchg = PendingXchg{};
     return true;
 }
-thread_local const ctcb_proj_t* g_proj = nullptr;      // ctcb_proj_*: the projection whose epilogue replaces k_emit in this call
-struct DecodeRequest { int32_t* tokens; int32_t* lengths; int unk; };
-thread_local const DecodeRequest* g_decode = nullptr;  // ctcb_proj_forward_decode: the greedy decode the projection's epilogue adds
-thread_local bool g_recompute = false;                 // ctcb_proj_forward(keep_for_backward, no logits): the occupancy table follows
-thread_local cudaEvent_t* g_prof_events = nullptr;   // when set: one event recorded after every launch
-thread_local int g_prof_count = 0;
+
+// phase bits
+enum { PH_FORWARD = 1, PH_BACKWARD = 2 };
+
+// what one ABI call asks of the launch path besides the problem: filled in by the entry, read by enqueue and launch_proj
+struct Request {
+    int phases;
+    bool keep_hist;
+    int ldt;                                // element type of p->logits and p->grad (CTCB_F32 or CTCB_BF16)
+    const ctcb_proj_t* proj = nullptr;      // ctcb_proj_*: the projection whose epilogue replaces k_emit (p->logits may be NULL)
+    int32_t* tokens = nullptr;              // ctcb_proj_forward_decode: the greedy decode the projection's epilogue adds
+    int32_t* lengths = nullptr;
+    int unk = -1;
+    bool recompute = false;                 // ctcb_proj_forward(keep_for_backward, no logits): the occupancy table follows
+    cudaEvent_t* events = nullptr;          // ctcb_loss_grad_timed: one event recorded after every launch (at most 8) ...
+    int n_events = 0;                       // ... and how many were
+    Request(int phases_, bool keep_hist_, int ldt_ = CTCB_F32) : phases(phases_), keep_hist(keep_hist_), ldt(ldt_) {}
+};
+// ctcb_loss_grad*: the backward too when there is a gradient buffer
+Request loss_grad_request(const ctcb_problem_t* p, int ldt) {
+    const bool need_grad = p && p->grad != nullptr;
+    return Request(need_grad ? (PH_FORWARD | PH_BACKWARD) : PH_FORWARD, need_grad, ldt);
+}
 
 // ---- tuning / experiment switches -----------------------------------------------------------
 // Read from the environment ONCE (CTCB_<NAME>, at first use) and changeable through ctcb_set_option (tests, A/B
@@ -164,9 +177,11 @@ bool meet_wanted(int B) {
     return false;
 }
 
+}  // namespace
+
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) only when a launch needs more than any before it
 // (per device and kernel): it is a driver call, and this sits on the per-step host path
-cudaError_t ensure_dynamic_smem(const void* fn, size_t bytes) {
+cudaError_t ctcb::ensure_dynamic_smem(const void* fn, size_t bytes) {
     static std::mutex mu;
     static std::vector<std::pair<std::pair<int, const void*>, size_t>> seen;
     int dev = 0;
@@ -183,6 +198,9 @@ cudaError_t ensure_dynamic_smem(const void* fn, size_t bytes) {
     if (rc == cudaSuccess) seen.push_back({{dev, fn}, bytes});
     return rc;
 }
+
+namespace {
+using ctcb::ensure_dynamic_smem;
 
 struct Layout {
     size_t off_Tb, off_Lb, off_flags, off_lab, off_rank, off_dl, off_nd, off_fr, off_E, off_hA, off_hB, off_oA, off_oB, off_gprog, off_runv, off_pinfo, off_tflag, off_meet, off_meetlz, off_meetcnt, total;
@@ -291,12 +309,13 @@ bool rows16(const void* base, long long st_t, long long st_b, int V, int esz) {
 }
 inline int dtype_size(int logits_dtype) { return logits_dtype == CTCB_BF16 ? 2 : 4; }
 
-int validate(const ctcb_problem_t* p) {
+// logits_optional: the projection entries, whose logits come from the encoder output
+int validate(const ctcb_problem_t* p, bool logits_optional) {
     if (!p) return fail(CTCB_INVALID_VALUE, "problem is NULL");
     if (p->T <= 0 || p->B <= 0 || p->V <= 1 || p->Lmax < 0)
         return fail(CTCB_INVALID_VALUE, "bad shape T=%d B=%d V=%d Lmax=%d", p->T, p->B, p->V, p->Lmax);
     if (p->blank < 0 || p->blank >= p->V) return fail(CTCB_INVALID_VALUE, "blank %d outside [0,%d)", p->blank, p->V);
-    if ((!p->logits && !g_proj) || !p->loss) return fail(CTCB_INVALID_VALUE, "logits and loss must not be NULL");
+    if ((!p->logits && !logits_optional) || !p->loss) return fail(CTCB_INVALID_VALUE, "logits and loss must not be NULL");
     if (p->Lmax > 0 && !p->labels) return fail(CTCB_INVALID_VALUE, "labels is NULL");
     auto dt_ok = [](int d) { return d >= CTCB_I32 && d <= CTCB_F64; };
     if (!dt_ok(p->label_dtype) || (p->data_lengths && !dt_ok(p->data_lengths_dtype)) ||
@@ -338,6 +357,21 @@ void* pinned_device_alias(const void* ptr) {
     return at.type == cudaMemoryTypeHost ? at.devicePointer : nullptr;
 }
 
+// every pointer is CUDA device memory (or NULL)
+bool on_device(std::initializer_list<const void*> ptrs) {
+    for (const void* ptr : ptrs)
+        if (!is_device_ptr(ptr)) return false;
+    return true;
+}
+
+int check_workspace(const void* workspace, size_t workspace_bytes, const Layout& lay) {
+    if (!workspace) return fail(CTCB_INVALID_VALUE, "workspace is NULL");
+    if (workspace_bytes < lay.total)
+        return fail(CTCB_WORKSPACE_TOO_SMALL, "workspace %zu < required %zu bytes", workspace_bytes, lay.total);
+    if (reinterpret_cast<uintptr_t>(workspace) % 256) return fail(CTCB_INVALID_VALUE, "workspace must be 256-byte aligned");
+    return CTCB_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -375,12 +409,9 @@ int ctcb_workspace_bytes(int32_t T, int32_t B, int32_t V, int32_t Lmax, int32_t 
 
 namespace {
 
-// phase bits
-enum { PH_FORWARD = 1, PH_BACKWARD = 2 };
-
-inline void mark(cudaStream_t stream) {
+inline void mark(Request& rq, cudaStream_t stream) {
     ++g_launches;
-    if (g_prof_events && g_prof_count < 8) cudaEventRecord(g_prof_events[g_prof_count++], stream);
+    if (rq.events && rq.n_events < 8) cudaEventRecord(rq.events[rq.n_events++], stream);
 }
 
 // cuTensorMapEncodeTiled through the runtime's driver entry point: libcuda is not linked
@@ -398,8 +429,19 @@ EncodeTiledFn encode_tiled() {
     return fn;
 }
 
-// the projection's operands (hidden, weight, bias): element type, 16-byte strides and bases, device memory
-int check_proj_operands(const ctcb_proj_t* pj) {
+// the problems the projection kernel's lattice epilogue takes: a gathered (V > 64, V > Lmax + 1) emission table, unpacked rows
+int check_proj_problem(const ctcb_problem_t* p, const Layout& lay) {
+    if (lay.fused || lay.dense)
+        return fail(CTCB_UNSUPPORTED, "projection fused with the loss needs V > 64 and V > Lmax + 1 (V=%d, Lmax=%d)", p->V, p->Lmax);
+    if (p->logits_row_offsets) return fail(CTCB_UNSUPPORTED, "projection: packed logits are not supported");
+    return CTCB_OK;
+}
+
+// the projection's operands (hidden, weight, bias): present, element type, 16-byte strides and bases, device memory.
+// lay != nullptr (the forward entries): the problem's shape is refused between the NULL and the format checks
+int check_proj_operands(const ctcb_proj_t* pj, const ctcb_problem_t* p, const Layout* lay) {
+    if (!pj->hidden || !pj->weight || pj->K <= 0) return fail(CTCB_INVALID_VALUE, "projection: hidden / weight is NULL or K <= 0");
+    if (lay) { if (int rc = check_proj_problem(p, *lay)) return rc; }
     if (pj->operand_dtype != CTCB_PROJ_F32 && pj->operand_dtype != CTCB_PROJ_BF16)
         return fail(CTCB_INVALID_VALUE, "projection: operand_dtype %d is neither CTCB_PROJ_F32 nor CTCB_PROJ_BF16", pj->operand_dtype);
     const int per16 = pj->operand_dtype == CTCB_PROJ_BF16 ? 8 : 4;
@@ -411,105 +453,123 @@ int check_proj_operands(const ctcb_proj_t* pj) {
     return CTCB_OK;
 }
 
-// the TMA maps of the projection's operands: hidden (K, T, B) in boxes of one 128-byte K block x kPM frames, weight (K, V) in
-// boxes of one K block x the CTA's share of a vocabulary tile
-int encode_proj_maps(const ctcb_proj_t* pj, int T, int B, int V, int ctas, CUtensorMap* tmA, CUtensorMap* tmB) {
+// CTA pairs (tcgen05 cta_group::2: 256 frames per pair, each CTA stages half of the vocabulary tile) or single CTAs
+// (measured: pairs 186 us, single CTAs 190 us per fused forward at cfg3, H = 512)
+inline int proj_ctas() { return opt(OPT_PROJ_CTAS) == 1 ? 1 : 2; }
+
+// one launch of the projection kernel, prepared: the operands' tensor maps, the output's (tmA while there is none), the
+// launch fields of the projection and the problem (the caller adds the workspace and the outputs), grid and shared memory
+struct ProjLaunch {
+    CUtensorMap tmA, tmB, tmC;
+    ctcb::ProjArgs pa;
+    dim3 grid;
+    size_t smem;
+};
+
+// every projection entry, after its checks: the kernel's shared memory (refused beyond the opt-in maximum when it holds
+// label columns; lay: the layout of a problem with labels, or nullptr), the TMA maps of the operands -- hidden (K, T, B) in
+// boxes of one 128-byte K block x kPM frames, weight (K, V) in boxes of one K block x the CTA's share of a vocabulary tile --,
+// the launch fields and the grid.  mode: what the epilogue computes (k_proj_emit)
+int prepare_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const Layout* lay, int mode, ProjLaunch* pl) {
+    const int ctas = proj_ctas();
+    const int NT = (p->V + ctcb::kPN - 1) / ctcb::kPN;
+    const bool store = mode == ctcb::kProjGrad || p->logits != nullptr;
+    const bool decode = mode == ctcb::kProjLossDecode || mode == ctcb::kProjDecode;
+    pl->smem = ctcb::proj_smem_bytes(p->Lmax, lay ? lay->Lp : 0, store, NT, ctas, decode);
+    if (lay && pl->smem > 232448 - 64)
+        return fail(CTCB_UNSUPPORTED, "projection: Lmax=%d label columns do not fit the kernel's shared memory", p->Lmax);
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return fail(CTCB_UNSUPPORTED, "cuTensorMapEncodeTiled is not available from this driver");
     const bool bf = pj->operand_dtype == CTCB_PROJ_BF16;
     const int esz = bf ? 2 : 4;
     {
-        const cuuint64_t gdim[3] = {(cuuint64_t)pj->K, (cuuint64_t)T, (cuuint64_t)B};
+        const cuuint64_t gdim[3] = {(cuuint64_t)pj->K, (cuuint64_t)p->T, (cuuint64_t)p->B};
         const cuuint64_t gstr[2] = {(cuuint64_t)pj->hidden_stride_t * esz, (cuuint64_t)pj->hidden_stride_b * esz};
         const cuuint32_t box[3] = {(cuuint32_t)(128 / esz), (cuuint32_t)ctcb::kPM, 1};
         const cuuint32_t est[3] = {1, 1, 1};
-        const CUresult r = enc(tmA, bf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(pj->hidden), gdim, gstr, box, est,
+        const CUresult r = enc(&pl->tmA, bf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(pj->hidden), gdim, gstr, box, est,
                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return fail(CTCB_INVALID_VALUE, "cuTensorMapEncodeTiled(hidden) failed: %d", (int)r);
     }
     {
-        const cuuint64_t gdim[2] = {(cuuint64_t)pj->K, (cuuint64_t)V};
+        const cuuint64_t gdim[2] = {(cuuint64_t)pj->K, (cuuint64_t)p->V};
         const cuuint64_t gstr[1] = {(cuuint64_t)pj->K * esz};
         const cuuint32_t box[2] = {(cuuint32_t)(128 / esz), (cuuint32_t)(ctcb::kPN / ctas)};
         const cuuint32_t est[2] = {1, 1};
-        const CUresult r = enc(tmB, bf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(pj->weight), gdim, gstr, box, est,
+        const CUresult r = enc(&pl->tmB, bf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(pj->weight), gdim, gstr, box, est,
                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return fail(CTCB_INVALID_VALUE, "cuTensorMapEncodeTiled(weight) failed: %d", (int)r);
     }
+    pl->tmC = pl->tmA;
+    ctcb::ProjArgs& pa = pl->pa;
+    pa = ctcb::ProjArgs{};
+    pa.p = to_device_problem(p);
+    pa.bias = pj->bias;
+    pa.K = pj->K; pa.NT = NT; pa.KB = (pj->K + 128 / esz - 1) / (128 / esz);
+    pa.bf16 = bf ? 1 : 0;
+    pa.ctas = ctas;
+    pa.dbg = opt(OPT_PROJ_DBG) > 0 ? opt(OPT_PROJ_DBG) : 0;
+    pa.vec4 = (p->V % 4 == 0 && reinterpret_cast<uintptr_t>(pj->bias) % 16 == 0) ? 1 : 0;
+    pa.unk = -1;
+    const int mtiles = (p->T + ctcb::kPM - 1) / ctcb::kPM;
+    pl->grid = dim3(ctas, p->B, (mtiles + ctas - 1) / ctas);
     return CTCB_OK;
 }
 
-// the launch fields that depend on the projection alone (the caller adds the problem, workspace and outputs)
-ctcb::ProjArgs proj_args(const ctcb_proj_t* pj, int V, int ctas) {
-    const int esz = pj->operand_dtype == CTCB_PROJ_BF16 ? 2 : 4;
-    ctcb::ProjArgs pa{};
-    pa.bias = pj->bias;
-    pa.K = pj->K; pa.NT = (V + ctcb::kPN - 1) / ctcb::kPN; pa.KB = (pj->K + 128 / esz - 1) / (128 / esz);
-    pa.bf16 = esz == 2 ? 1 : 0;
-    pa.ctas = ctas;
-    pa.dbg = opt(OPT_PROJ_DBG) > 0 ? opt(OPT_PROJ_DBG) : 0;
-    pa.vec4 = (V % 4 == 0 && reinterpret_cast<uintptr_t>(pj->bias) % 16 == 0) ? 1 : 0;
-    pa.unk = -1;
-    return pa;
+// the projection kernel's fp32 output (the logits, or G) leaves through TMA tile stores (ProjArgs::store 1, through *tm)
+// when its rows allow a tensor map, else through direct stores (2).  A (T,B,V) buffer has the batch stride below the frame
+// stride: the map's dimensions stay (V, T, B), the strides say the rest
+int encode_out_map(const float* out, long long st_t, long long st_b, int T, int B, int V, CUtensorMap* tm) {
+    if (st_t % 4 != 0 || st_b % 4 != 0 || reinterpret_cast<uintptr_t>(out) % 16 != 0) return 2;
+    const cuuint64_t gdim[3] = {(cuuint64_t)V, (cuuint64_t)T, (cuuint64_t)B};
+    const cuuint64_t gstr[2] = {(cuuint64_t)st_t * 4, (cuuint64_t)st_b * 4};
+    const cuuint32_t box[3] = {32, 32, 1};
+    const cuuint32_t est[3] = {1, 1, 1};
+    const CUresult r = encode_tiled()(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(out), gdim, gstr, box, est,
+                                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    return r == CUDA_SUCCESS ? 1 : 2;
 }
 
-// CTA pairs (tcgen05 cta_group::2: 256 frames per pair, each CTA stages half of the vocabulary tile) or single CTAs
-// (measured: pairs 186 us, single CTAs 190 us per fused forward at cfg3, H = 512)
-inline int proj_ctas() { return opt(OPT_PROJ_CTAS) == 1 ? 1 : 2; }
+// k_greedy_collapse keeps two words per frame in shared memory
+int check_collapse_rows(int T) {
+    if (2 * sizeof(int) * (size_t)T > 200 * 1024) return fail(CTCB_UNSUPPORTED, "T=%d too long for the decode kernel", T);
+    return CTCB_OK;
+}
+
+// the hypotheses from the projection's per-frame words.  tflag: the projection's tile flags, acquired per tile (nullptr: the
+// projection kernel is complete in stream order)
+int launch_greedy_collapse(const int* tflag, int ntile, const void* data_lengths, int data_lengths_dtype, int T, int B, int blank,
+                           int unk, int32_t* tokens, int32_t* lengths, cudaStream_t stream) {
+    const size_t dsm = 2 * sizeof(int) * (size_t)T;
+    if (dsm > 48 * 1024) CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(ctcb::k_greedy_collapse), dsm));
+    ctcb::k_greedy_collapse<<<B, 256, dsm, stream>>>(tflag, ntile, data_lengths, data_lengths_dtype, T, blank, unk, tokens, lengths);
+    return CTCB_OK;
+}
 
 // the projection kernel (ctcb_proj.cuh) in k_emit's place: {row max, normaliser} and the emission table from the
 // encoder output, then the metadata CTAs of k_emit (one per utterance)
 // beside: the recursion kernel will be launched as the projection's programmatic dependent and follow its tiles (loss
 // evaluation only): the metadata kernel then goes FIRST (the walkers poll its "ready" word) and the projection starts beside it
-int launch_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const ctcb::Problem& dp, const ctcb::Workspace& w,
-                const Layout& lay, cudaStream_t stream, bool beside) {
-    if (!pj->hidden || !pj->weight || pj->K <= 0) return fail(CTCB_INVALID_VALUE, "projection: hidden / weight is NULL or K <= 0");
-    if (lay.fused || lay.dense)
-        return fail(CTCB_UNSUPPORTED, "projection fused with the loss needs V > 64 and V > Lmax + 1 (V=%d, Lmax=%d)", p->V, p->Lmax);
-    if (p->logits_row_offsets) return fail(CTCB_UNSUPPORTED, "projection: packed logits are not supported");
-    if (int rc = check_proj_operands(pj)) return rc;
-    const int ctas = proj_ctas();
-    const size_t smem = ctcb::proj_smem_bytes(p->Lmax, lay.Lp, p->logits != nullptr, (p->V + ctcb::kPN - 1) / ctcb::kPN, ctas, g_decode != nullptr);
-    if (smem > 232448 - 64) return fail(CTCB_UNSUPPORTED, "projection: Lmax=%d label columns do not fit the kernel's shared memory", p->Lmax);
-    CUtensorMap tmA, tmB;
-    if (int rc = encode_proj_maps(pj, p->T, p->B, p->V, ctas, &tmA, &tmB)) return rc;
-    ctcb::ProjArgs pa = proj_args(pj, p->V, ctas);
-    pa.p = dp; pa.w = w; pa.logits = const_cast<float*>(p->logits);
-    pa.tok = g_decode ? g_decode->tokens : nullptr;
-    pa.unk = g_decode ? g_decode->unk : -1;
-    // the logits (kept for the gradient kernel) leave through TMA stores when their rows allow a tensor map
-    CUtensorMap tmC = tmA;
-    pa.store = 0;
+int launch_proj(Request& rq, const ctcb_problem_t* p, const ctcb::Workspace& w, const Layout& lay, cudaStream_t stream, bool beside) {
+    if (int rc = check_proj_operands(rq.proj, p, &lay)) return rc;
+    const int mode = rq.tokens ? ctcb::kProjLossDecode : ctcb::kProjLoss;
+    ProjLaunch pl;
+    if (int rc = prepare_proj(rq.proj, p, &lay, mode, &pl)) return rc;
+    ctcb::ProjArgs& pa = pl.pa;
+    pa.w = w; pa.logits = const_cast<float*>(p->logits);
+    pa.tok = rq.tokens;
+    pa.unk = rq.unk;
+    // the logits (kept for the gradient kernel)
+    pa.store = p->logits ? encode_out_map(p->logits, p->logits_stride_t, p->logits_stride_b, p->T, p->B, p->V, &pl.tmC) : 0;
     pa.smem_stash = ctcb::proj_smem_stash(p->Lmax, p->logits != nullptr) ? 1 : 0;
-    if (p->logits) {
-        pa.store = 2;
-        if (p->logits_stride_t % 4 == 0 && p->logits_stride_b % 4 == 0 && reinterpret_cast<uintptr_t>(p->logits) % 16 == 0) {
-            const cuuint64_t gdim[3] = {(cuuint64_t)p->V, (cuuint64_t)p->T, (cuuint64_t)p->B};
-            const cuuint64_t gstr[2] = {(cuuint64_t)p->logits_stride_t * 4, (cuuint64_t)p->logits_stride_b * 4};
-            const cuuint32_t box[3] = {32, 32, 1};
-            const cuuint32_t est[3] = {1, 1, 1};
-            // a (T,B,V) buffer has the batch stride below the frame stride: the map's dimensions stay (V, T, B), strides say the rest
-            const CUresult r = encode_tiled()(&tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(p->logits), gdim, gstr, box, est,
-                                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r == CUDA_SUCCESS) pa.store = 1;
-        }
-    }
-    const int mtiles = (p->T + ctcb::kPM - 1) / ctcb::kPM;
-    const dim3 pgrid(ctas, p->B, (mtiles + ctas - 1) / ctas);
-    const int mode = g_decode ? ctcb::kProjLossDecode : ctcb::kProjLoss;
     auto launch_meta = [&](bool programmatic) -> int {
         // per-utterance metadata: k_emit's extra CTA alone (grid.x = 1: every CTA is the metadata CTA)
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3(1, p->B); cfg.blockDim = dim3(128); cfg.dynamicSmemBytes = ctcb::emit_smem_bytes(lay.Lp, 0); cfg.stream = stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr; cfg.numAttrs = programmatic ? 1 : 0;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, ctcb::k_emit<1, 0>, dp, w));
-        mark(stream);
+        CUDA_TRY(ctcb::launch_ex(ctcb::k_emit<1, 0>, dim3(1, p->B), dim3(128), ctcb::emit_smem_bytes(lay.Lp, 0), stream, programmatic, 1,
+                                 pa.p, w));
+        mark(rq, stream);
         return CTCB_OK;
     };
     if (beside) {
@@ -517,39 +577,34 @@ int launch_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const ctcb::Prob
         CUDA_TRY(cudaMemsetAsync(w.tflag, 0, sizeof(int) * (size_t)p->B * w.ntile, stream));
         CUDA_TRY(cudaMemsetAsync(w.gprog, 0, sizeof(int) * 4 * (size_t)p->B, stream));
         if (int rc = launch_meta(false)) return rc;
-        CUDA_TRY(ctcb::launch_proj_emit(tmA, tmB, tmC, pa, mode, pgrid, smem, stream, true));    // programmatic: beside the metadata kernel
-        mark(stream);
+        CUDA_TRY(ctcb::launch_proj_emit(pl.tmA, pl.tmB, pl.tmC, pa, mode, pl.grid, pl.smem, stream, true));    // programmatic: beside the metadata kernel
+        mark(rq, stream);
         return CTCB_OK;
     }
     // decoding: k_greedy_collapse acquires the tile flags, which a previous call on this workspace may have left set
-    if (g_decode) CUDA_TRY(cudaMemsetAsync(w.tflag, 0, sizeof(int) * (size_t)p->B * w.ntile, stream));
-    CUDA_TRY(ctcb::launch_proj_emit(tmA, tmB, tmC, pa, mode, pgrid, smem, stream, false));
-    mark(stream);
+    if (rq.tokens) CUDA_TRY(cudaMemsetAsync(w.tflag, 0, sizeof(int) * (size_t)p->B * w.ntile, stream));
+    CUDA_TRY(ctcb::launch_proj_emit(pl.tmA, pl.tmB, pl.tmC, pa, mode, pl.grid, pl.smem, stream, false));
+    mark(rq, stream);
     // the metadata kernel as the projection kernel's programmatic dependent -- it starts at once and runs beside it (it
     // reads nothing the projection writes); the recursion kernel that follows is an ordinary launch and waits for both
-    if (int rc = launch_meta(!g_prof_events)) return rc;
+    if (int rc = launch_meta(!rq.events)) return rc;
     return CTCB_OK;
 }
 
-// ldt: element type of p->logits and p->grad (CTCB_F32 or CTCB_BF16)
-int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream_, int phases, bool keep_hist,
-            int ldt = CTCB_F32) {
+int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream_, Request& rq) {
     g_grad_kernel = 0;
-    if (int rc = validate(p)) return rc;
+    if (int rc = validate(p, rq.proj != nullptr)) return rc;
+    const int ldt = rq.ldt, phases = rq.phases;
     if (ldt != CTCB_F32 && ldt != CTCB_BF16)
         return fail(CTCB_INVALID_VALUE, "logits dtype %d is neither CTCB_F32 nor CTCB_BF16 (fp16 logits are not supported)", ldt);
-    if (ldt != CTCB_F32 && g_proj) return fail(CTCB_INVALID_VALUE, "the fused projection writes fp32 logits");
+    if (ldt != CTCB_F32 && rq.proj) return fail(CTCB_INVALID_VALUE, "the fused projection writes fp32 logits");
     const bool bf = ldt == CTCB_BF16;
     const int esz = dtype_size(ldt);
-    const bool need_grad = keep_hist || (phases & PH_BACKWARD);
+    const bool need_grad = rq.keep_hist || (phases & PH_BACKWARD);
     if ((phases & PH_BACKWARD) && !p->grad) return fail(CTCB_INVALID_VALUE, "grad is NULL");
     const Layout lay = make_layout(p->T, p->B, p->V, p->Lmax, need_grad);
-    if (!workspace) return fail(CTCB_INVALID_VALUE, "workspace is NULL");
-    if (workspace_bytes < lay.total)
-        return fail(CTCB_WORKSPACE_TOO_SMALL, "workspace %zu < required %zu bytes", workspace_bytes, lay.total);
-    if (reinterpret_cast<uintptr_t>(workspace) % 256) return fail(CTCB_INVALID_VALUE, "workspace must be 256-byte aligned");
-    if (!is_device_ptr(p->logits) || !(is_device_ptr(p->loss) || pinned_device_alias(p->loss)) || !is_device_ptr(workspace) || !is_device_ptr(p->grad) ||
-        !is_device_ptr(p->labels) || !is_device_ptr(p->logits_row_offsets))
+    if (int rc = check_workspace(workspace, workspace_bytes, lay)) return rc;
+    if (!on_device({p->logits, p->grad, p->labels, p->logits_row_offsets, workspace}) || !(is_device_ptr(p->loss) || pinned_device_alias(p->loss)))
         return fail(CTCB_INVALID_VALUE, "logits/labels/loss/grad/workspace must be CUDA device memory (there is no CPU path)");
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     const ctcb::Problem dp = to_device_problem(p);
@@ -569,8 +624,8 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
             CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(mfn), msm));
             g_walk_p = mp; g_walk_nw = 1; g_grad_kernel = 3;
             mfn<<<p->B, 256, msm, stream>>>(ma);
-            mark(stream);
-            if (launch_pending_xchg(stream)) mark(stream);
+            mark(rq, stream);
+            if (launch_pending_xchg(stream)) mark(rq, stream);
             CUDA_TRY(cudaGetLastError());
             return CTCB_OK;
         }
@@ -641,17 +696,17 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
 #undef EMIT_NQ
 #undef EMIT_LAUNCH
             }
-            mark(stream);
+            mark(rq, stream);
             return CTCB_OK;
         };
         // ctcb_mailbox_exchange_with_next on a forward-only call: the exchange kernel goes first and the recursion
         // kernel is its programmatic dependent -- it starts while the exchange's one warp talks to the peers.
         // (With a gradient kernel in the call the exchange goes behind that one instead, see below.)
         const bool xchg = !(phases & PH_BACKWARD) && launch_pending_xchg(stream);
-        if (xchg) mark(stream);
+        if (xchg) mark(rq, stream);
         // loss evaluation from the encoder output: the recursion kernel is the projection's programmatic dependent and
         // follows its 128-frame tiles (the utterances' first tiles are scheduled first) instead of waiting for the kernel
-        const bool beside = g_proj && !need_grad && !xchg && !g_prof_events && opt(OPT_PROJ_OVERLAP) != 0;
+        const bool beside = rq.proj && !need_grad && !xchg && !rq.events && opt(OPT_PROJ_OVERLAP) != 0;
         // loss evaluation (no history): the alpha and the beta walker take half of the frames each and meet in the middle --
         // while every walker CTA of the batch can be resident at once (beyond that one walker per utterance does less work:
         // cfg5, B = 1024: 136 us against 153).  Beside the projection kernel one walker per utterance is the better schedule
@@ -671,34 +726,27 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
             wa.hw_wait = opt(OPT_WALK_HW_WAIT) >= 0 ? opt(OPT_WALK_HW_WAIT) : (2 * p->B > 148 ? 1 : 0);
             // the per-group progress is for gradient CTAs that run concurrently with the walkers; a gradient kernel that
             // runs afterwards polls the same words once, so the final count is enough
-            wa.publish = ((phases & PH_BACKWARD) && !g_prof_events && overlap_allowed(p->B, lay.fused != 0)) ? 1 : 2;
+            wa.publish = ((phases & PH_BACKWARD) && !rq.events && overlap_allowed(p->B, lay.fused != 0)) ? 1 : 2;
             const int wthreads = (we->NW + (lay.fused ? ctcb::kFusedProducers + 1 : 1)) * 32;
-            cudaLaunchConfig_t cfg{};
-            cfg.gridDim = dim3(p->B, (need_grad || meet_fwd) ? 2 : 1); cfg.blockDim = dim3(wthreads); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-            attr[0].val.programmaticStreamSerializationAllowed = 1;
-            cfg.attrs = attr; cfg.numAttrs = (after_xchg || pdl) ? 1 : 0;
-            CUDA_TRY(cudaLaunchKernelEx(&cfg, wfn, wa));
-            mark(stream);
+            CUDA_TRY(ctcb::launch_ex(wfn, dim3(p->B, (need_grad || meet_fwd) ? 2 : 1), dim3(wthreads), smem, stream, after_xchg || pdl, 1, wa));
+            mark(rq, stream);
             return CTCB_OK;
         };
-        if (g_proj) {
-            if (int rc = launch_proj(g_proj, p, dp, w, lay, stream, beside)) return rc;
+        if (rq.proj) {
+            if (int rc = launch_proj(rq, p, w, lay, stream, beside)) return rc;
         } else if (!lay.fused) { if (int rc = launch_emit()) return rc; }
         if (int rc = launch_walk((xchg && lay.fused != 0) || beside, beside)) return rc;
-        if (g_recompute) {
+        if (rq.recompute) {
             // the recomputing training forward: the history becomes the occupancy table O that ctcb_proj_backward reads
             CUDA_TRY(ctcb::launch_proj_occ(dp, w, stream));
-            mark(stream);
+            mark(rq, stream);
         }
-        if (g_decode) {
-            // the hypotheses from the projection's per-frame words (an ordinary launch: it acquires the tile flags itself)
-            const size_t dsm = 2 * sizeof(int) * (size_t)p->T;
-            if (dsm > 48 * 1024) CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(ctcb::k_greedy_collapse), dsm));
-            ctcb::k_greedy_collapse<<<p->B, 256, dsm, stream>>>(w.tflag, w.ntile, p->data_lengths, p->data_lengths_dtype, p->T, p->blank,
-                                                                g_decode->unk, g_decode->tokens, g_decode->lengths);
-            mark(stream);
+        if (rq.tokens) {
+            // an ordinary launch: it acquires the tile flags itself
+            if (int rc = launch_greedy_collapse(w.tflag, w.ntile, p->data_lengths, p->data_lengths_dtype, p->T, p->B, p->blank, rq.unk,
+                                                rq.tokens, rq.lengths, stream))
+                return rc;
+            mark(rq, stream);
         }
     }
     if (phases & PH_BACKWARD) {
@@ -714,7 +762,6 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
         const int ch = gch;
         const int units = (p->V / vec + 31) / 32;
         const int xq = units <= 1 ? 1 : units <= 2 ? 2 : units <= 4 ? 4 : 0;
-        const dim3 ggrid(p->B, lay.NB);                  // one frame block per CTA, utterance-fastest
         using GradFn = void (*)(ctcb::GradArgs);
         GradFn gfn = nullptr;
 #define GRAD_X(V_, C_, T_) (xq == 1 ? ctcb::k_grad<V_, C_, 1, 0, T_> : xq == 2 ? ctcb::k_grad<V_, C_, 2, 0, T_> : \
@@ -726,7 +773,7 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
 #undef GRAD_CH
 #undef GRAD_X
         // batches that run after the walkers (no overlap): the high-occupancy variant of the register-resident kernels
-        if (ch >= 1 && ch <= 4 && !((phases & PH_FORWARD) && !g_prof_events && overlap_allowed(p->B, lay.fused != 0))) {
+        if (ch >= 1 && ch <= 4 && !((phases & PH_FORWARD) && !rq.events && overlap_allowed(p->B, lay.fused != 0))) {
 #define GRADO_X(V_, C_, T_) (xq == 1 ? ctcb::k_grad<V_, C_, 1, 1, T_> : xq == 2 ? ctcb::k_grad<V_, C_, 2, 1, T_> : \
                              xq == 4 ? ctcb::k_grad<V_, C_, 4, 1, T_> : ctcb::k_grad<V_, C_, 0, 1, T_>)
 #define GRADO_CH(V_, T_) (ch == 1 ? GRADO_X(V_, 1, T_) : ch == 2 ? GRADO_X(V_, 2, T_) : GRADO_X(V_, 4, T_))
@@ -743,7 +790,7 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
         if (lay.fused && p->V <= 64 && ch >= 1 && want_grad2) {
             // two register budgets (profiles/r3e_*, r3f_*): 80 registers / 6 CTAs per SM while the walkers run beside the
             // kernel, 72 registers / 7 CTAs per SM for batches whose gradient kernel runs after the walkers
-            bool occ = (phases & PH_FORWARD) && !g_prof_events && overlap_allowed(p->B, true);
+            bool occ = (phases & PH_FORWARD) && !rq.events && overlap_allowed(p->B, true);
             if (opt(OPT_GRAD2_OCC) >= 0) occ = opt(OPT_GRAD2_OCC) != 0;
 #define GRAD2_O(V_, C_, T_) (occ ? ctcb::k_grad2<V_, C_, 1, T_> : ctcb::k_grad2<V_, C_, 0, T_>)
 #define GRAD2_CH(V_, T_) (ch == 1 ? GRAD2_O(V_, 1, T_) : ch == 2 ? GRAD2_O(V_, 2, T_) : ch == 4 ? GRAD2_O(V_, 4, T_) : \
@@ -773,23 +820,18 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
         // start while the walkers run and wait per frame block on Workspace::gprog.  Not when
         // per-kernel events sit between the launches (ctcb_loss_grad_timed) or for batches whose
         // walkers do not fit the GPU at once (the waiting CTAs would hold slots the walkers need).
-        const bool overlap = (phases & PH_FORWARD) && !g_prof_events && overlap_allowed(p->B, lay.fused != 0);
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = ggrid; cfg.blockDim = dim3(gthreads); cfg.dynamicSmemBytes = gsm; cfg.stream = stream;
+        const bool overlap = (phases & PH_FORWARD) && !rq.events && overlap_allowed(p->B, lay.fused != 0);
+        dim3 ggrid(p->B, lay.NB);                  // one frame block per CTA, utterance-fastest
         if (grad2) {
             // k_grad2: a CTA takes several consecutive frame blocks (metadata and P(l|x) once per CTA)
             const int gb = opt(OPT_GRAD2_BLOCKS) > 0 ? opt(OPT_GRAD2_BLOCKS) : 4;      // one whole frame block per warp
-            cfg.gridDim = dim3(p->B, (lay.NB + gb - 1) / gb);
+            ggrid = dim3(p->B, (lay.NB + gb - 1) / gb);
         }
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr; cfg.numAttrs = overlap ? 1 : 0;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, gfn, ga));
+        CUDA_TRY(ctcb::launch_ex(gfn, ggrid, dim3(gthreads), gsm, stream, overlap, 1, ga));
         g_grad_kernel = grad2 ? 2 : 1;
-        mark(stream);
+        mark(rq, stream);
         // ctcb_mailbox_exchange_with_next: behind the gradient kernel, as its programmatic dependent
-        if (launch_pending_xchg(stream, true)) mark(stream);
+        if (launch_pending_xchg(stream, true)) mark(rq, stream);
     }
     CUDA_TRY(cudaGetLastError());
     return CTCB_OK;
@@ -803,8 +845,8 @@ int ctcb_loss_grad(const ctcb_problem_t* p, void* workspace, size_t workspace_by
 
 int ctcb_loss_grad_typed(const ctcb_problem_t* p, int32_t logits_dtype, void* workspace, size_t workspace_bytes, void* stream) {
     g_launches = 0;
-    const bool need_grad = p && p->grad != nullptr;
-    return enqueue(p, workspace, workspace_bytes, stream, need_grad ? (PH_FORWARD | PH_BACKWARD) : PH_FORWARD, need_grad, logits_dtype);
+    Request rq = loss_grad_request(p, logits_dtype);
+    return enqueue(p, workspace, workspace_bytes, stream, rq);
 }
 
 int ctcb_loss_grad_timed(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream_,
@@ -814,14 +856,14 @@ int ctcb_loss_grad_timed(const ctcb_problem_t* p, void* workspace, size_t worksp
     cudaEvent_t ev[9];
     for (auto& e : ev) CUDA_TRY(cudaEventCreate(&e));
     CUDA_TRY(cudaEventRecord(ev[0], stream));
-    g_prof_events = ev + 1; g_prof_count = 0;
-    const int rc = ctcb_loss_grad(p, workspace, workspace_bytes, stream);
-    const int n = g_prof_count;
-    g_prof_events = nullptr; g_prof_count = 0;
+    g_launches = 0;
+    Request rq = loss_grad_request(p, CTCB_F32);
+    rq.events = ev + 1;
+    const int rc = enqueue(p, workspace, workspace_bytes, stream, rq);
     if (rc == CTCB_OK) {
         CUDA_TRY(cudaStreamSynchronize(stream));
-        for (int i = 0; i < n; ++i) CUDA_TRY(cudaEventElapsedTime(&kernel_ms[i], ev[i], ev[i + 1]));
-        *n_kernels = n;
+        for (int i = 0; i < rq.n_events; ++i) CUDA_TRY(cudaEventElapsedTime(&kernel_ms[i], ev[i], ev[i + 1]));
+        *n_kernels = rq.n_events;
     }
     for (auto& e : ev) cudaEventDestroy(e);
     return rc;
@@ -834,7 +876,8 @@ int ctcb_forward(const ctcb_problem_t* p, int32_t keep_for_backward, void* works
 int ctcb_forward_typed(const ctcb_problem_t* p, int32_t logits_dtype, int32_t keep_for_backward, void* workspace,
                        size_t workspace_bytes, void* stream) {
     g_launches = 0;
-    return enqueue(p, workspace, workspace_bytes, stream, PH_FORWARD, keep_for_backward != 0, logits_dtype);
+    Request rq(PH_FORWARD, keep_for_backward != 0, logits_dtype);
+    return enqueue(p, workspace, workspace_bytes, stream, rq);
 }
 
 int ctcb_backward(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream) {
@@ -843,34 +886,40 @@ int ctcb_backward(const ctcb_problem_t* p, void* workspace, size_t workspace_byt
 
 int ctcb_backward_typed(const ctcb_problem_t* p, int32_t logits_dtype, void* workspace, size_t workspace_bytes, void* stream) {
     g_launches = 0;
-    return enqueue(p, workspace, workspace_bytes, stream, PH_BACKWARD, true, logits_dtype);
+    Request rq(PH_BACKWARD, true, logits_dtype);
+    return enqueue(p, workspace, workspace_bytes, stream, rq);
 }
+
+namespace {
+// ctcb_proj_forward and ctcb_proj_forward_decode (rq: the decode's outputs, or none)
+int proj_forward(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t keep_for_backward, void* workspace,
+                 size_t workspace_bytes, void* stream, Request& rq) {
+    if (!proj) return fail(CTCB_INVALID_VALUE, "proj is NULL");
+    g_launches = 0;
+    rq.keep_hist = keep_for_backward != 0;
+    rq.proj = proj;
+    // keep_for_backward without a logits buffer: the history is kept and turned into the occupancy table, the logits are
+    // never stored, and ctcb_proj_backward forms the product again
+    rq.recompute = keep_for_backward && p && !p->logits;
+    return enqueue(p, workspace, workspace_bytes, stream, rq);
+}
+}  // namespace
 
 int ctcb_proj_forward(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t keep_for_backward, void* workspace,
                       size_t workspace_bytes, void* stream) {
-    if (!proj) return fail(CTCB_INVALID_VALUE, "proj is NULL");
-    g_launches = 0;
-    g_proj = proj;
-    // keep_for_backward without a logits buffer: the history is kept and turned into the occupancy table, the logits are
-    // never stored, and ctcb_proj_backward forms the product again
-    g_recompute = keep_for_backward && p && !p->logits;
-    const int rc = enqueue(p, workspace, workspace_bytes, stream, PH_FORWARD, keep_for_backward != 0);
-    g_proj = nullptr;
-    g_recompute = false;
-    return rc;
+    Request rq(PH_FORWARD, false);
+    return proj_forward(proj, p, keep_for_backward, workspace, workspace_bytes, stream, rq);
 }
 
 int ctcb_proj_forward_decode(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t keep_for_backward, int32_t unk,
                              int32_t* out_tokens, int32_t* out_lengths, void* workspace, size_t workspace_bytes, void* stream) {
     if (!out_tokens || !out_lengths) return fail(CTCB_INVALID_VALUE, "NULL argument");
     if (p && unk >= p->V) return fail(CTCB_INVALID_VALUE, "unk %d outside the vocabulary (V=%d; -1 = no <unk> rule)", unk, p->V);
-    if (p && p->T > 0 && 2 * sizeof(int) * (size_t)p->T > 200 * 1024) return fail(CTCB_UNSUPPORTED, "T=%d too long for the decode kernel", p->T);
-    if (!is_device_ptr(out_tokens) || !is_device_ptr(out_lengths)) return fail(CTCB_INVALID_VALUE, "buffers must be CUDA device memory");
-    const DecodeRequest req{out_tokens, out_lengths, unk < 0 ? -1 : unk};
-    g_decode = &req;
-    const int rc = ctcb_proj_forward(proj, p, keep_for_backward, workspace, workspace_bytes, stream);
-    g_decode = nullptr;
-    return rc;
+    if (p && p->T > 0) { if (int rc = check_collapse_rows(p->T)) return rc; }
+    if (!on_device({out_tokens, out_lengths})) return fail(CTCB_INVALID_VALUE, "buffers must be CUDA device memory");
+    Request rq(PH_FORWARD, false);
+    rq.tokens = out_tokens; rq.lengths = out_lengths; rq.unk = unk < 0 ? -1 : unk;
+    return proj_forward(proj, p, keep_for_backward, workspace, workspace_bytes, stream, rq);
 }
 
 int ctcb_proj_greedy_decode(const ctcb_proj_t* proj, int32_t T, int32_t B, int32_t V, const void* data_lengths,
@@ -882,32 +931,25 @@ int ctcb_proj_greedy_decode(const ctcb_proj_t* proj, int32_t T, int32_t B, int32
     if (unk >= V) return fail(CTCB_INVALID_VALUE, "unk %d outside the vocabulary (V=%d; -1 = no <unk> rule)", unk, V);
     if (data_lengths && (data_lengths_dtype < CTCB_I32 || data_lengths_dtype > CTCB_F64))
         return fail(CTCB_INVALID_VALUE, "unsupported length dtype %d", data_lengths_dtype);
-    const size_t dsm = 2 * sizeof(int) * (size_t)T;
-    if (dsm > 200 * 1024) return fail(CTCB_UNSUPPORTED, "T=%d too long for the decode kernel", T);
-    if (!proj->hidden || !proj->weight || proj->K <= 0) return fail(CTCB_INVALID_VALUE, "projection: hidden / weight is NULL or K <= 0");
-    if (int rc = check_proj_operands(proj)) return rc;
-    if (!is_device_ptr(out_tokens) || !is_device_ptr(out_lengths) || !is_device_ptr(data_lengths))
-        return fail(CTCB_INVALID_VALUE, "buffers must be CUDA device memory");
-    const int ctas = proj_ctas();
-    const int NT = (V + ctcb::kPN - 1) / ctcb::kPN;
-    CUtensorMap tmA, tmB;
-    if (int rc = encode_proj_maps(proj, T, B, V, ctas, &tmA, &tmB)) return rc;
+    if (int rc = check_collapse_rows(T)) return rc;
+    if (int rc = check_proj_operands(proj, nullptr, nullptr)) return rc;
+    if (!on_device({out_tokens, out_lengths, data_lengths})) return fail(CTCB_INVALID_VALUE, "buffers must be CUDA device memory");
     // no labels and no workspace: of the problem the decode-only epilogue reads the shape and the frame counts
-    ctcb::ProjArgs pa = proj_args(proj, V, ctas);
-    pa.p.T = T; pa.p.B = B; pa.p.V = V; pa.p.blank = blank;
-    pa.p.data_len = data_lengths; pa.p.data_len_dtype = data_lengths_dtype;
-    pa.tok = out_tokens;
-    pa.unk = unk < 0 ? -1 : unk;
-    const int mtiles = (T + ctcb::kPM - 1) / ctcb::kPM;
+    ctcb_problem_t q{};
+    q.T = T; q.B = B; q.V = V; q.blank = blank;
+    q.data_lengths = data_lengths; q.data_lengths_dtype = data_lengths_dtype;
+    ProjLaunch pl;
+    if (int rc = prepare_proj(proj, &q, nullptr, ctcb::kProjDecode, &pl)) return rc;
+    pl.pa.tok = out_tokens;
+    pl.pa.unk = unk < 0 ? -1 : unk;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    CUDA_TRY(ctcb::launch_proj_emit(tmA, tmB, tmA, pa, ctcb::kProjDecode, dim3(ctas, B, (mtiles + ctas - 1) / ctas),
-                                    ctcb::proj_smem_bytes(0, 0, false, NT, ctas, true), st, false));
-    mark(st);
+    CUDA_TRY(ctcb::launch_proj_emit(pl.tmA, pl.tmB, pl.tmC, pl.pa, ctcb::kProjDecode, pl.grid, pl.smem, st, false));
+    ++g_launches;
     // the collapse right behind the projection: stream order, no tile flags
-    if (dsm > 48 * 1024) CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(ctcb::k_greedy_collapse), dsm));
-    ctcb::k_greedy_collapse<<<B, 256, dsm, st>>>(nullptr, 0, data_lengths, data_lengths_dtype, T, blank, pa.unk, out_tokens, out_lengths);
+    if (int rc = launch_greedy_collapse(nullptr, 0, data_lengths, data_lengths_dtype, T, B, blank, pl.pa.unk, out_tokens, out_lengths, st))
+        return rc;
     CUDA_TRY(cudaGetLastError());
-    mark(st);
+    ++g_launches;
     return CTCB_OK;
 }
 
@@ -915,58 +957,29 @@ int ctcb_proj_loss_grad(const ctcb_proj_t* proj, const ctcb_problem_t* p, void* 
     if (!proj) return fail(CTCB_INVALID_VALUE, "proj is NULL");
     if (p && (!p->logits || !p->grad)) return fail(CTCB_INVALID_VALUE, "ctcb_proj_loss_grad needs p->logits and p->grad");
     g_launches = 0;
-    g_proj = proj;
-    const int rc = enqueue(p, workspace, workspace_bytes, stream, PH_FORWARD | PH_BACKWARD, true);
-    g_proj = nullptr;
-    return rc;
+    Request rq(PH_FORWARD | PH_BACKWARD, true);
+    rq.proj = proj;
+    return enqueue(p, workspace, workspace_bytes, stream, rq);
 }
 
 int ctcb_proj_backward(const ctcb_proj_t* proj, const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream_) {
     g_launches = 0;
     if (!proj) return fail(CTCB_INVALID_VALUE, "proj is NULL");
-    g_proj = proj;                                  // validate: the logits pointer is not needed
-    const int vrc = validate(p);
-    g_proj = nullptr;
-    if (vrc) return vrc;
+    if (int rc = validate(p, true)) return rc;
     if (!p->grad) return fail(CTCB_INVALID_VALUE, "grad is NULL");
     const Layout lay = make_layout(p->T, p->B, p->V, p->Lmax, 1);
-    if (lay.fused || lay.dense)
-        return fail(CTCB_UNSUPPORTED, "projection fused with the loss needs V > 64 and V > Lmax + 1 (V=%d, Lmax=%d)", p->V, p->Lmax);
-    if (p->logits_row_offsets) return fail(CTCB_UNSUPPORTED, "projection: packed logits are not supported");
-    if (!workspace) return fail(CTCB_INVALID_VALUE, "workspace is NULL");
-    if (workspace_bytes < lay.total)
-        return fail(CTCB_WORKSPACE_TOO_SMALL, "workspace %zu < required %zu bytes", workspace_bytes, lay.total);
-    if (reinterpret_cast<uintptr_t>(workspace) % 256) return fail(CTCB_INVALID_VALUE, "workspace must be 256-byte aligned");
-    if (!is_device_ptr(workspace) || !is_device_ptr(p->grad) || !is_device_ptr(p->labels) || !is_device_ptr(p->head_grad))
+    if (int rc = check_proj_problem(p, lay)) return rc;          // a shape the forward refuses: before the workspace
+    if (int rc = check_workspace(workspace, workspace_bytes, lay)) return rc;
+    if (!on_device({workspace, p->grad, p->labels, p->head_grad}))
         return fail(CTCB_INVALID_VALUE, "labels/grad/head_grad/workspace must be CUDA device memory (there is no CPU path)");
-    if (!proj->hidden || !proj->weight || proj->K <= 0) return fail(CTCB_INVALID_VALUE, "projection: hidden / weight is NULL or K <= 0");
-    if (int rc = check_proj_operands(proj)) return rc;
-    const int ctas = proj_ctas();
-    const int NT = (p->V + ctcb::kPN - 1) / ctcb::kPN;
-    const size_t smem = ctcb::proj_smem_bytes(p->Lmax, lay.Lp, true, NT, ctas);
-    if (smem > 232448 - 64) return fail(CTCB_UNSUPPORTED, "projection: Lmax=%d label columns do not fit the kernel's shared memory", p->Lmax);
-    CUtensorMap tmA, tmB;
-    if (int rc = encode_proj_maps(proj, p->T, p->B, p->V, ctas, &tmA, &tmB)) return rc;
-    ctcb::ProjArgs pa = proj_args(proj, p->V, ctas);
-    pa.p = to_device_problem(p);
-    pa.w = carve(lay, workspace);
-    // G leaves through TMA tile stores when its rows allow a tensor map, else as coalesced rows from the staging tiles
-    CUtensorMap tmC = tmA;
-    pa.store = 2;
-    if (p->grad_stride_t % 4 == 0 && p->grad_stride_b % 4 == 0 && reinterpret_cast<uintptr_t>(p->grad) % 16 == 0) {
-        const cuuint64_t gdim[3] = {(cuuint64_t)p->V, (cuuint64_t)p->T, (cuuint64_t)p->B};
-        const cuuint64_t gstr[2] = {(cuuint64_t)p->grad_stride_t * 4, (cuuint64_t)p->grad_stride_b * 4};
-        const cuuint32_t box[3] = {32, 32, 1};
-        const cuuint32_t est[3] = {1, 1, 1};
-        const CUresult r = encode_tiled()(&tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, p->grad, gdim, gstr, box, est,
-                                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r == CUDA_SUCCESS) pa.store = 1;
-    }
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    const int mtiles = (p->T + ctcb::kPM - 1) / ctcb::kPM;
-    CUDA_TRY(ctcb::launch_proj_emit(tmA, tmB, tmC, pa, ctcb::kProjGrad, dim3(ctas, p->B, (mtiles + ctas - 1) / ctas), smem, stream, false));
-    mark(stream);
+    if (int rc = check_proj_operands(proj, nullptr, nullptr)) return rc;
+    ProjLaunch pl;
+    if (int rc = prepare_proj(proj, p, &lay, ctcb::kProjGrad, &pl)) return rc;
+    pl.pa.w = carve(lay, workspace);
+    // G leaves as TMA tile stores or as coalesced rows from the staging tiles
+    pl.pa.store = encode_out_map(p->grad, p->grad_stride_t, p->grad_stride_b, p->T, p->B, p->V, &pl.tmC);
+    CUDA_TRY(ctcb::launch_proj_emit(pl.tmA, pl.tmB, pl.tmC, pl.pa, ctcb::kProjGrad, pl.grid, pl.smem, static_cast<cudaStream_t>(stream_), false));
+    ++g_launches;
     return CTCB_OK;
 }
 
@@ -1007,6 +1020,27 @@ int packed_logits_bytes(const ctcb_problem_t* hp, size_t* bytes) {
     *bytes = sizeof(float) * (size_t)hi;
     return CTCB_OK;
 }
+
+// the host entries take compact buffers only: logits whose strides describe TNC or NTC exactly (n_log: their bytes, packed or
+// not; gst_t, gst_b: the strides of a dense gradient in their layout) and NT or TN labels.  host_grad: the gradient is copied
+// back into hp->grad, which must then be dense in the logits' layout
+struct HostLayout { bool packed, tnc; long long gst_t, gst_b; size_t n_dense, n_log; };
+int host_layout(const ctcb_problem_t* hp, bool host_grad, HostLayout* hl) {
+    const int T = hp->T, B = hp->B, V = hp->V, Lmax = hp->Lmax;
+    hl->packed = hp->logits_row_offsets != nullptr;
+    hl->tnc = !hl->packed && hp->logits_stride_t == (long long)B * V && hp->logits_stride_b == V;
+    const bool ntc = hl->packed || (hp->logits_stride_t == V && hp->logits_stride_b == (long long)T * V);
+    if (!hl->tnc && !ntc) return fail(CTCB_INVALID_VALUE, "host entry needs compact TNC or NTC logits");
+    hl->gst_t = hl->tnc ? (long long)B * V : V;
+    hl->gst_b = hl->tnc ? V : (long long)T * V;
+    if (host_grad && (hp->grad_stride_t != hl->gst_t || hp->grad_stride_b != hl->gst_b))
+        return fail(CTCB_INVALID_VALUE, "host entry needs a dense grad in the logits' layout");
+    if (Lmax > 0 && !((hp->label_stride_b == Lmax && hp->label_stride_l == 1) || (hp->label_stride_b == 1 && hp->label_stride_l == B)))
+        return fail(CTCB_INVALID_VALUE, "host entry needs compact NT or TN labels");
+    hl->n_dense = sizeof(float) * (size_t)T * B * V;
+    hl->n_log = hl->n_dense;
+    return hl->packed ? packed_logits_bytes(hp, &hl->n_log) : CTCB_OK;
+}
 }
 
 int ctcb_loss_grad_host(const ctcb_problem_t* hp, int device) { return loss_grad_host_impl(hp, device, nullptr); }
@@ -1020,7 +1054,7 @@ namespace {
 // dev_grad != nullptr: the gradient is computed but stays in the device scratch (its address is
 // returned); hp->grad is ignored
 int loss_grad_host_impl(const ctcb_problem_t* hp, int device, float** dev_grad) {
-    if (int rc = validate(hp)) return rc;
+    if (int rc = validate(hp, false)) return rc;
     if (device < 0 || device >= 64) return fail(CTCB_INVALID_VALUE, "device %d out of range", device);
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || device >= ndev)
@@ -1028,22 +1062,12 @@ int loss_grad_host_impl(const ctcb_problem_t* hp, int device, float** dev_grad) 
     CUDA_TRY(cudaSetDevice(device));
     const int T = hp->T, B = hp->B, V = hp->V, Lmax = hp->Lmax;
     const bool need_grad = hp->grad != nullptr || dev_grad != nullptr;
-    // the host entry takes compact buffers only: strides must describe TNC or NTC exactly
-    const bool packed = hp->logits_row_offsets != nullptr;
-    const bool tnc = !packed && hp->logits_stride_t == (long long)B * V && hp->logits_stride_b == V;
-    const bool ntc = packed || (hp->logits_stride_t == V && hp->logits_stride_b == (long long)T * V);
-    if (!tnc && !ntc) return fail(CTCB_INVALID_VALUE, "host entry needs compact TNC or NTC logits");
-    const long long gst_t = tnc ? (long long)B * V : V, gst_b = tnc ? V : (long long)T * V;      // dense gradient, the logits' layout
-    if (need_grad && !dev_grad && (hp->grad_stride_t != gst_t || hp->grad_stride_b != gst_b))
-        return fail(CTCB_INVALID_VALUE, "host entry needs a dense grad in the logits' layout");
-    if (Lmax > 0 && !((hp->label_stride_b == Lmax && hp->label_stride_l == 1) || (hp->label_stride_b == 1 && hp->label_stride_l == B)))
-        return fail(CTCB_INVALID_VALUE, "host entry needs compact NT or TN labels");
-
+    HostLayout hl;
+    if (int rc = host_layout(hp, need_grad && !dev_grad, &hl)) return rc;
+    const bool packed = hl.packed;
+    const size_t n_dense = hl.n_dense, n_log = hl.n_log;
     size_t ws_bytes = 0;
     ctcb_workspace_bytes(T, B, V, Lmax, need_grad, &ws_bytes);
-    const size_t n_dense = sizeof(float) * (size_t)T * B * V;
-    size_t n_log = n_dense;
-    if (packed) { if (int rc = packed_logits_bytes(hp, &n_log)) return rc; }
     const size_t n_lab = dt_size(hp->label_dtype) * (size_t)B * (Lmax > 0 ? Lmax : 1);
     const size_t n_dl = hp->data_lengths ? dt_size(hp->data_lengths_dtype) * (size_t)B : 0;
     const size_t n_ll = hp->label_lengths ? dt_size(hp->label_lengths_dtype) * (size_t)B : 0;
@@ -1083,7 +1107,7 @@ int loss_grad_host_impl(const ctcb_problem_t* hp, int device, float** dev_grad) 
         d.logits = reinterpret_cast<float*>(base + o_log);
         d.logits_row_offsets = packed ? reinterpret_cast<const int64_t*>(base + o_off) : nullptr;
         d.grad = need_grad ? reinterpret_cast<float*>(base + o_grad) : nullptr;
-        if (dev_grad) { d.grad_stride_t = gst_t; d.grad_stride_b = gst_b; }
+        if (dev_grad) { d.grad_stride_t = hl.gst_t; d.grad_stride_b = hl.gst_b; }
         d.labels = base + o_lab;
         d.data_lengths = hp->data_lengths ? base + o_dl : nullptr;
         d.label_lengths = hp->label_lengths ? base + o_ll : nullptr;
@@ -1211,17 +1235,12 @@ int ctcb_pipe_destroy(ctcb_pipe_t* p) {
 
 int ctcb_pipe_submit(ctcb_pipe_t* p, const ctcb_problem_t* hp, int64_t* ticket) {
     if (!p || !ticket) return fail(CTCB_INVALID_VALUE, "pipe / ticket is NULL");
-    if (int rc = validate(hp)) return rc;
+    if (int rc = validate(hp, false)) return rc;
     const int T = hp->T, B = hp->B, V = hp->V, Lmax = hp->Lmax;
-    const bool packed = hp->logits_row_offsets != nullptr;
-    const bool tnc = !packed && hp->logits_stride_t == (long long)B * V && hp->logits_stride_b == V;
-    const bool ntc = packed || (hp->logits_stride_t == V && hp->logits_stride_b == (long long)T * V);
-    if (!tnc && !ntc) return fail(CTCB_INVALID_VALUE, "host entry needs compact TNC or NTC logits");
-    if (Lmax > 0 && !((hp->label_stride_b == Lmax && hp->label_stride_l == 1) || (hp->label_stride_b == 1 && hp->label_stride_l == B)))
-        return fail(CTCB_INVALID_VALUE, "host entry needs compact NT or TN labels");
-    const size_t n_dense = sizeof(float) * (size_t)T * B * V;
-    size_t n_log = n_dense;
-    if (packed) { if (int rc = packed_logits_bytes(hp, &n_log)) return rc; }
+    HostLayout hl;
+    if (int rc = host_layout(hp, false, &hl)) return rc;     // the gradient stays on the device
+    const bool packed = hl.packed;
+    const size_t n_dense = hl.n_dense, n_log = hl.n_log;
     CUDA_TRY(cudaSetDevice(p->device));
     ctcb_pipe::Slot& sl = p->slots[p->next % p->depth];
     if (sl.busy) {   // the caller did not collect this slot's previous batch: its results are overwritten
@@ -1290,7 +1309,7 @@ int ctcb_pipe_submit(ctcb_pipe_t* p, const ctcb_problem_t* hp, int64_t* ticket) 
     d.head_grad = in[4].n ? reinterpret_cast<const float*>(sl.in + in[4].off) : nullptr;
     d.logits_row_offsets = in[5].n ? reinterpret_cast<const int64_t*>(sl.in + in[5].off) : nullptr;
     d.grad = reinterpret_cast<float*>(sl.out + o_grad);
-    d.grad_stride_t = tnc ? (long long)B * V : V; d.grad_stride_b = tnc ? V : (long long)T * V;      // dense, the logits' layout
+    d.grad_stride_t = hl.gst_t; d.grad_stride_b = hl.gst_b;
     d.loss = reinterpret_cast<float*>(sl.out + o_loss);
     // A pinned host loss buffer is written by the recursion kernel itself (B stores of 4 bytes over PCIe): a device->host
     // copy of the loss would queue on the copy engine BEHIND the next batch's 2.4 MB host->device copy, the host would see
@@ -1375,12 +1394,12 @@ int ctcb_greedy_decode_typed(const void* logits, int32_t logits_dtype, int64_t s
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (logits_dtype == CTCB_BF16) {
         if (smem > 48 * 1024)
-            CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(ctcb::k_greedy_decode<ctcb::bf16>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(ctcb::k_greedy_decode<ctcb::bf16>), smem));
         ctcb::k_greedy_decode<ctcb::bf16><<<B, 256, smem, st>>>(static_cast<const ctcb::bf16*>(logits), stride_t, stride_b, data_lengths,
                                                                 data_lengths_dtype, T, B, V, blank, unk < 0 ? -1 : unk, out_tokens, out_lengths);
     } else {
         if (smem > 48 * 1024)
-            CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(ctcb::k_greedy_decode<float>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(ctcb::k_greedy_decode<float>), smem));
         ctcb::k_greedy_decode<float><<<B, 256, smem, st>>>(static_cast<const float*>(logits), stride_t, stride_b, data_lengths,
                                                            data_lengths_dtype, T, B, V, blank, unk < 0 ? -1 : unk, out_tokens, out_lengths);
     }
@@ -1400,7 +1419,7 @@ int ctcb_edit_distance(const int32_t* ref, int64_t ref_stride, const int32_t* re
     const size_t smem = sizeof(int) * ((size_t)max_hyp + 2 * ((size_t)max_hyp + 1));
     if (smem > 200 * 1024) return fail(CTCB_UNSUPPORTED, "max_hyp=%d too long for the edit-distance kernel", max_hyp);
     if (smem > 48 * 1024)
-        CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(ctcb::k_edit_distance), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(ctcb::k_edit_distance), smem));
     ctcb::k_edit_distance<<<B, 128, smem, static_cast<cudaStream_t>(stream)>>>(ref, ref_stride, ref_len, hyp, hyp_stride,
                                                                              hyp_len, max_ref, max_hyp, out_dist, totals);
     CUDA_TRY(cudaGetLastError());
@@ -1631,9 +1650,9 @@ int ctcb_loss_grad_dlpack(const DLManagedTensor* logits, const DLManagedTensor* 
         p.loss_sum = static_cast<double*>(dl_data(s));
     }
     const int phase = (layout_flags >> 8) & 3;   // 0: fused, 1: forward (keep history), 2: backward
-    if (phase == 1) return enqueue(&p, workspace, workspace_bytes, stream, PH_FORWARD, (layout_flags & CTCB_KEEP_FOR_BACKWARD) != 0, ldt);
-    if (phase == 2) return enqueue(&p, workspace, workspace_bytes, stream, PH_BACKWARD, true, ldt);
-    return enqueue(&p, workspace, workspace_bytes, stream, p.grad ? (PH_FORWARD | PH_BACKWARD) : PH_FORWARD, p.grad != nullptr, ldt);
+    Request rq = phase == 1 ? Request(PH_FORWARD, (layout_flags & CTCB_KEEP_FOR_BACKWARD) != 0, ldt)
+               : phase == 2 ? Request(PH_BACKWARD, true, ldt) : loss_grad_request(&p, ldt);
+    return enqueue(&p, workspace, workspace_bytes, stream, rq);
 }
 
 }  // extern "C"

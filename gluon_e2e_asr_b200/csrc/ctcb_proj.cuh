@@ -99,6 +99,32 @@ constexpr int kOccBlocksPerCta = 16;
 constexpr int kOccThreads = 256;
 constexpr int kGradOcc = 8;               // kProjGrad: occupancies of a chunk's label columns in flight per round trip
 
+// ---- host side, shared by ctcb.cu and ctcb_proj.cu ----
+// raises a kernel's opt-in dynamic shared-memory size when a launch needs more than any before it (defined in ctcb.cu)
+cudaError_t ensure_dynamic_smem(const void* fn, size_t bytes);
+// cudaLaunchKernelEx, optionally with programmatic stream serialization (the kernel may start beside the one enqueued
+// before it) and clusters of cluster_x CTAs along x
+template <typename... Params, typename... Args>
+cudaError_t launch_ex(void (*fn)(Params...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, bool programmatic,
+                      int cluster_x, Args&&... args) {
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+    cudaLaunchAttribute attr[2];
+    int na = 0;
+    if (cluster_x > 1) {
+        attr[na].id = cudaLaunchAttributeClusterDimension;
+        attr[na].val.clusterDim.x = cluster_x; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
+        ++na;
+    }
+    if (programmatic) {
+        attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[na].val.programmaticStreamSerializationAllowed = 1;
+        ++na;
+    }
+    cfg.attrs = attr; cfg.numAttrs = na;
+    return cudaLaunchKernelEx(&cfg, fn, static_cast<Args&&>(args)...);
+}
+
 // (a.ctas == 2: grid.x even, launched as clusters of two CTAs along x)
 // host-side launcher, defined in ctcb_proj.cu (its own translation unit: the kernel below is compiled there only)
 // mode: kProjLoss, kProjLossDecode or kProjDecode (what the epilogue computes, see k_proj_emit)

@@ -39,7 +39,8 @@ def _proj_struct(hidden, weight, bias):
     return pj
 
 
-def _check_inputs(hidden, weight, bias):
+def _operands(hidden, weight, bias):
+    """hidden, weight and bias checked and laid out as the projection kernel reads them (unit stride along K)."""
     for name, t in (("hidden", hidden), ("weight", weight)) + ((("bias", bias),) if bias is not None else ()):
         if not isinstance(t, torch.Tensor) or not t.is_cuda:
             raise RuntimeError("proj_ctc_loss has no CPU path: %s must be a CUDA tensor" % name)
@@ -52,6 +53,24 @@ def _check_inputs(hidden, weight, bias):
         raise ValueError("hidden must be (B, T, K) and weight (V, K)")
     if bias is not None and (bias.dim() != 1 or bias.shape[0] != weight.shape[0]):
         raise ValueError("bias must be (V,)")
+    if hidden.stride(2) != 1:
+        hidden = hidden.contiguous()
+    return hidden, weight.contiguous(), bias.contiguous() if bias is not None else None
+
+
+def _proj_problem(hidden, weight, logits, label, pred_lengths, label_lengths, blank_last, tn, need_grad):
+    """The lattice problem of ``hidden @ weight.T``: ``(call, loss, ws, p)``.  ``logits``: the (B, T, V) fp32 buffer the
+    forward writes, or None -- then the problem's logits pointer is NULL and only their shape is known."""
+    B, T, _ = hidden.shape
+    dev = hidden.device
+    shape = logits if logits is not None else torch.empty((B, T, weight.shape[0]), dtype=torch.float32, device="meta")
+    call = _Call(_MetaLogits(shape, dev), label, pred_lengths, label_lengths, blank_last, True, tn)
+    loss = torch.empty((B,), dtype=torch.float32, device=dev)
+    ws = _alloc_ws(call, need_grad)
+    p = call.problem(loss)
+    if logits is None:
+        p.logits = None
+    return call, loss, ws, p
 
 
 class _tf32_matmul:
@@ -70,13 +89,8 @@ class _ProjCtcLossFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, hidden, weight, bias, label, pred_lengths, label_lengths, blank_last, tn, fused=True):
         # fused: False (library product + CtcLoss), True (fused forward with a logits store) or "recompute"
-        _check_inputs(hidden, weight, bias)
-        if hidden.stride(2) != 1:
-            hidden = hidden.contiguous()
-        weight = weight.contiguous()
-        bias = bias.contiguous() if bias is not None else None
-        B, T, K = hidden.shape
-        V = weight.shape[0]
+        hidden, weight, bias = _operands(hidden, weight, bias)
+        B, T, _ = hidden.shape
         dev = hidden.device
         need = any(ctx.needs_input_grad[:3])
         recompute = need and fused == "recompute"        # no logits: the backward forms the product again
@@ -87,14 +101,8 @@ class _ProjCtcLossFn(torch.autograd.Function):
             with _tf32_matmul():      # the library product, written once: what the gradient kernel reads
                 logits = torch.nn.functional.linear(hidden, weight, bias)
         else:
-            logits = torch.empty((B, T, V), dtype=torch.float32, device=dev) if need and not recompute else None
-        shape_only = logits if logits is not None else torch.empty((B, T, V), dtype=torch.float32, device="meta")
-        call = _Call(_MetaLogits(shape_only, dev), label, pred_lengths, label_lengths, blank_last, True, tn)
-        loss = torch.empty((B,), dtype=torch.float32, device=dev)
-        ws = _alloc_ws(call, need)
-        p = call.problem(loss)
-        if logits is None:
-            p.logits = None
+            logits = torch.empty((B, T, weight.shape[0]), dtype=torch.float32, device=dev) if need and not recompute else None
+        call, loss, ws, p = _proj_problem(hidden, weight, logits, label, pred_lengths, label_lengths, blank_last, tn, need)
         pj = _proj_struct(hidden, weight, bias)
         with _on_device(dev):
             if need and not fused:
@@ -195,23 +203,13 @@ def proj_ctc_eval(hidden, weight, bias, label, pred_lengths=None, label_lengths=
     ``blank_label="last"``): the projection's epilogue keeps each frame's best two symbols while it reduces the row, and a
     small kernel collapses repeats and blanks.  The outputs go straight into ``edit_distance``.  fp32 (tf32 product) or
     bfloat16 operands; no autograd graph."""
-    _check_inputs(hidden, weight, bias)
-    if hidden.stride(2) != 1:
-        hidden = hidden.contiguous()
-    weight = weight.detach().contiguous()
-    bias = bias.detach().contiguous() if bias is not None else None
-    B, T, K = hidden.shape
-    V = weight.shape[0]
+    hidden, weight, bias = _operands(hidden, weight, bias)
+    B, T, _ = hidden.shape
     dev = hidden.device
-    meta = torch.empty((B, T, V), dtype=torch.float32, device="meta")
-    call = _Call(_MetaLogits(meta, dev), label, pred_lengths, label_lengths, _blank_last(blank_label), True,
-                 label_layout == "TN")
-    loss = torch.empty((B,), dtype=torch.float32, device=dev)
+    _, loss, ws, p = _proj_problem(hidden, weight, None, label, pred_lengths, label_lengths, _blank_last(blank_label),
+                                   label_layout == "TN", False)
     tokens = torch.empty((B, T), dtype=torch.int32, device=dev)
     lengths = torch.empty((B,), dtype=torch.int32, device=dev)
-    ws = _alloc_ws(call, False)
-    p = call.problem(loss)
-    p.logits = None
     pj = _proj_struct(hidden, weight, bias)
     with _on_device(dev):
         rc = _lib.load().ctcb_proj_forward_decode(ctypes.byref(pj), ctypes.byref(p), 0, -1 if unk is None else int(unk),
@@ -230,11 +228,7 @@ def proj_greedy_decode(hidden, weight, bias, pred_lengths=None, blank=0, unk=Non
     Tokens and lengths are bit-identical to those of ``proj_ctc_eval`` for the same operands, lengths, blank and ``unk``,
     whatever its labels.  Any vocabulary size (no lattice, so no V > 64 condition).  fp32 (tf32 product) or bfloat16
     operands; no autograd graph.  The outputs go straight into ``edit_distance``."""
-    _check_inputs(hidden, weight, bias)
-    if hidden.stride(2) != 1:
-        hidden = hidden.contiguous()
-    weight = weight.detach().contiguous()
-    bias = bias.detach().contiguous() if bias is not None else None
+    hidden, weight, bias = _operands(hidden, weight, bias)
     B, T, _ = hidden.shape
     V = weight.shape[0]
     dev = hidden.device
