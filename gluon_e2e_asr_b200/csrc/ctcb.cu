@@ -466,18 +466,26 @@ struct ProjLaunch {
     size_t smem;
 };
 
-// every projection entry, after its checks: the kernel's shared memory (refused beyond the opt-in maximum when it holds
-// label columns; lay: the layout of a problem with labels, or nullptr), the TMA maps of the operands -- hidden (K, T, B) in
-// boxes of one 128-byte K block x kPM frames, weight (K, V) in boxes of one K block x the CTA's share of a vocabulary tile --,
-// the launch fields and the grid.  mode: what the epilogue computes (k_proj_emit)
-int prepare_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const Layout* lay, int mode, ProjLaunch* pl) {
-    const int ctas = proj_ctas();
+// the projection kernel's shared memory for `mode` (lay: the layout of a problem with labels, or nullptr): it grows with the
+// label row (Lp) and the vocabulary tiles (NT) and is refused beyond the opt-in maximum when it holds label columns
+int proj_smem(const ctcb_problem_t* p, const Layout* lay, int mode, size_t* smem) {
     const int NT = (p->V + ctcb::kPN - 1) / ctcb::kPN;
     const bool store = mode == ctcb::kProjGrad || p->logits != nullptr;
     const bool decode = mode == ctcb::kProjLossDecode || mode == ctcb::kProjDecode;
-    pl->smem = ctcb::proj_smem_bytes(p->Lmax, lay ? lay->Lp : 0, store, NT, ctas, decode);
-    if (lay && pl->smem > 232448 - 64)
-        return fail(CTCB_UNSUPPORTED, "projection: Lmax=%d label columns do not fit the kernel's shared memory", p->Lmax);
+    *smem = ctcb::proj_smem_bytes(p->Lmax, lay ? lay->Lp : 0, store, NT, proj_ctas(), decode);
+    if (lay && *smem > 232448 - 64)
+        return fail(CTCB_UNSUPPORTED, "projection: Lmax=%d, V=%d: the label columns and vocabulary tiles do not fit the kernel's "
+                    "shared memory (%zu bytes)", p->Lmax, p->V, *smem);
+    return CTCB_OK;
+}
+
+// every projection entry, after its checks: the kernel's shared memory (proj_smem), the TMA maps of the operands -- hidden
+// (K, T, B) in boxes of one 128-byte K block x kPM frames, weight (K, V) in boxes of one K block x the CTA's share of a
+// vocabulary tile --, the launch fields and the grid.  mode: what the epilogue computes (k_proj_emit)
+int prepare_proj(const ctcb_proj_t* pj, const ctcb_problem_t* p, const Layout* lay, int mode, ProjLaunch* pl) {
+    const int ctas = proj_ctas();
+    const int NT = (p->V + ctcb::kPN - 1) / ctcb::kPN;
+    if (int rc = proj_smem(p, lay, mode, &pl->smem)) return rc;
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return fail(CTCB_UNSUPPORTED, "cuTensorMapEncodeTiled is not available from this driver");
     const bool bf = pj->operand_dtype == CTCB_PROJ_BF16;
@@ -603,6 +611,14 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
     const bool need_grad = rq.keep_hist || (phases & PH_BACKWARD);
     if ((phases & PH_BACKWARD) && !p->grad) return fail(CTCB_INVALID_VALUE, "grad is NULL");
     const Layout lay = make_layout(p->T, p->B, p->V, p->Lmax, need_grad);
+    if (rq.recompute) {
+        // the recomputing forward keeps its history for ctcb_proj_backward alone: a shape whose backward kernel does not fit
+        // shared memory (it holds 64 KB of G staging tiles more than this forward's kernel: single CTAs from Lp + NT > 2020,
+        // e.g. a 512k vocabulary) is refused here, with the backward's error, before anything runs
+        size_t smem = 0;
+        if (int rc = check_proj_problem(p, lay)) return rc;
+        if (int rc = proj_smem(p, &lay, ctcb::kProjGrad, &smem)) return rc;
+    }
     if (int rc = check_workspace(workspace, workspace_bytes, lay)) return rc;
     if (!on_device({p->logits, p->grad, p->labels, p->logits_row_offsets, workspace}) || !(is_device_ptr(p->loss) || pinned_device_alias(p->loss)))
         return fail(CTCB_INVALID_VALUE, "logits/labels/loss/grad/workspace must be CUDA device memory (there is no CPU path)");

@@ -222,9 +222,9 @@ __global__ void __launch_bounds__(128, CH <= 4 ? (OCC ? 6 : 7) : (CH == 8 ? 4 : 
                 float zb = 0.0f;
                 auto occupancy = [&](int2 av, int hb, int hl, int c) {
                     // alpha's high word with the block's exponent shift applied: an exact zero stays zero, anything that leaves
-                    // the normal range (an occupancy below 2^-1022 times the largest beta') is flushed to zero
+                    // the normal range is flushed to zero (hw_normal_or_zero)
                     int tb = av.x != 0 ? (int)((unsigned)av.x + (unsigned)dsb[c]) : 0, tl = av.y != 0 ? (int)((unsigned)av.y + (unsigned)dsl[c]) : 0;
-                    tb = tb < (1 << 20) ? 0 : tb; tl = tl < (1 << 20) ? 0 : tl;
+                    tb = hw_normal_or_zero(tb); tl = hw_normal_or_zero(tl);
                     zb += (float)(__hiloint2double(tb, 0) * __hiloint2double(tb ? hb : 0, 0));
                     gbuf[rk[c]] = (float)(__hiloint2double(tl, 0) * __hiloint2double(tl ? hl : 0, 0));
                 };

@@ -1469,6 +1469,11 @@ constexpr int kNoState = INT_MIN / 2;
 
 // high word of a positive fp64 -> its 20 mantissa bits as a float in [1,2)
 __device__ __forceinline__ float hw_mant(int h) { return __int_as_float(((h & 0x000fffff) << 3) | 0x3f800000); }
+// alpha's high word after an exponent shift was added to it (k_grad2, k_meet, k_proj_occ): kept while it is a normal positive
+// double, else 0 -- below the normal range (an occupancy below 2^-1022 times the largest beta'; a negative word when the
+// shift wrapped) and at exponent 2047 (inf / NaN).  The latter is reached only by a state whose beta' is exactly 0 (every
+// other state's occupancy is <= 1), where inf * 0 would be NaN; the product is 0 there
+__device__ __forceinline__ int hw_normal_or_zero(int h) { return (unsigned)h - (1u << 20) < 0x7FE00000u ? h : 0; }
 // weight (mantissa product in [1,4), total exponent) of alpha*beta' for one state; an exactly-zero
 // factor (high word 0) gives the exponent kNoState, which xscale0 turns into weight 0
 __device__ __forceinline__ void hw_weight(int ha, int hb, int off, float& wgt, int& e) {

@@ -638,9 +638,9 @@ __device__ __forceinline__ void meet_helper(const MeetCtx& c, const Problem& p, 
                 for (int q = 0; q < P; ++q) {
                     const int2 a_ = ha[f][q];
                     // alpha's high word with the block's exponent shift applied: an exact zero stays zero, anything that
-                    // leaves the normal range (gamma below 2^-1022 times the largest beta') is flushed to zero
+                    // leaves the normal range is flushed to zero (hw_normal_or_zero)
                     int tb = a_.x != 0 ? (int)((unsigned)a_.x + (unsigned)dsb[q]) : 0, tl = a_.y != 0 ? (int)((unsigned)a_.y + (unsigned)dsl[q]) : 0;
-                    tb = tb < (1 << 20) ? 0 : tb; tl = tl < (1 << 20) ? 0 : tl;
+                    tb = hw_normal_or_zero(tb); tl = hw_normal_or_zero(tl);
                     zb[f] += (float)(__hiloint2double(tb, 0) * __hiloint2double(tb ? hbb[f][q] : 0, 0));
                     const float gl = (float)(__hiloint2double(tl, 0) * __hiloint2double(tl ? hbl[f][q] : 0, 0));
                     sts_f32(rowbuf + (uint32_t)(f * PW + rk[q]) * 4u, gl);

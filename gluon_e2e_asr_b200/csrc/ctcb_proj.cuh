@@ -813,7 +813,7 @@ __global__ void __launch_bounds__(kOccThreads) k_proj_occ(Problem p, Workspace w
                     // k_grad2's occupancy: an exact zero stays zero, a value that leaves the normal range is flushed
                     int tb = av[f].x != 0 ? (int)((unsigned)av[f].x + (unsigned)dsb) : 0;
                     int tl = av[f].y != 0 ? (int)((unsigned)av[f].y + (unsigned)dsl) : 0;
-                    tb = tb < (1 << 20) ? 0 : tb; tl = tl < (1 << 20) ? 0 : tl;
+                    tb = hw_normal_or_zero(tb); tl = hw_normal_or_zero(tl);
                     zb[f] += (float)(__hiloint2double(tb, 0) * __hiloint2double(tb ? hb[f] : 0, 0));
                     zl[f] = (float)(__hiloint2double(tl, 0) * __hiloint2double(tl ? hl[f] : 0, 0)) * rP;
                 }

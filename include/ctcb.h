@@ -333,7 +333,9 @@ typedef struct ctcb_proj {
  * and d bias = sum G are plain library GEMMs (gluon_e2e_asr_b200/proj.py).  keep_for_backward with p->logits = NULL: no
  * logits are stored, the gradient comes from ctcb_proj_backward (below).  p->logits_row_offsets is not supported.
  * CTCB_UNSUPPORTED for V <= 64 or V <= Lmax + 1 (there the logits are a few per cent of the projection's traffic and the
- * walkers' fused producers read them once anyway) and for label rows too long for the kernel's shared memory. */
+ * walkers' fused producers read them once anyway) and for label rows or vocabularies too large for the kernel's shared
+ * memory -- with keep_for_backward and p->logits = NULL, too large for ctcb_proj_backward's kernel (refused before anything
+ * runs: with proj_ctas = 1 from ceil(Lmax / 4) * 4 + ceil(V / 256) > 2020, e.g. V > 514048 at Lmax = 12). */
 int ctcb_proj_forward(const ctcb_proj_t* proj, const ctcb_problem_t* p, int32_t keep_for_backward, void* workspace,
                       size_t workspace_bytes, void* stream);
 /* ctcb_proj_forward plus the greedy decode of ctcb_greedy_decode_unk on the logits the projection forms

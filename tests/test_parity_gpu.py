@@ -892,6 +892,19 @@ def test_meet_kernel_edge_cases(dev):
     assert l[1] == 0 and l[3] == 0 and not g[1].any() and not g[3].any()
     feas = [0, 2, 4, 5]
     _check(l[feas], g[feas], lo[feas], go[feas], "k_meet edge cases")
+    # tight utterances (T_b = L_b + repeats for nine of the 64 rows): beta' is exactly 0 on most states of their late
+    # frames, where k_meet must count a state as empty rather than multiply its shifted alpha by zero
+    d = make_batch(64, 140, 46, 120, seed=3)
+    lo, go, ok = _c_oracle(d)
+    assert ok.all()
+    t = _to(dev, d)
+    with _env(meet=1):
+        ops._ws_cache.clear()
+        loss, grad = ctc_loss_and_grad(t["pred"], t["label"], t["pred_lengths"], t["label_lengths"])
+        assert _lib_launches() == 1
+    ops._ws_cache.clear()
+    assert torch.isfinite(grad).all()
+    _check(loss.cpu().numpy(), grad.cpu().numpy(), lo, go, "k_meet tight utterances")
 
 
 # ---- k_grad2: the gradient kernel that normalises by P(l|x) (ctcb_grad2.cuh) ---------------------------
@@ -899,6 +912,9 @@ def test_meet_kernel_edge_cases(dev):
     (2, 12, 5, 3, 1, False, 1), (3, 7, 46, 2, 3, False, 4), (5, 100, 33, 40, 5, False, 2), (6, 64, 64, 31, 6, False, 4),
     (8, 200, 46, 50, 1, True, 3), (32, 500, 46, 120, 0, False, 4), (8, 300, 46, 200, 7, False, 2),
     (16, 2000, 46, 300, 0, False, 16), (300, 120, 46, 120, 60, False, 4),
+    (4, 1100, 46, 383, 13, False, 2), (3, 1100, 64, 511, 17, False, 4),    # walker configurations (2,6) and (2,8)
+    # T barely above L: most utterances have T_b = L_b + repeats, so beta' is exactly 0 on most states of their late frames
+    (16, 530, 64, 511, 19, False, 4), (64, 140, 46, 120, 23, False, 4),
 ])
 def test_grad2_kernel_vs_c_oracle(dev, B, T, V, L, seed, peaky, blocks):
     """k_grad2 forced on (it is the default only from 64 utterances on): every register-chunk variant (CH 1..16),

@@ -98,6 +98,29 @@ def test_backward_entry_is_unsupported_where_the_forward_is(lib, V, L):
     assert b"V > 64" in l.ctcb_last_error()
 
 
+def test_recompute_forward_refuses_what_its_backward_cannot_take(lib):
+    """proj_ctas=1: the backward's kernel does not fit shared memory once Lp + NT > 2020 (label-row words, 256-column
+    vocabulary tiles); at Lmax = 4 that is V > 256 * 2016.  ctcb_proj_forward(keep_for_backward=1, logits NULL) refuses such
+    a shape before it looks at the workspace, with the backward's error; one vocabulary tile fewer, without
+    keep_for_backward, or with CTA pairs, the shape passes that check (and these host buffers fail at the workspace)."""
+    l, keep = lib.load(), []
+    pj, p = _args(lib, keep)                     # host buffers of a small shape: only the shape fields change below
+    p.grad = None
+
+    def forward(V, keep_for_backward):
+        p.V = V
+        return l.ctcb_proj_forward(ctypes.byref(pj), ctypes.byref(p), keep_for_backward, None, 0, None)
+
+    limit = 256 * (2020 - 4)
+    with lib.options(proj_ctas=1):
+        assert forward(limit + 1, 1) == lib.CTCB_UNSUPPORTED
+        assert b"shared memory" in l.ctcb_last_error()
+        for V, k in ((limit, 1), (limit + 1, 0)):
+            assert forward(V, k) == lib.CTCB_INVALID_VALUE and b"workspace" in l.ctcb_last_error(), (V, k)
+    with lib.options(proj_ctas=2):
+        assert forward(limit + 1, 1) == lib.CTCB_INVALID_VALUE and b"workspace" in l.ctcb_last_error()
+
+
 def test_recompute_option_is_validated_and_has_no_cpu_path():
     torch = pytest.importorskip("torch")
     from gluon_e2e_asr_b200 import proj_ctc_loss
