@@ -17,6 +17,12 @@
  *     labels/lengths and no `.asscalar()` (train_ctc_ce.py:367-368).
  *   - the caller owns every buffer including the workspace; the library borrows them for
  *     the duration of the enqueued work.
+ *   - the workspace's contents on entry do not matter to ctcb_loss_grad*, ctcb_forward*, ctcb_proj_forward,
+ *     ctcb_proj_forward_decode and ctcb_proj_loss_grad: no clearing is needed, whatever an earlier call or another
+ *     tensor left there.  It may be larger than ctcb_workspace_bytes asks, and one buffer (sized for the largest problem)
+ *     may be shared by calls of any shapes enqueued on ONE stream.  The exception is the history of a forward with
+ *     keep_for_backward: the buffer must be left untouched between that forward and its ctcb_backward /
+ *     ctcb_proj_backward.
  *   - there is no CPU fallback: a missing CUDA device or non-device pointer is an error.
  */
 #ifndef CTCB_H_
