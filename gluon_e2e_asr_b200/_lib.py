@@ -30,7 +30,7 @@ EXPORTS = (
     "ctcb_set_option", "ctcb_get_option", "ctcb_greedy_decode_unk", "ctcb_last_grad_kernel",
     "ctcb_proj_forward", "ctcb_proj_loss_grad",
     "ctcb_loss_grad_typed", "ctcb_forward_typed", "ctcb_backward_typed", "ctcb_greedy_decode_typed",
-    "ctcb_proj_forward_decode", "ctcb_proj_greedy_decode", "ctcb_proj_backward",
+    "ctcb_proj_forward_decode", "ctcb_proj_greedy_decode", "ctcb_proj_backward", "ctcb_forward_decode_typed",
 )
 
 
@@ -88,6 +88,7 @@ def load():
     lib.ctcb_loss_grad_typed.argtypes = [PP, i32, vp, sz, vp]
     lib.ctcb_forward_typed.argtypes = [PP, i32, i32, vp, sz, vp]
     lib.ctcb_backward_typed.argtypes = [PP, i32, vp, sz, vp]
+    lib.ctcb_forward_decode_typed.argtypes = [PP, i32, i32, vp, vp, vp, sz, vp]
     lib.ctcb_loss_grad_timed.argtypes = [PP, vp, sz, vp, ctypes.POINTER(ctypes.c_float), ctypes.POINTER(i32)]
     lib.ctcb_loss_grad_host.argtypes = [PP, ctypes.c_int]
     lib.ctcb_loss_grad_host_resident.argtypes = [PP, ctypes.c_int, ctypes.POINTER(vp)]

@@ -122,11 +122,9 @@ struct WalkEntry { int P, NW; WalkFn fn[2][2]; WalkFn fused_bf16[2]; };   // fn[
 #ifdef CTCB_SMALL_TABLE   // experiment builds: the configurations the BASELINE shapes use
 const WalkEntry kWalkTable[] = { WALK(1, 1), WALK(2, 1), WALK(1, 4), WALK(2, 2), WALK(4, 1), WALK(2, 3), WALK(2, 5) };
 #else
-const WalkEntry kWalkTable[] = {
-    WALK(1, 1), WALK(2, 1), WALK(4, 1), WALK(1, 2), WALK(2, 2), WALK(4, 2), WALK(1, 3), WALK(2, 3), WALK(4, 3),
-    WALK(1, 4), WALK(2, 4), WALK(4, 4), WALK(2, 5), WALK(2, 6), WALK(1, 8), WALK(2, 8), WALK(4, 8),
-    WALK(2, 12), WALK(2, 16), WALK(4, 16),
-};
+#define WALK_ENTRY(P_, NW_) WALK(P_, NW_),
+const WalkEntry kWalkTable[] = { CTCB_WALK_CONFIGS(WALK_ENTRY) };
+#undef WALK_ENTRY
 #endif
 #undef WALK
 
@@ -576,7 +574,7 @@ int launch_proj(Request& rq, const ctcb_problem_t* p, const ctcb::Workspace& w, 
     auto launch_meta = [&](bool programmatic) -> int {
         // per-utterance metadata: k_emit's extra CTA alone (grid.x = 1: every CTA is the metadata CTA)
         CUDA_TRY(ctcb::launch_ex(ctcb::k_emit<1, 0>, dim3(1, p->B), dim3(128), ctcb::emit_smem_bytes(lay.Lp, 0), stream, programmatic, 1,
-                                 pa.p, w));
+                                 pa.p, w, ctcb::DecodeOut{nullptr, -1}));
         mark(rq, stream);
         return CTCB_OK;
     };
@@ -599,12 +597,17 @@ int launch_proj(Request& rq, const ctcb_problem_t* p, const ctcb::Workspace& w, 
     return CTCB_OK;
 }
 
+int check_logits_dtype(int ldt) {
+    if (ldt != CTCB_F32 && ldt != CTCB_BF16)
+        return fail(CTCB_INVALID_VALUE, "logits dtype %d is neither CTCB_F32 nor CTCB_BF16 (fp16 logits are not supported)", ldt);
+    return CTCB_OK;
+}
+
 int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, void* stream_, Request& rq) {
     g_grad_kernel = 0;
     if (int rc = validate(p, rq.proj != nullptr)) return rc;
     const int ldt = rq.ldt, phases = rq.phases;
-    if (ldt != CTCB_F32 && ldt != CTCB_BF16)
-        return fail(CTCB_INVALID_VALUE, "logits dtype %d is neither CTCB_F32 nor CTCB_BF16 (fp16 logits are not supported)", ldt);
+    if (int rc = check_logits_dtype(ldt)) return rc;
     if (ldt != CTCB_F32 && rq.proj) return fail(CTCB_INVALID_VALUE, "the fused projection writes fp32 logits");
     const bool bf = ldt == CTCB_BF16;
     const int esz = dtype_size(ldt);
@@ -655,7 +658,11 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
         int stages = 0;
         if (!pick_stages(lay.W, we->NW, lay.fused ? lay.Lp : 0, &stages))
             return fail(CTCB_UNSUPPORTED, "Lmax=%d V=%d: the emission ring does not fit in shared memory", p->Lmax, p->V);
-        const WalkFn wfn = (bf && lay.fused) ? we->fused_bf16[need_grad ? 1 : 0] : we->fn[lay.fused][need_grad ? 1 : 0];
+        // ctcb_forward_decode_typed: the greedy decode rides on the pass that reads the logits -- the fused walkers' producers
+        // (small vocabularies) or k_emit -- and k_greedy_collapse follows the walkers (no history: need_grad is false)
+        const ctcb::DecodeOut dec{rq.proj ? nullptr : rq.tokens, rq.unk};
+        const WalkFn wfn = (dec.tok && lay.fused) ? ctcb::walk_decode_kernel(we->P, we->NW, bf)
+                         : (bf && lay.fused) ? we->fused_bf16[need_grad ? 1 : 0] : we->fn[lay.fused][need_grad ? 1 : 0];
         size_t smem = ctcb::walk_smem_bytes(lay.W, we->NW, stages, lay.fused ? lay.Lp : 0);
         if (lay.fused && need_grad && (phases & PH_BACKWARD) && overlap_allowed(p->B, true)) {
             // SM partitioning by shared-memory reservation: the gradient kernel runs concurrently
@@ -695,12 +702,16 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
             const int nblk = (lay.NB + bpc - 1) / bpc + 1;          // + the metadata CTA of each utterance
             const dim3 egrid(nblk, p->B);
             const size_t esm = ctcb::emit_smem_bytes(lay.Lp, staged ? p->V : 0);
-            if (staged) {
+            if (dec.tok) {
+                const ctcb::EmitKernel efn = ctcb::emit_decode_kernel(staged ? 4 : vec, nq, bf);
+                if (esm > 48 * 1024) CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(efn), esm));
+                efn<<<egrid, staged ? 256 : 128, esm, stream>>>(dp, w, dec);
+            } else if (staged) {
                 auto efn = bf ? ctcb::k_emit<4, -1, ctcb::bf16> : ctcb::k_emit<4, -1>;
                 if (esm > 48 * 1024) CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(efn), esm));
-                efn<<<egrid, 256, esm, stream>>>(dp, w);
+                efn<<<egrid, 256, esm, stream>>>(dp, w, dec);
             } else {
-#define EMIT_LAUNCH(V_, Q_) (bf ? ctcb::k_emit<V_, Q_, ctcb::bf16> : ctcb::k_emit<V_, Q_>)<<<egrid, 128, esm, stream>>>(dp, w)
+#define EMIT_LAUNCH(V_, Q_) (bf ? ctcb::k_emit<V_, Q_, ctcb::bf16> : ctcb::k_emit<V_, Q_>)<<<egrid, 128, esm, stream>>>(dp, w, dec)
 #define EMIT_NQ(V_) switch (nq) { case 1: EMIT_LAUNCH(V_, 1); break; case 2: EMIT_LAUNCH(V_, 2); break; \
                                   case 4: EMIT_LAUNCH(V_, 4); break; case 8: EMIT_LAUNCH(V_, 8); break;  \
                                   case 16: EMIT_LAUNCH(V_, 16); break; default: EMIT_LAUNCH(V_, 0); break; }
@@ -733,6 +744,7 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
         auto launch_walk = [&](bool after_xchg, bool beside_proj) -> int {
             ctcb::WalkArgs wa{dp, w, p->T, stages, p->blank, p->loss, p->loss_sum, nullptr, 0, 1, 0, 0, 0};
             wa.beside_proj = beside_proj ? 1 : 0;
+            wa.dec = dec;
             // the fused recursion kernel behind whatever the stream holds (the previous step's gradient kernel in a training
             // loop's graph): launched programmatically, its CTAs become resident during that kernel's tail and wait there
             const bool pdl = lay.fused && !after_xchg && !beside_proj && opt(OPT_WALK_PDL) != 0;
@@ -758,8 +770,8 @@ int enqueue(const ctcb_problem_t* p, void* workspace, size_t workspace_bytes, vo
             mark(rq, stream);
         }
         if (rq.tokens) {
-            // an ordinary launch: it acquires the tile flags itself
-            if (int rc = launch_greedy_collapse(w.tflag, w.ntile, p->data_lengths, p->data_lengths_dtype, p->T, p->B, p->blank, rq.unk,
+            // an ordinary launch: it acquires the projection's tile flags itself; behind k_emit / the walkers stream order is enough
+            if (int rc = launch_greedy_collapse(rq.proj ? w.tflag : nullptr, w.ntile, p->data_lengths, p->data_lengths_dtype, p->T, p->B, p->blank, rq.unk,
                                                 rq.tokens, rq.lengths, stream))
                 return rc;
             mark(rq, stream);
@@ -893,6 +905,20 @@ int ctcb_forward_typed(const ctcb_problem_t* p, int32_t logits_dtype, int32_t ke
                        size_t workspace_bytes, void* stream) {
     g_launches = 0;
     Request rq(PH_FORWARD, keep_for_backward != 0, logits_dtype);
+    return enqueue(p, workspace, workspace_bytes, stream, rq);
+}
+
+int ctcb_forward_decode_typed(const ctcb_problem_t* p, int32_t logits_dtype, int32_t unk, int32_t* out_tokens,
+                              int32_t* out_lengths, void* workspace, size_t workspace_bytes, void* stream) {
+    g_launches = 0;
+    if (!out_tokens || !out_lengths) return fail(CTCB_INVALID_VALUE, "NULL argument");
+    if (int rc = validate(p, false)) return rc;
+    if (unk >= p->V) return fail(CTCB_INVALID_VALUE, "unk %d outside the vocabulary (V=%d; -1 = no <unk> rule)", unk, p->V);
+    if (int rc = check_collapse_rows(p->T)) return rc;
+    if (int rc = check_logits_dtype(logits_dtype)) return rc;
+    if (!on_device({out_tokens, out_lengths})) return fail(CTCB_INVALID_VALUE, "buffers must be CUDA device memory");
+    Request rq(PH_FORWARD, false, logits_dtype);
+    rq.tokens = out_tokens; rq.lengths = out_lengths; rq.unk = unk < 0 ? -1 : unk;
     return enqueue(p, workspace, workspace_bytes, stream, rq);
 }
 

@@ -128,6 +128,57 @@ __device__ __forceinline__ float warp_sum(float v) {
     return v;
 }
 
+// ---- greedy decode (k_greedy_decode and the decoding variants of k_emit / k_walk) ----
+// a frame's best two {value, index}: ties go to the lowest index, NaN never wins (better() is a total order on the
+// non-NaN pairs, so the order in which a kernel visits the columns does not change the result)
+struct Top2 { float v1; int i1; float v2; int i2; };
+__device__ __forceinline__ bool better(float va, int ia, float vb, int ib) { return va > vb || (va == vb && ia < ib); }
+__device__ __forceinline__ void top2_push(Top2& t, float v, int i) {
+    if (better(v, i, t.v1, t.i1)) { t.v2 = t.v1; t.i2 = t.i1; t.v1 = v; t.i1 = i; }
+    else if (better(v, i, t.v2, t.i2)) { t.v2 = v; t.i2 = i; }
+}
+// top2_push as selects: the decoding variants insert inside long unrolled bodies, where top2_push's branches would
+// cost reconvergence regions and registers (the result is the same)
+__device__ __forceinline__ void top2_insert(Top2& t, float v, int i) {
+    const bool b1 = better(v, i, t.v1, t.i1), b2 = better(v, i, t.v2, t.i2);
+    t.v2 = b1 ? t.v1 : (b2 ? v : t.v2); t.i2 = b1 ? t.i1 : (b2 ? i : t.i2);
+    t.v1 = b1 ? v : t.v1;               t.i1 = b1 ? i : t.i1;
+}
+constexpr Top2 kTop2Empty{-INFINITY, 0x7fffffff, -INFINITY, 0x7fffffff};
+// merges the lists of the lanes `o` apart.  two = false: the best symbol alone (no <unk> rule), half the shuffles
+__device__ __forceinline__ void top2_merge_xor(Top2& tp, int o) {
+    const float ov1 = __shfl_xor_sync(0xffffffffu, tp.v1, o), ov2 = __shfl_xor_sync(0xffffffffu, tp.v2, o);
+    const int oi1 = __shfl_xor_sync(0xffffffffu, tp.i1, o), oi2 = __shfl_xor_sync(0xffffffffu, tp.i2, o);
+    top2_push(tp, ov1, oi1);
+    top2_push(tp, ov2, oi2);
+}
+__device__ __forceinline__ void top2_merge_xor(Top2& tp, int o, bool two) {
+    const float ov1 = __shfl_xor_sync(0xffffffffu, tp.v1, o);
+    const int oi1 = __shfl_xor_sync(0xffffffffu, tp.i1, o);
+    if (two) {
+        const float ov2 = __shfl_xor_sync(0xffffffffu, tp.v2, o);
+        const int oi2 = __shfl_xor_sync(0xffffffffu, tp.i2, o);
+        top2_insert(tp, ov1, oi1);
+        top2_insert(tp, ov2, oi2);
+    } else {
+        const bool b = better(ov1, oi1, tp.v1, tp.i1);
+        tp.v1 = b ? ov1 : tp.v1; tp.i1 = b ? oi1 : tp.i1;
+    }
+}
+__device__ __forceinline__ void top2_warp_merge(Top2& tp, bool two) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) top2_merge_xor(tp, o, two);
+}
+// the word a decoding kernel leaves per valid frame for k_greedy_collapse: the symbol after the <unk> rule (the second
+// best when the best is `unk`), bit 31 set when the raw best symbol is `unk` (k_proj_emit's DECODE epilogue writes the same)
+__device__ __forceinline__ int decode_word(const Top2& tp, int unk) {
+    const bool is_unk = unk >= 0 && tp.i1 == unk;
+    const int sym = (is_unk && tp.i2 != 0x7fffffff) ? tp.i2 : tp.i1;
+    return sym | (is_unk ? (int)0x80000000 : 0);
+}
+// where the decoding variants of k_emit / k_walk leave their words: tok (B, T), one word per valid frame; unk < 0: no rule
+struct DecodeOut { int* tok; int unk; };
+
 // ---- fp64 exponent-field helpers ------------------------------------------------------
 __device__ __forceinline__ int dexp11(double v) { return (__double2hiint(v) >> 20) & 0x7ff; }   // biased
 __device__ __forceinline__ int dexp(double v) { return dexp11(v) - 1023; }
@@ -224,6 +275,21 @@ __device__ __forceinline__ LT* grad_row(const Problem& p, int b, int t) {
     return reinterpret_cast<LT*>(p.grad) + b * p.gst_b + (long long)t * p.gst_t;
 }
 
+// frames [0, n) of one utterance (frame t at logits + base + t * st_t), a warp per frame -- warp w of nw takes frames w,
+// w + nw, ...: the frame's best two symbols, handed to emit(t, top2) in lane 0
+template <typename LT, typename Emit>
+__device__ __forceinline__ void greedy_frames(const LT* logits, long long base, long long st_t, int n, int V, int warp, int nw, int lane,
+                                              Emit&& emit) {
+    for (int t = warp; t < n; t += nw) {
+        const LT* row = logits + base + t * st_t;
+        Top2 tp = kTop2Empty;
+        for (int v = lane; v < V; v += 32) top2_push(tp, ldx(row + v), v);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) top2_merge_xor(tp, o);
+        if (lane == 0) emit(t, tp);
+    }
+}
+
 __device__ __forceinline__ void st_release_gpu(int* p, int v);
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count);
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes);
@@ -243,8 +309,10 @@ __host__ __device__ inline size_t emit_smem_bytes(int Lp, int staged_V) {
     return staged_V ? emit_slab_bytes(Lp) + (size_t)kG * staged_V * 4 + 64 : (size_t)2 * Lp * sizeof(int);
 }
 
-template <int VEC, int NQ, typename LT = float>
-__global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspace w) {
+// DEC (loss evaluation with the greedy decode, ctcb_forward_decode_typed): every valid frame's best two symbols from the
+// values the variant already holds, one word per frame into dec.tok (decode_word); dec is read by these variants only
+template <int VEC, int NQ, typename LT = float, bool DEC = false>
+__global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspace w, DecodeOut dec) {
     using V_t = typename LV<LT, VEC>::type;
     using S_t = typename LV<LT, 4>::type;          // staged rows: four elements per shared-memory load
     // (a programmatic dependent -- the fused projection, ctcb_proj.cuh -- needs nothing from this kernel and may start at once)
@@ -321,12 +389,27 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
                 mbar_wait(rbar + warp, 0);
                 const S_t* sv = reinterpret_cast<const S_t*>(srowL + (size_t)warp * p.V);
                 float m0 = -INFINITY, m1 = -INFINITY;
+                Top2 tp = kTop2Empty;
                 for (int k = lane; k < nvec; k += 64) {
                     float a[4]; LV<LT, 4>::get(sv[k], a);
                     m0 = fmaxf(m0, fmaxf(fmaxf(a[0], a[1]), fmaxf(a[2], a[3])));
-                    if (k + 32 < nvec) { float c[4]; LV<LT, 4>::get(sv[k + 32], c); m1 = fmaxf(m1, fmaxf(fmaxf(c[0], c[1]), fmaxf(c[2], c[3]))); }
+                    if (DEC) {
+#pragma unroll
+                        for (int i = 0; i < 4; ++i) top2_insert(tp, a[i], 4 * k + i);
+                    }
+                    if (k + 32 < nvec) {
+                        float c[4]; LV<LT, 4>::get(sv[k + 32], c); m1 = fmaxf(m1, fmaxf(fmaxf(c[0], c[1]), fmaxf(c[2], c[3])));
+                        if (DEC) {
+#pragma unroll
+                            for (int i = 0; i < 4; ++i) top2_insert(tp, c[i], 4 * (k + 32) + i);
+                        }
+                    }
                 }
                 const float mx = warp_max(fmaxf(m0, m1));
+                if (DEC) {
+                    top2_warp_merge(tp, dec.unk >= 0);
+                    if (lane == 0) dec.tok[(size_t)b * p.T + t0 + warp] = decode_word(tp, dec.unk);
+                }
                 float s0 = 0.0f, s1 = 0.0f;
                 for (int k = lane; k < nvec; k += 64) {
                     float a[4]; LV<LT, 4>::get(sv[k], a);
@@ -391,6 +474,23 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
                         for (int i = 0; i < VEC; ++i) m = fmaxf(m, e[i]); }
                     mx[f] = m;
                 }
+                if (DEC) {
+                    // frame by frame: the lane's columns (tail included), the warp's merge, lane f writes frame f's word
+#pragma unroll
+                    for (int f = 0; f < F; ++f) {
+                        Top2 tp = kTop2Empty;
+                        if (VEC > 1 && nvec * VEC + lane < p.V) top2_insert(tp, xt[f], nvec * VEC + lane);
+#pragma unroll
+                        for (int q = 0; q < NQ1; ++q) {
+                            if (q * 32 + lane >= nvec) continue;         // the -inf fill of absent loads is not a column
+                            float e[VEC]; LV<LT, VEC>::get(x[f][q], e);
+#pragma unroll
+                            for (int i = 0; i < VEC; ++i) top2_insert(tp, e[i], (q * 32 + lane) * VEC + i);
+                        }
+                        top2_warp_merge(tp, dec.unk >= 0);
+                        if (lane == f && t0 + jf + f < Tb) dec.tok[(size_t)b * p.T + t0 + jf + f] = decode_word(tp, dec.unk);
+                    }
+                }
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1)
 #pragma unroll
@@ -439,13 +539,22 @@ __global__ void __launch_bounds__(NQ < 0 ? 256 : 128) k_emit(Problem p, Workspac
                 const LT* row = rows + j * p.st_t;
                 const V_t* rowv = reinterpret_cast<const V_t*>(row);
                 float mx = -INFINITY;
+                Top2 tp = kTop2Empty;
                 for (int k = lane; k < nvec; k += 32) {
                     float x[VEC]; LV<LT, VEC>::get(__ldg(rowv + k), x);
 #pragma unroll
-                    for (int i = 0; i < VEC; ++i) mx = fmaxf(mx, x[i]);
+                    for (int i = 0; i < VEC; ++i) { mx = fmaxf(mx, x[i]); if (DEC) top2_insert(tp, x[i], k * VEC + i); }
                 }
-                for (int v = nvec * VEC + lane; v < p.V; v += 32) mx = fmaxf(mx, ldx(row + v));
+                for (int v = nvec * VEC + lane; v < p.V; v += 32) {
+                    const float xv = ldx(row + v);
+                    mx = fmaxf(mx, xv);
+                    if (DEC) top2_insert(tp, xv, v);
+                }
                 mx = warp_max(mx);
+                if (DEC) {
+                    top2_warp_merge(tp, dec.unk >= 0);
+                    if (lane == 0) dec.tok[(size_t)b * p.T + t] = decode_word(tp, dec.unk);
+                }
                 float sum = 0.0f;
                 for (int k = lane; k < nvec; k += 32) {          // second pass hits L1/L2
                     float x[VEC]; LV<LT, VEC>::get(__ldg(rowv + k), x);
@@ -666,6 +775,7 @@ struct WalkArgs {
                            // and execute griddepcontrol.wait before they touch memory
     int beside_proj;       // unfused variant launched as the programmatic dependent of the fused projection: metadata and
                            // emission blocks are awaited through Workspace::gprog / tflag instead of the stream order
+    DecodeOut dec;         // read by the decoding variant only (k_walk's DEC): where its producers leave each frame's word
 };
 
 #ifdef CTCB_TRACE
@@ -688,7 +798,7 @@ __host__ __device__ inline size_t walk_smem_bytes(int W, int NW, int stages, int
            (size_t)NW * sizeof(int) + 64 + (fused_Lp ? 16 + kFusedProducers * 64 + (size_t)fused_Lp * sizeof(int) : 0);
 }
 
-template <int P, int NW, int DIR, bool HIST, bool FUSED, typename LT = float>
+template <int P, int NW, int DIR, bool HIST, bool FUSED, typename LT = float, bool DEC = false>
 __device__ __forceinline__ void walk_dir(const WalkArgs& a, unsigned char* smem_raw, int Tb, int Lb, int uflags) {
     constexpr int PW = 32 * P;
     constexpr unsigned FULL = 0xffffffffu;
@@ -761,6 +871,19 @@ __device__ __forceinline__ void walk_dir(const WalkArgs& a, unsigned char* smem_
             for (int i = 1; i < CPL; ++i) mx = fmaxf(mx, cur[i]);
             mx = fmaxf(mx, __shfl_xor_sync(FULL, mx, 1));
             mx = fmaxf(mx, __shfl_xor_sync(FULL, mx, 2));
+            if (DEC) {
+                // the greedy decode while the row is in registers: each frame's best two of its four lanes' columns
+                // (two shuffle steps; the best alone without an <unk> rule), one word per valid frame.  The alpha
+                // producers cover blocks [0, NQr), the beta producers under `meet` the others: every valid frame once
+                Top2 tp = kTop2Empty;
+#pragma unroll
+                for (int i = 0; i < CPL; ++i)
+                    if (i < cpl && col0 + i < V) top2_insert(tp, cur[i], col0 + i);
+                const bool two = a.dec.unk >= 0;
+                top2_merge_xor(tp, 1, two);
+                top2_merge_xor(tp, 2, two);
+                if (valid && qk == 0) a.dec.tok[(size_t)b * a.T + t] = decode_word(tp, a.dec.unk);
+            }
             float e[CPL], sm = 0.0f;
 #pragma unroll
             for (int i = 0; i < CPL; ++i) {                            // rows past T_b are all -inf: keep NaN out
@@ -1253,7 +1376,8 @@ __device__ __forceinline__ void walk_dir(const WalkArgs& a, unsigned char* smem_
     }
 }
 
-template <int P, int NW, bool HIST, bool FUSED, typename LT = float>
+// DEC (fused, loss evaluation only): the producers also leave each valid frame's greedy-decode word (WalkArgs::dec)
+template <int P, int NW, bool HIST, bool FUSED, typename LT = float, bool DEC = false>
 __global__ void __launch_bounds__((NW + (FUSED ? kFusedProducers + 1 : 1)) * 32) k_walk(WalkArgs a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     if (a.pdl_wait) asm volatile("griddepcontrol.wait;" ::: "memory");   // everything enqueued before this kernel is complete and visible
@@ -1346,10 +1470,27 @@ __global__ void __launch_bounds__((NW + (FUSED ? kFusedProducers + 1 : 1)) * 32)
             w.Tb[b] = Tb; w.Lb[b] = L; w.flags[b] = flags;
         }
     }
-    if (flags & UTT_INFEASIBLE) return;
-    if (blockIdx.y == 0) walk_dir<P, NW, 0, HIST, true, LT>(a, smem_raw, Tb, L, flags);
-    else                 walk_dir<P, NW, 1, HIST, true, LT>(a, smem_raw, Tb, L, flags);
+    if (flags & UTT_INFEASIBLE) {
+        // no producers run, but hypotheses do not depend on the labels: the alpha CTA decodes the frames, a warp per frame
+        if (DEC && blockIdx.y == 0)
+            greedy_frames(utt_logits<LT>(p, b), 0, p.st_t, Tb, p.V, tid >> 5, nthr >> 5, tid & 31,
+                          [&](int t, const Top2& tp) { a.dec.tok[(size_t)b * p.T + t] = decode_word(tp, a.dec.unk); });
+        return;
+    }
+    if (blockIdx.y == 0) walk_dir<P, NW, 0, HIST, true, LT, DEC>(a, smem_raw, Tb, L, flags);
+    else                 walk_dir<P, NW, 1, HIST, true, LT, DEC>(a, smem_raw, Tb, L, flags);
 }
+
+// the walker configurations {P, NW} the library instantiates (ctcb.cu's table, ctcb_decode.cu's decoding variants)
+#define CTCB_WALK_CONFIGS(X) X(1, 1) X(2, 1) X(4, 1) X(1, 2) X(2, 2) X(4, 2) X(1, 3) X(2, 3) X(4, 3) \
+    X(1, 4) X(2, 4) X(4, 4) X(2, 5) X(2, 6) X(1, 8) X(2, 8) X(4, 8) X(2, 12) X(2, 16) X(4, 16)
+
+// host side: the decoding instantiations (k_walk<P, NW, false, true, LT, true> and k_emit<VEC, NQ, LT, true>) are compiled
+// in a translation unit of their own, ctcb_decode.cu, which hands their addresses to ctcb.cu's launch path
+using WalkKernel = void (*)(WalkArgs);
+using EmitKernel = void (*)(Problem, Workspace, DecodeOut);
+WalkKernel walk_decode_kernel(int P, int NW, bool bf16);    // nullptr for a configuration outside CTCB_WALK_CONFIGS
+EmitKernel emit_decode_kernel(int vec, int nq, bool bf16);  // nq: -1 staged (vec 4), 0 two-pass, 1..16 register-resident
 
 // ---------------------------------------------------------------------------------------
 // k_mailbox_exchange: the loss-sum exchange of section 8e over NVLink peer memory.  One warp.
@@ -1927,12 +2068,6 @@ __global__ void __launch_bounds__(256) k_scale_rows(float* grad, long long gst_t
 // it differs from the RAW best symbol of frame j-1 (the reference compares against trans[j-1], not against
 // the substituted symbol) and is not the blank.
 // ---------------------------------------------------------------------------------------
-struct Top2 { float v1; int i1; float v2; int i2; };
-__device__ __forceinline__ bool better(float va, int ia, float vb, int ib) { return va > vb || (va == vb && ia < ib); }
-__device__ __forceinline__ void top2_push(Top2& t, float v, int i) {
-    if (better(v, i, t.v1, t.i1)) { t.v2 = t.v1; t.i2 = t.i1; t.v1 = v; t.i1 = i; }
-    else if (better(v, i, t.v2, t.i2)) { t.v2 = v; t.i2 = i; }
-}
 #ifndef CTCB_NO_PLAIN_KERNELS   // non-template kernels: defined in ctcb.cu's translation unit only
 // the collapse of frames 0..n-1 by a block of 256 threads: keep[t] = sym[t] != blank && (t == 0 || sym[t] != path[t-1]),
 // compacted in order into out[0..len).  Returns len (in every thread); s_scan: 8 ints of shared memory

@@ -47,6 +47,16 @@ class CtcLoss(torch.nn.Module):
 
     hybrid_forward = forward   # name used by the reference (loss.py:121)
 
+    def evaluate(self, pred, label, pred_lengths=None, label_lengths=None, unk=None):
+        """The validation pass (train_ctc_ce.py:143-168) in one read of the logits: ``ops.ctc_eval`` with this block's
+        layouts and blank -- ``(loss (B,), tokens (B,T) int32, lengths (B,) int32)``, the loss weighted as ``forward``
+        weights it, no autograd graph.  ``tokens`` / ``lengths`` go straight into ``edit_distance``."""
+        loss, tokens, lengths = ops.ctc_eval(pred, label, pred_lengths, label_lengths, self._blank_label, self._layout,
+                                             self._label_layout, unk)
+        if self._weight is not None:
+            loss = loss * self._weight
+        return loss, tokens, lengths
+
     def fused(self, pred, label, pred_lengths=None, label_lengths=None, head_grad=None, **kw):
         """loss and d(sum head*loss)/d pred in one library call (training hot path)."""
         return ops.ctc_loss_and_grad(pred, label, pred_lengths, label_lengths, head_grad,

@@ -18,7 +18,7 @@ from torch.utils import dlpack as _dlpack
 
 from . import _lib
 
-__all__ = ["ctc_loss", "CTCLoss", "ctc_loss_and_grad", "greedy_decode", "workspace_bytes"]
+__all__ = ["ctc_loss", "CTCLoss", "ctc_loss_and_grad", "ctc_eval", "greedy_decode", "workspace_bytes"]
 
 _DT = {torch.int32: _lib.DT_I32, torch.int64: _lib.DT_I64, torch.float32: _lib.DT_F32, torch.float64: _lib.DT_F64}
 # logits element types: float32, and bfloat16 (a mixed-precision model's logits; loss fp32, gradient bf16 -- include/ctcb.h)
@@ -305,6 +305,32 @@ def ctc_loss_and_grad(pred, label, pred_lengths=None, label_lengths=None, head_g
     call.run(_lib.PHASE_FUSED, ws, loss, grad=grad, head=head_grad, loss_sum=loss_sum, status=status,
              handoff=handoff)
     return loss, grad
+
+
+def ctc_eval(pred, label, pred_lengths=None, label_lengths=None, blank_label="first", layout="NTC",
+             label_layout="NT", unk=None):
+    """The validation pass over logits (train_ctc_ce.py:143-160) in one read of them: ``(loss (B,), tokens (B,T) int32,
+    lengths (B,) int32)``.
+
+    ``loss`` is bit-identical to the loss ``ctc_loss`` computes under ``torch.no_grad()``; ``tokens`` / ``lengths`` are
+    bit-identical to ``greedy_decode(pred, pred_lengths, blank, layout, unk)`` (blank 0, or V - 1 for
+    ``blank_label="last"``).  The kernel pass that reads each logits row for the loss also keeps its best two symbols, and
+    a small kernel collapses repeats and blanks (``ctcb_forward_decode_typed``).  float32 or bfloat16 ``pred``; no autograd
+    graph.  The outputs go straight into ``edit_distance``."""
+    pred = _check_data(pred)
+    call = _Call(pred, label, pred_lengths, label_lengths, _blank_last(blank_label), layout == "NTC", label_layout == "TN")
+    dev = pred.device
+    ws = _alloc_ws(call, False)                 # the loss evaluation's size: no history
+    loss = torch.empty((call.B,), dtype=torch.float32, device=dev)
+    tokens = torch.empty((call.B, call.T), dtype=torch.int32, device=dev)
+    lengths = torch.empty((call.B,), dtype=torch.int32, device=dev)
+    p = call.problem(loss)
+    with _on_device(dev):
+        rc = _lib.load().ctcb_forward_decode_typed(ctypes.byref(p), call.ldt, -1 if unk is None else int(unk),
+                                                   tokens.data_ptr(), lengths.data_ptr(), ws.data_ptr(), ws.numel(),
+                                                   _stream_ptr(dev))
+    _lib.check(rc)
+    return loss, tokens, lengths
 
 
 def greedy_decode(pred, pred_lengths=None, blank=0, layout="NTC", unk=None):

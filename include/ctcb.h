@@ -156,6 +156,17 @@ int ctcb_forward_typed(const ctcb_problem_t* p, int32_t logits_dtype, int32_t ke
                        size_t workspace_bytes, void* stream);
 int ctcb_backward_typed(const ctcb_problem_t* p, int32_t logits_dtype, void* workspace, size_t workspace_bytes,
                         void* stream);
+/* The validation pass over logits in one read of them (train_ctc_ce.py:143-160): the loss evaluation of
+ * ctcb_forward_typed(p, logits_dtype, keep_for_backward = 0, ...) -- same loss, loss_sum, status, packed logits and pending
+ * ctcb_mailbox_exchange_with_next -- plus ctcb_greedy_decode_typed on the same logits: frame counts from p->data_lengths
+ * (truncated, clamped to [0, T]), blank p->blank, unk = -1 (or below) for no <unk> rule.  The pass that reads the logits
+ * (the fused walkers' producer warps for V <= 64, k_emit otherwise) also keeps each frame's best two symbols and
+ * k_greedy_collapse turns them into hypotheses behind the walkers.  out_tokens (B, T) int32, hypothesis prefix then zeros;
+ * out_lengths (B,) int32: bit-identical to ctcb_greedy_decode_typed's.  The workspace is the need_grad = 0 size of
+ * ctcb_workspace_bytes; there is no keep_for_backward.  CTCB_UNSUPPORTED for T too long for the collapse kernel (2 T ints
+ * <= 200 KB).  Device buffers.  Detected by symbol, like the other *_typed entries. */
+int ctcb_forward_decode_typed(const ctcb_problem_t* p, int32_t logits_dtype, int32_t unk, int32_t* out_tokens,
+                              int32_t* out_lengths, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Measurement aid (bench.py's roofline leg): ctcb_loss_grad with a CUDA event recorded on
  * `stream` after every kernel; synchronises and returns the per-kernel device times in launch
